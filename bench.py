@@ -19,7 +19,9 @@ else the oracle port of the same code path.
 
 Rank 0 prints ONE compact JSON line (< 4 KB: the contract keys + roofline + hbm_kernels + cpu_baseline +
 e2e).  The per-kernel tables, the other BASELINE configs and every variant go to
-profiles/bench_last_full.json (--full-out).
+a new <tempdir>/yolo_b200_bench_full_*.json (--full-out).  `--dump-outputs DIR` writes the losses, gradients and
+detections of the last timed step as .npy files; the inputs are seeded, so two builds run with the same arguments
+can be compared output for output.
 """
 import argparse
 import ctypes
@@ -27,6 +29,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -79,9 +82,16 @@ def parse(argv=None):
                          "batch, 0 = auto: as many (same seeds, first images of the batch) as keep the whole K+W-step run "
                          "within --cpu-budget-s, measured on a 2-image calibration pass")
     ap.add_argument("--cpu-budget-s", type=float, default=150.0)
-    ap.add_argument("--full-out", default=os.path.join(ROOT, "profiles", "bench_last_full.json"),
-                    help="file that receives the full, uncompacted result ('' = none)")
-    return ap.parse_args(argv)
+    ap.add_argument("--full-out", default=None,
+                    help="file that receives the full, uncompacted result ('' = none); default: a new file in the "
+                         "temporary directory (the source tree may be read-only), named in the printed line's `full`")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last timed step of the main workload computed (losses, "
+                         "gradients, detections) as DIR/<name>.npy, for comparing two builds output for output")
+    args = ap.parse_args(argv)
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -110,6 +120,53 @@ def make_heads(B, img, nc, seed):
 
 def tensor_bytes(ts):
     return int(sum(t.numel() * t.element_size() for t in ts))
+
+
+DUMP_BUDGET_BYTES = 64 << 20
+# the detections' share of the budget: their number depends on the data, the gradients' size only on the arguments
+DUMP_DETECTIONS_BYTES = 16 << 20
+DUMP_SMALL_BYTES = 1 << 20      # losses, offsets, candidate counts: always whole
+
+
+def _sample_rows(a, nbytes):
+    """Rows of `a` (first axis) at fixed seeded positions, sorted, chosen from len(a) and nbytes alone; each kept
+    row also costs 8 bytes of stored position."""
+    k = int(nbytes // (a[0].nbytes + 8))
+    return np.unique(np.random.default_rng(1234).integers(0, len(a), k))
+
+
+def dump_outputs(out_dir, losses, grads, det, rows, offsets):
+    """--dump-outputs: what a caller of the step receives, as out_dir/<name>.npy (float32, or float64 for integers):
+      losses (4,) [total, bbox, obj, cls];  grad_s<k>: d total / d heads[k], shaped like the heads;
+      detections (n, 6) [x1, y1, x2, y2, conf, class], the kept boxes of every image in order, best first;
+      detection_offsets (B+1,): image b's detections are rows offsets[b]:offsets[b+1];
+      candidates (B,): boxes per image that passed the confidence threshold.
+    The files stay within DUMP_BUDGET_BYTES.  Gradients larger together than their share are written as a sample of
+    their flattened elements, and detections larger than DUMP_DETECTIONS_BYTES as a sample of their rows.  The sampled
+    positions are drawn from a fixed seed and depend only on the array's own shape (the gradients' shapes, for their
+    share), so two builds that compute the same arrays write the same files.  A sampled array <name> comes with
+    <name>_index.npy (the positions, float64) and <name>_shape.npy (its full shape)."""
+    torch.cuda.synchronize()
+    n = max(int(offsets[-1]), 0)
+    arrays = {"losses": losses}
+    arrays.update({f"grad_s{k}": g for k, g in enumerate(grads)})
+    arrays.update({"detections": rows[:n], "detection_offsets": offsets, "candidates": det["counts"]})
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    arrays = {k: v.astype(np.float32 if v.dtype == np.float32 else np.float64) for k, v in arrays.items()}
+    grad_budget = DUMP_BUDGET_BYTES - DUMP_DETECTIONS_BYTES - DUMP_SMALL_BYTES
+    grad_bytes = sum(arrays[f"grad_s{k}"].nbytes for k in range(len(grads)))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        pick = None
+        if k.startswith("grad_s") and grad_bytes > grad_budget:
+            pick = _sample_rows(a.reshape(-1), grad_budget * a.nbytes / grad_bytes)
+        elif k == "detections" and a.nbytes > DUMP_DETECTIONS_BYTES:
+            pick = _sample_rows(a, DUMP_DETECTIONS_BYTES)
+        if pick is not None:
+            np.save(os.path.join(out_dir, k + "_index.npy"), pick.astype(np.float64))
+            np.save(os.path.join(out_dir, k + "_shape.npy"), np.array(a.shape, dtype=np.float64))
+            a = a.reshape(-1)[pick] if k.startswith("grad_s") else a[pick]
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def r3(x):
@@ -404,18 +461,23 @@ def b200_main(args, rank, local_rank, world):
     if rank != 0:
         return
     full["numa"] = numa
+    full_out = args.full_out
+    if full_out is None:   # a new file of this run's own: the temporary directory may be shared by several users
+        fd, full_out = tempfile.mkstemp(prefix="yolo_b200_bench_full_", suffix=".json")
+        os.close(fd)
+    full["full_out"] = full_out or None
     full["other_configs"] = others
     full["dist_parity"] = dist_parity
     if not args.no_cpu_baseline:
         full["cpu_baseline"] = cpu_baseline_subprocess(args)
     line = compact_line(full)
-    if args.full_out:
+    if full_out:
         try:
-            os.makedirs(os.path.dirname(args.full_out), exist_ok=True)
-            with open(args.full_out, "w") as f:
+            os.makedirs(os.path.dirname(full_out) or ".", exist_ok=True)
+            with open(full_out, "w") as f:
                 json.dump(full, f, indent=1)
         except OSError as e:  # pragma: no cover
-            print(f"bench.py: could not write {args.full_out}: {e}", file=sys.stderr)
+            print(f"bench.py: could not write {full_out}: {e}", file=sys.stderr)
     print(json.dumps(line, separators=(",", ":")), flush=True)
 
 
@@ -459,7 +521,7 @@ def compact_line(full):
     if full.get("dist_parity") is not None:
         line["dist_parity"] = full["dist_parity"]
     line["numa"] = full.get("numa")
-    line["full"] = "profiles/bench_last_full.json"
+    line["full"] = full.get("full_out")
     n = len(json.dumps(line, separators=(",", ":")))
     for drop in ("kernels_us", "variants", "e2e_graph", "torch_gpu_baseline", "numa"):  # never exceed the driver's parse window
         if n <= MAX_LINE_BYTES:
@@ -572,6 +634,7 @@ def run_workload(args, rank, local_rank, world, dev, group, lib, full):
 
     # ---- device-resident step, eager launches ----------------------------------------------------
     ev = [[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(args.steps)]
+    last_eager = {}   # outputs of the most recent eager step, for --dump-outputs with --launch eager
 
     def step(i, conf=None, record=None):
         heads, tg, packed = dev_sets[i % n_sets]
@@ -585,6 +648,8 @@ def run_workload(args, rank, local_rank, world, dev, group, lib, full):
         det = ops.detect_batch(heads, anchors, img, nc, args.conf if conf is None else conf, args.iou, layout=layout)
         if record:
             record[2].record()
+        if args.dump_outputs:
+            last_eager["out"] = (out4, grads, det)
         return out4, det
 
     for i in range(max(args.warmup, 3)):
@@ -667,6 +732,9 @@ def run_workload(args, rank, local_rank, world, dev, group, lib, full):
 
         reps_ms = timed_reps(graph_steps, args.steps, args.reps, barrier, max_over_ranks)
         assert int(graphs[0].det["n_keep"].min()) >= 0
+        if full and rank == 0 and args.dump_outputs:
+            g = graphs[(args.steps - 1) % n_sets]   # the graph the last timed step replayed
+            dump_outputs(args.dump_outputs, g.losses, g.grads, g.det, g.rows, g.offsets)
         # extra (N=1 only; `value` stays the strictly sequential replay): the same K steps with the graphs of
         # consecutive input sets alternating between two streams, as a double-buffered consumer would run them — the
         # narrow tail of step i (resolve, pack: 64 CTAs) overlaps the head of step i+1.  Not used at N>1: two graphs
@@ -690,6 +758,9 @@ def run_workload(args, rank, local_rank, world, dev, group, lib, full):
     else:
         sampler.samples.clear()
         reps_ms = timed_reps(eager_steps, args.steps, args.reps, barrier, max_over_ranks)
+        if full and rank == 0 and args.dump_outputs:
+            out4, grads, det = last_eager.pop("out")
+            dump_outputs(args.dump_outputs, out4, grads, det, *ops.pack_detections(det))
     sampler.stop_flag = True
     sampler.join()
     step_ms = float(np.median(reps_ms))

@@ -10,7 +10,7 @@ Pinning: `oracle/make_golden.py` imported the real reference from /root/referenc
 installed torchvision 0.26.0 in the build container and wrote `tests/golden/*.npz` (decode, CIoU,
 losses + gradients, target assignment, predict() detections, eval_epoch() metrics, NMS keep sets);
 `tests/test_oracle_cpu.py` checks this restatement against those vectors, against the reference's
-own known-answer tests (tests/test_inference.py:16-76, tests/test_utils.py:82-90), and, when
-/root/reference is present, against the live reference.
+own known-answer tests (tests/test_inference.py:16-76, tests/test_utils.py:82-90), and against the
+original's outputs and signatures stored by `oracle/make_golden_pinned.py`.
 """
 from .ref_path import *  # noqa: F401,F403

@@ -21,6 +21,7 @@ sys.path.insert(0, ROOT)
 import train as ref  # noqa: E402  the reference itself
 import torchvision  # noqa: E402
 from PIL import Image  # noqa: E402
+from oracle.golden_store import pack_seeded_randn  # noqa: E402  seeded randn inputs stored compactly
 
 
 def gen(seed):
@@ -155,7 +156,7 @@ def golden_loss():
         out[f"{name}_cfg"] = np.array([B, img, nc])
         out[f"{name}_losses"] = np.array([float(r) for r in res], dtype=np.float32)
         for s in range(3):
-            out[f"{name}_pred{s}"] = preds[s].detach().numpy()
+            out.update(pack_seeded_randn(f"{name}_pred{s}", preds[s].detach().numpy(), 50 + s))
             out[f"{name}_tgt{s}"] = tgts[s].numpy()
             out[f"{name}_grad{s}"] = preds[s].grad.numpy()
         # single-scale yolo_loss on scale 1 (weights 0.05/1.0/0.5)
@@ -170,7 +171,7 @@ def golden_loss():
     res = ref.yolo_loss_multiscale(preds, tgts, anchors3(), 1)
     out["empty_losses"] = np.array([float(r) for r in res], dtype=np.float32)
     for s in range(3):
-        out[f"empty_pred{s}"] = preds[s].numpy()
+        out.update(pack_seeded_randn(f"empty_pred{s}", preds[s].numpy(), 60 + s))
     np.savez_compressed(os.path.join(OUT, "loss.npz"), **out)
 
 
@@ -325,7 +326,7 @@ def golden_eval():
             imgs = torch.zeros(B, 3, 8, 8)
             loader.append((imgs, [[tgts[s][b] for s in range(3)] for b in range(B)]))
             for s in range(3):
-                out[f"{name}_b{k}_head{s}"] = heads[s].numpy()
+                out.update(pack_seeded_randn(f"{name}_b{k}_head{s}", heads[s].numpy(), (900 + k + img) * 10 + s))
                 out[f"{name}_b{k}_tgt{s}"] = tgts[s].numpy()
         model = FakeEvalModel(batches, img, anchors3())
         res = ref.eval_epoch(model, loader, torch.device("cpu"), num_classes=nc, iou_threshold=iou, conf_threshold=conf)

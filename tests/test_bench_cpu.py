@@ -115,3 +115,45 @@ def test_reference_arm_honours_steps_and_warmup():
     assert "2 of 2 images" in d["cpu_baseline"]["sample"]     # every image of the batch, not a subset
     ref_staged = os.path.exists(os.path.join(ROOT, "baseline", "_ref", "train.py"))
     assert d["cpu_baseline"]["kind"] == ("reference" if ref_staged else "port")
+
+
+def test_dump_outputs_are_float_arrays_within_the_budget(tmp_path, monkeypatch):
+    """--dump-outputs: one float32/float64 .npy per output; small arrays whole, the detections cut at offsets[B]; over
+    the budget, gradients and detections are sampled at seeded positions that depend on their own shapes only, so
+    a different detection count leaves the gradient files unchanged, and the positions and shapes are stored."""
+    import numpy as np
+    bench, _ = _fake_full()
+    monkeypatch.setattr(torch.cuda, "synchronize", lambda *a: None)
+    monkeypatch.setattr(bench, "DUMP_BUDGET_BYTES", 1 << 20)
+    monkeypatch.setattr(bench, "DUMP_DETECTIONS_BYTES", 1 << 12)
+    monkeypatch.setattr(bench, "DUMP_SMALL_BYTES", 1 << 14)
+    g = torch.Generator().manual_seed(0)
+    grads = [torch.randn(2, G, G, 3, 85, generator=g) for G in (32, 16, 8)]
+    rows = torch.randn(2 * 500, 6, generator=g)
+    det = {"counts": torch.tensor([600, 700], dtype=torch.int32)}
+    for out, last in (("a", 900), ("b", 900), ("c", 901)):
+        offsets = torch.tensor([0, 400, last], dtype=torch.int32)
+        bench.dump_outputs(str(tmp_path / out), torch.arange(4.0), grads, det, rows, offsets)
+    load = lambda d, n: np.load(str(tmp_path / d / n))
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(["candidates.npy", "detection_offsets.npy", "losses.npy"] +
+                           [f"{k}{x}.npy" for k in ("detections", "grad_s0", "grad_s1", "grad_s2")
+                            for x in ("", "_index", "_shape")])
+    assert sum(load("a", n).nbytes for n in names) <= 1 << 20
+    for n in names:
+        assert load("a", n).dtype in (np.float32, np.float64) and np.array_equal(load("a", n), load("b", n)), n
+        if n.startswith("grad_s"):
+            assert np.array_equal(load("a", n), load("c", n)), n     # independent of the detection count
+    for s, gr in enumerate(grads):
+        idx, v = load("a", f"grad_s{s}_index.npy").astype(np.int64), load("a", f"grad_s{s}.npy")
+        assert 0 < v.size < gr.numel() and load("a", f"grad_s{s}_shape.npy").tolist() == list(gr.shape)
+        assert np.array_equal(v, gr.numpy().reshape(-1)[idx])
+    idx = load("a", "detections_index.npy").astype(np.int64)
+    assert load("a", "detections_shape.npy").tolist() == [900, 6] and idx.max() < 900
+    assert np.array_equal(load("a", "detections.npy"), rows[:900].numpy()[idx])
+    assert np.array_equal(load("a", "detection_offsets.npy"), [0, 400, 900]) and load("a", "losses.npy").shape == (4,)
+    monkeypatch.setattr(bench, "DUMP_BUDGET_BYTES", 64 << 20)
+    monkeypatch.setattr(bench, "DUMP_DETECTIONS_BYTES", 16 << 20)
+    bench.dump_outputs(str(tmp_path / "whole"), torch.arange(4.0), grads, det, rows, offsets)
+    assert np.array_equal(load("whole", "grad_s0.npy"), grads[0].numpy()) and not os.path.exists(tmp_path / "whole" / "grad_s0_index.npy")
+    assert np.array_equal(load("whole", "detections.npy"), rows[:901].numpy())

@@ -1088,3 +1088,49 @@ def test_batched_sigmoid_is_bit_identical_exhaustively(yb):
     out = (ctypes.c_ulonglong * 2)(7, 7)
     yb._lib.check(yb._lib.lib().yb_selftest_sigmoid(out, torch.cuda.current_stream().cuda_stream), "yb_selftest_sigmoid")
     assert (int(out[0]), int(out[1])) == (0, 0)
+
+
+def test_bench_dump_outputs_are_the_last_timed_step(yb, tmp_path):
+    """bench.py --dump-outputs: graph replay and eager launches dump the same files, and they are what the step
+    computes on the input set of the last timed step ((steps - 1) % n_sets), not on another set."""
+    import importlib.util
+    import os
+    import subprocess
+    import sys
+    from yolo_from_scratch_b200 import ops
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    bench_py = os.path.join(root, "bench.py")
+    B, img, nc, steps = 4, 160, 3, 3
+    base = [sys.executable, bench_py, "--batch", str(B), "--img", str(img), "--nc", str(nc), "--steps", str(steps),
+            "--warmup", "1", "--reps", "1", "--no-other-configs", "--no-variants", "--no-e2e", "--no-cpu-baseline",
+            "--no-torch-gpu-baseline", "--full-out", ""]
+    for launch in ("graph", "eager"):
+        p = subprocess.run(base + ["--launch", launch, "--dump-outputs", str(tmp_path / launch)], capture_output=True,
+                           text=True, timeout=900)
+        assert p.returncode == 0, p.stderr[-3000:]
+    names = sorted(os.listdir(tmp_path / "graph"))
+    assert names == sorted(os.listdir(tmp_path / "eager")) and "grad_s0.npy" in names and "detections.npy" in names
+    load = lambda d, n: np.load(str(tmp_path / d / n))
+    for n in names:
+        assert np.array_equal(load("graph", n), load("eager", n)), n
+
+    spec = importlib.util.spec_from_file_location("bench_mod", bench_py)
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    dev = torch.device("cuda")
+    anchors, grids = ops.default_anchors(dev), [img // 8, img // 16, img // 32]
+
+    def step_of_set(k):   # run_workload's input set k on rank 0
+        heads = [h.to(dev) for h in bench.make_heads(B, img, nc, 1234 + 1000 * k)]
+        tg = ops.build_targets(bench.make_labels(np.random.default_rng(4321 + k), B, nc), anchors, grids, nc, img)
+        out4, _, grads = ops.loss_forward_backward(heads, tg, anchors, nc, ops.MULTISCALE_OBJ_WEIGHTS, [True] * 3)
+        rows, offsets = ops.pack_detections(ops.detect_batch(heads, anchors, img, nc, bench.CONF, bench.IOU))
+        return out4.cpu().numpy(), [g.cpu().numpy() for g in grads], rows[:int(offsets[-1])].cpu().numpy()
+
+    last = (steps - 1) % 4
+    losses, grads, dets = step_of_set(last)
+    np.testing.assert_array_equal(load("graph", "losses.npy"), losses)
+    for s in range(3):
+        np.testing.assert_array_equal(load("graph", f"grad_s{s}.npy"), grads[s])
+    np.testing.assert_array_equal(load("graph", "detections.npy"), dets)
+    assert not np.array_equal(step_of_set(last - 1)[0], losses)

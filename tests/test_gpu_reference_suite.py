@@ -1,31 +1,37 @@
 """north_star: "train.py, eval.py and the existing pytest suite run unchanged with the new path swapped in".
 
-These tests run the UNMODIFIED reference (a byte-identical copy staged by __graft_entry__.build() into the
-git-ignored baseline/_ref/, which travels to the GPU box) through the drop-in boundary on a real GPU:
+These tests run the UNMODIFIED reference (a checkout of the original yolo-from-scratch, see conftest.REFERENCE_DIR)
+through the drop-in boundary on a real GPU:
   * its own pytest suite (everything except tests/test_cli.py, which shells out to `python train.py` without the swap)
     under `-p yolo_from_scratch_b200.pytest_plugin`;
   * its CLI (`train.py data.yaml --epochs 1`, eval mode, inference mode) under `python -m yolo_from_scratch_b200.run`;
-  * `predict` through the rebinding against the golden detections the reference itself produced (tests/golden/predict.npz).
-Logs go to gpurun_out/ (copied into profiles/ by hand for the record).  Skipped when baseline/_ref is absent.
+  * the unchanged model in NHWC through the swap.
+They execute the original's own code, which is not part of this repository and cannot be stored as data, so they
+skip from a clean checkout.  `predict` through the rebinding is checked without the original,
+against the golden detections the reference itself produced (tests/golden/predict.npz).
+Logs go to $YOLO_B200_TEST_LOGS when it is set.
 """
 import os
 import re
 import subprocess
 import sys
+import types
 
 import numpy as np
 import pytest
 import torch
 
+from conftest import REFERENCE_DIR as REF
+
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "baseline", "_ref")
-LOGDIR = os.path.join(ROOT, "gpurun_out")
+LOGDIR = os.environ.get("YOLO_B200_TEST_LOGS", "")
 
 
 def _need_ref():
     if not os.path.exists(os.path.join(REF, "train.py")):
-        pytest.skip("baseline/_ref not staged (run __graft_entry__.build() where /root/reference exists)")
+        pytest.skip("runs the original yolo-from-scratch's own code, which is not part of this repository "
+                    "(YOLO_FROM_SCRATCH_REFERENCE names a checkout of it)")
 
 
 def _env():
@@ -35,6 +41,8 @@ def _env():
 
 
 def _log(name, text):
+    if not LOGDIR:
+        return
     try:
         os.makedirs(LOGDIR, exist_ok=True)
         with open(os.path.join(LOGDIR, name), "w") as f:
@@ -153,29 +161,45 @@ def _canon(dets):
     return a[np.lexsort((a[:, 3], a[:, 2], a[:, 1], a[:, 0], -a[:, 4]))]
 
 
+def _train_stand_in(scale, pad_top, pad_left):
+    """A module with the names install() rebinds in the reference's `train`.  Its letterbox_resize returns the
+    scale and padding the reference's own letterbox_resize gave for the golden image (oracle/make_golden.py:
+    golden_predict stores them in <name>_cfg); everything predict() does after it is the B200 path."""
+    from PIL import Image
+    from yolo_from_scratch_b200.install import PATCHED_FUNCTIONS
+    m = types.ModuleType("train")
+    m.Image = Image
+    m.letterbox_resize = lambda pil_img, img_size: (pil_img, scale, pad_top, pad_left)
+    for n in PATCHED_FUNCTIONS + ("predict",):
+        setattr(m, n, lambda *a, **k: "ref")
+    return m
+
+
 @pytest.mark.parametrize("device", ["cpu", "cuda"])
 @pytest.mark.parametrize("name,wh", [("p_nc1", (200, 160)), ("p_nc3", (224, 224)), ("p_nc80", (100, 128)), ("p_nc1_dense", (160, 160))])
 def test_rebound_predict_reproduces_the_reference_goldens(tmp_path, golden, name, wh, device):
-    """f-3: `train.predict` rebound by install() — same signature, the reference's own image loading and
+    """f-3: `train.predict` rebound by install() — same signature, the module's own image loading and
     letterbox, everything after the model call on the B200 path — against the detections the unmodified
     predict() produced (oracle/make_golden.py: golden_predict), for a CPU model (the reference tests' case)
     and a CUDA model; predict_batch gives the same per image."""
-    _need_ref()
     from PIL import Image
-    sys.path.insert(0, REF)
-    from yolo_from_scratch_b200.install import enable_import_hook
-    enable_import_hook()
-    import train
+    from yolo_from_scratch_b200.install import install, uninstall
     from oracle import ref_path as R
-    assert train.predict.__doc__.startswith("Drop-in")
     g = golden("predict")
     img, nc, conf, iou, scale, pt, pl = g[f"{name}_cfg"]
+    train = install(_train_stand_in(float(scale), int(pt), int(pl)))
+    assert train.predict.__doc__.startswith("Drop-in")
     path = str(tmp_path / f"{name}.png")
     Image.fromarray(np.zeros((wh[1], wh[0], 3), dtype=np.uint8)).save(path)
     dev = torch.device(device)
     heads = [torch.from_numpy(g[f"{name}_head{s}"]).to(dev) for s in range(3)]
     model = _PresetHeads(heads, int(img), [a.to(dev) for a in R.default_anchors()])
-    dets = train.predict(model, path, dev, num_classes=int(nc), conf_threshold=float(conf), iou_threshold=float(iou))
+    try:
+        dets = train.predict(model, path, dev, num_classes=int(nc), conf_threshold=float(conf), iou_threshold=float(iou))
+        many = train.predict_batch(_PresetHeads([torch.cat([h, h]) for h in heads], int(img), model.anchors), [path, path],
+                                   dev, num_classes=int(nc), conf_threshold=float(conf), iou_threshold=float(iou))
+    finally:
+        uninstall(train)
     want = g[f"{name}_dets"]
     assert isinstance(dets, list) and all(isinstance(d, tuple) and len(d) == 6 and isinstance(d[5], int) for d in dets)
     # the golden ran torchvision's CPU kernel; candidates within a few ulp of the confidence threshold may differ
@@ -184,8 +208,6 @@ def test_rebound_predict_reproduces_the_reference_goldens(tmp_path, golden, name
         a, b = _canon(dets), _canon(want)
         assert np.array_equal(a[:, 5], b[:, 5])
         assert np.allclose(a[:, :4], b[:, :4], rtol=1e-4, atol=1e-2) and np.allclose(a[:, 4], b[:, 4], rtol=1e-4, atol=1e-6)
-    many = train.predict_batch(_PresetHeads([torch.cat([h, h]) for h in heads], int(img), model.anchors), [path, path], dev,
-                               num_classes=int(nc), conf_threshold=float(conf), iou_threshold=float(iou))
     assert len(many) == 2 and many[0] == dets and many[1] == dets
 
 

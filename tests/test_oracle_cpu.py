@@ -1,6 +1,6 @@
 """Pins the oracle (oracle/) against the reference: committed golden vectors produced by the
-unmodified reference (oracle/make_golden.py), the reference's own known-answer tests, the
-installed torchvision operator, and — in the build container — the live reference."""
+unmodified reference (oracle/make_golden.py, oracle/make_golden_pinned.py), the reference's own known-answer
+tests and the installed torchvision operator."""
 import numpy as np
 import pytest
 import torch
@@ -211,20 +211,13 @@ def test_cuda_arith_differs_only_by_fma():
     np.testing.assert_array_equal(R.nms_indices(b, s, 0.4, "cpu"), R.nms_indices(b, s, 0.4, "cuda"))
 
 
-# ---- live reference (build container only) ----------------------------------------------------
-def test_live_reference_agrees(reference_module):
-    ref = reference_module
-    g = torch.Generator().manual_seed(77)
-    x = torch.randn(2, 10, 10, 3, 8, generator=g)
-    assert torch.equal(ref.decode_predictions(x, ANCH[2], 320), R.decode(x, ANCH[2], 320))
-    tg = torch.zeros_like(x)
-    tg[0, 3, 4, 1, :5] = torch.tensor([0.4, 0.35, 0.2, 0.3, 1.0])
-    tg[0, 3, 4, 1, 6] = 1.0
-    tg[1, 9, 0, 2, :5] = torch.tensor([0.05, 0.95, 0.1, 0.1, 1.0])
-    tg[1, 9, 0, 2, 5] = 1.0
-    a = ref.yolo_loss(x, tg, ANCH[2], 3)
+# ---- the original's decode_predictions / yolo_loss on one seeded input (oracle/make_golden_pinned.py) ----
+def test_live_reference_agrees(golden):
+    g = golden("live_reference")
+    x, tg, img = T(g["x"]), T(g["tgt"]), int(g["img"])
+    assert torch.equal(R.decode(x, ANCH[2], img), T(g["decode"]))
     b = R.single_scale_loss(x, tg, ANCH[2], 3)
-    assert [float(v) for v in a] == [float(v) for v in b]
+    assert [float(v) for v in b] == g["yolo_loss"].tolist()
 
 
 @pytest.mark.parametrize("name", ["e640", "e320"])
