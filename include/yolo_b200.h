@@ -263,6 +263,54 @@ int yb_pack_detections(const float* boxes, const float* scores, const int64_t* c
 int yb_eval_counts(const yb_heads_desc* d, const float* const* targets_host, double conf_threshold,
                    double iou_threshold, long long* counts3, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * mAP (COCO bbox protocol: COCOeval.evaluateImg + accumulate, area "all", no crowd)
+ *   No reference equivalent: the reference scores a model with eval_epoch's precision/recall only.
+ *   Stage 1, yb_map_match, once per batch, on the output of yb_filter_compact + yb_batched_nms:
+ *     detections of image b = the first min(n_keep[b], max_det) entries of keep[b] (one overall cap);
+ *     ground truth = labels (B,max_gt,5) fp64 [cls, xc, yc, w, h] normalised to the original image,
+ *       n_gt (B) int32, letterbox (B,5) fp64 [orig_w, orig_h, ...] (yb_build_targets' inputs):
+ *       x1 = (xc - w/2)*orig_w, y1 = (yc - h/2)*orig_h, x2 = (xc + w/2)*orig_w, y2 = (yc + h/2)*orig_h;
+ *       nc == 1: every ground truth is class 0 (train.py:201-202);
+ *     IoU = compute_iou_corners (train.py:1064-1084) in fp64 on the fp32 detection corners, 0 if union <= 0;
+ *     per image, class and threshold t: each detection in keep order takes the not yet matched ground truth
+ *       of its class with the highest IoU >= iou_thr[t] (the later one on equal IoU) -> TP, else FP.
+ *   records (B, min(max_det,cap)) receive {score, class, TP bit t of tp}; unused slots have class -1.
+ *   gt_count (nc) int64 += ground truths per class (the caller zeroes it once per evaluation);
+ *   *status |= YB_MAP_BAD_CLASS (ground-truth id outside [0,nc) with nc > 1, or a detection class outside
+ *   [0,nc)), YB_MAP_NMS_FAILED (n_keep[b] < 0; that image contributes no detections).
+ * Between the stages the CALLER orders the records of all batches stably by (class ascending, score
+ *   descending), keeping image order (batch after batch, then batch position) and keep order among equal
+ *   scores — COCO's argsort(-scores, kind="mergesort") over the images in order; class -1 last.  ops.py does it
+ *   with one torch.sort(stable=True) on an int64 key.  seg (nc+1) int64: class c is records [seg[c], seg[c+1]).
+ * Stage 2, yb_map_precision, once per evaluation, one CTA per class:
+ *   tp, fp = cumulative counts (doubles), rc = tp / n_gt_c, pr = tp / (fp + tp + 2^-52);
+ *   precision[t][r][c] = max of pr over positions with rc >= recall_thr[r] (0 if none), recall[t][c] = rc at the
+ *   last detection (0 without detections); both tables -1 for a class without ground truth.
+ *   ws: yb_map_workspace_bytes(number of records, total ground truths or an upper bound, T) bytes;
+ *   *status |= YB_MAP_INCONSISTENT when a class has more TPs than ground truths or ws is too small.
+ * ---------------------------------------------------------------------------------------- */
+#define YB_MAP_MAX_T 16
+#define YB_MAP_MAX_GT 4096
+#define YB_MAP_BAD_CLASS 1
+#define YB_MAP_NMS_FAILED 2
+#define YB_MAP_INCONSISTENT 4
+typedef struct yb_map_record {
+    float score;
+    int32_t cls;     /* -1: unused slot */
+    uint16_t tp;     /* bit t: TP at iou_thr[t] */
+    uint16_t pad;
+} yb_map_record;
+
+int yb_map_match(const float* boxes, const float* scores, const int64_t* classes, const int64_t* keep,
+                 const int* n_keep, int B, int cap, int max_det, const double* labels, const int* n_gt,
+                 const double* letterbox, int max_gt, int nc, const double* iou_thr, int T,
+                 yb_map_record* records, long long* gt_count, int* status, void* stream);
+size_t yb_map_workspace_bytes(long long n_records, long long n_gt_total, int T);
+int yb_map_precision(const yb_map_record* records, const long long* seg, const long long* gt_count, int nc,
+                     int T, const double* recall_thr, int R, double* precision, double* recall, void* ws,
+                     size_t ws_bytes, int* status, void* stream);
+
 /* Per-launch CUDA-event timing for bench.py: when enabled every kernel launch of the library is
  * bracketed by two events on its stream; yb_timing_collect synchronises them, writes
  * "name count total_ms" lines into buf (NUL terminated, truncated to n) and resets. */

@@ -27,6 +27,21 @@ def looks_like_reference(module) -> bool:
     return all(hasattr(module, n) for n in PATCHED_FUNCTIONS + ("YOLODataset", "predict"))
 
 
+def _read_labels(train_module, label_file):
+    """The label lines of one image as YOLODataset.__getitem__ reads them (train.py:148-154): (n,5) fp64
+    [class, xc, yc, w, h]; a missing file is an image without objects."""
+    import numpy as np
+    rows = []
+    label_path = train_module.__dict__["Path"](label_file)
+    if label_path.exists():
+        with open(label_path, encoding="utf-8") as f:
+            for line in f:
+                parts = line.strip().split()
+                if len(parts) == 5:
+                    rows.append([float(int(float(parts[0])))] + [float(x) for x in parts[1:]])
+    return np.array(rows, dtype=np.float64).reshape(-1, 5)
+
+
 def _make_getitem(train_module):
     """Replacement for YOLODataset.__getitem__ (train.py:133-207): image loading and letterbox stay
     the reference's (host image I/O is out of scope); the label loop runs in yb_build_targets."""
@@ -43,15 +58,7 @@ def _make_getitem(train_module):
         orig_w, orig_h = pil_img.size
         pil_img, scale, pad_top, pad_left = g["letterbox_resize"](pil_img, self.img_size)   # :137
         img = torch.from_numpy(np.array(pil_img)).permute(2, 0, 1).float() / 255.0    # :138
-        rows = []
-        label_path = g["Path"](self.labels[idx])
-        if label_path.exists():                                                       # :148-154
-            with open(label_path, encoding="utf-8") as f:
-                for line in f:
-                    parts = line.strip().split()
-                    if len(parts) == 5:
-                        rows.append([float(int(float(parts[0])))] + [float(x) for x in parts[1:]])
-        targets = ops.build_targets([np.array(rows, dtype=np.float64).reshape(-1, 5)], self.anchors, self.grid_sizes,
+        targets = ops.build_targets([_read_labels(train_module, self.labels[idx])], self.anchors, self.grid_sizes,
                                     self.num_classes, self.img_size,
                                     letterbox=[(orig_w, orig_h, scale, pad_top, pad_left)])
         return img, [t[0].cpu() for t in targets]
@@ -90,6 +97,39 @@ def _make_predict(train_module):
                                  letterbox=[lb for _, lb in loaded])
     predict.__doc__ = "Drop-in for train.predict (train.py:1114-1250): same arguments, same return value."
     return predict, predict_batch
+
+
+def _make_evaluate_map(train_module):
+    """`evaluate_map`, a name the reference does not have: COCO-style mAP of a model over a YOLODataset's images
+    and label files (ops.DetectionMAP).  Images are loaded and letterboxed by the module's own Image and
+    letterbox_resize, as predict() does (train.py:1134-1138)."""
+    def evaluate_map(model, dataset, device, num_classes=1, conf_threshold=0.001, iou_threshold=0.4, batch_size=8,
+                     max_det=300):
+        """mAP@[.5:.95] / mAP@0.5 of `model` on `dataset` (its imgs and labels lists).  Returns DetectionMAP.compute()'s
+        dict: map, map50, ap (nc,T), precision (T,R,nc), recall (T,nc), n_gt (nc), n_det (nc)."""
+        import numpy as np
+        import torch
+        g = train_module.__dict__
+        model.eval()
+        img_size = model.img_size
+        metric = ops.DetectionMAP(num_classes, max_det=max_det)
+        n = len(dataset.imgs)
+        with torch.no_grad():
+            for i0 in range(0, n, batch_size):
+                imgs, letterbox, labels = [], [], []
+                for i in range(i0, min(i0 + batch_size, n)):
+                    pil_img = g["Image"].open(dataset.imgs[i]).convert("RGB")
+                    orig_w, orig_h = pil_img.size
+                    pil_img, scale, pad_top, pad_left = g["letterbox_resize"](pil_img, img_size)
+                    imgs.append(torch.from_numpy(np.array(pil_img)).permute(2, 0, 1).float() / 255.0)
+                    letterbox.append((orig_w, orig_h, scale, pad_top, pad_left))
+                    labels.append(_read_labels(train_module, dataset.labels[i]))
+                preds = model(torch.stack(imgs).to(device))
+                det = ops.detect_batch(list(preds), model.anchors, img_size, num_classes, conf_threshold, iou_threshold,
+                                       letterbox=[lb[2:] for lb in letterbox])
+                metric.update(det, ops.pack_labels(labels, img_size, letterbox))
+        return metric.compute()
+    return evaluate_map
 
 
 def channels_last_heads(model):
@@ -139,7 +179,8 @@ def install(train_module, patch_torchvision=False, patch_dataset=True, patch_eva
     channels_last (default: environment YOLO_B200_CHANNELS_LAST=1) makes every `train.YOLO` built afterwards
     run in NHWC, so that the head layout conversion of train.py:608-609 costs nothing (channels_last_heads).
     patch_eval also swaps `eval_epoch` (SURVEY 8f-1: its per-anchor python loop becomes one kernel);
-    patch_predict swaps `predict` and adds `predict_batch` (SURVEY 8f-3); patch_torchvision additionally
+    patch_predict swaps `predict` and adds `predict_batch` (SURVEY 8f-3); `evaluate_map` (COCO-style mAP, a name
+    the reference does not have) is always added; patch_torchvision additionally
     rebinds torchvision.ops.batched_nms process-wide (off by default: predict no longer needs it)."""
     if getattr(train_module, _MARK, False):
         return train_module
@@ -153,6 +194,9 @@ def install(train_module, patch_torchvision=False, patch_dataset=True, patch_eva
     if patch_predict and hasattr(train_module, "predict"):
         saved["predict"] = train_module.predict
         train_module.predict, train_module.predict_batch = _make_predict(train_module)
+    if not hasattr(train_module, "evaluate_map"):
+        saved["evaluate_map"] = None
+        train_module.evaluate_map = _make_evaluate_map(train_module)
     if patch_dataset and hasattr(train_module, "YOLODataset"):
         cls = train_module.YOLODataset
         saved["YOLODataset.__getitem__"] = cls.__getitem__
@@ -187,6 +231,8 @@ def uninstall(train_module):
         train_module.predict = saved["predict"]
         if hasattr(train_module, "predict_batch"):
             del train_module.predict_batch
+    if "evaluate_map" in saved:
+        del train_module.evaluate_map
     if "YOLODataset.__getitem__" in saved:
         train_module.YOLODataset.__getitem__ = saved["YOLODataset.__getitem__"]
         train_module.YOLODataset.compute_anchor_iou = saved["YOLODataset.compute_anchor_iou"]

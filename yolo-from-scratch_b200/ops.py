@@ -13,6 +13,7 @@ include/yolo_b200.h).  PyTorch is used only for device memory, streams and autog
   filter_candidates       train.py:1152-1229 (per-scale body of predict), batched
   nms / batched_nms       torchvision.ops as called at train.py:1232-1233
   detect_batch            filter_candidates + batched_nms + gather (predict :1152-1238 for a batch)
+  DetectionMAP            COCO-style mAP of detect_batch's detections (new; no reference equivalent)
 
 CPU tensors are accepted (the reference's tests pass CPU tensors): they are staged to the GPU,
 computed there, and staged back.  That is staging, not a fallback: without CUDA every function
@@ -817,6 +818,129 @@ def predict_heads(preds, anchors_list, img_size, num_classes=1, conf_threshold=0
     det = detect_batch(list(preds), anchors_list, img_size, num_classes, conf_threshold, iou_threshold, letterbox=letterbox,
                        trick_max_numel=TRICK_MAX_NUMEL_CPU if on_cpu else TRICK_MAX_NUMEL_CUDA)
     return detections_to_lists(det)
+
+
+# --------------------------------------------------------------------------------------------
+# COCO-style mAP (no reference equivalent: the reference's eval_epoch reports precision/recall only)
+# --------------------------------------------------------------------------------------------
+COCO_IOU_THRESHOLDS = tuple(np.linspace(0.5, 0.95, 10).tolist())      # COCOeval Params.iouThrs
+COCO_RECALL_THRESHOLDS = tuple(np.linspace(0.0, 1.0, 101).tolist())   # COCOeval Params.recThrs
+
+
+class DetectionMAP:
+    """mAP@[.5:.95] and mAP@0.5 of the kept detections of `detect_batch`, accumulated over batches on the device.
+    COCO's bbox protocol (evaluateImg + accumulate, area range "all", no crowd) with one overall cap of `max_det`
+    detections per image instead of COCO's per-category maxDets; include/yolo_b200.h states the semantics.
+
+    update(det, labels) enqueues one matching kernel per batch and keeps its records; it never synchronises.
+    compute() sorts the records once, runs the precision kernel and synchronises once."""
+
+    def __init__(self, num_classes, iou_thresholds=COCO_IOU_THRESHOLDS, recall_thresholds=COCO_RECALL_THRESHOLDS,
+                 max_det=300):
+        self.nc = int(num_classes)
+        self.iou_thresholds = np.asarray(iou_thresholds, dtype=np.float64).reshape(-1)
+        self.recall_thresholds = np.asarray(recall_thresholds, dtype=np.float64).reshape(-1)
+        self.max_det = int(max_det)
+        if self.nc < 1:
+            raise ValueError("num_classes must be >= 1")
+        if not 1 <= len(self.iou_thresholds) <= _lib.MAP_MAX_T:
+            raise ValueError(f"1..{_lib.MAP_MAX_T} IoU thresholds supported, got {len(self.iou_thresholds)}")
+        if len(self.recall_thresholds) < 1:
+            raise ValueError("at least one recall threshold is needed")
+        if self.max_det < 0:
+            raise ValueError("max_det must be >= 0")
+        self.device = _device()
+        with torch.cuda.device(self.device):
+            self._iou_thr = torch.tensor(self.iou_thresholds, dtype=torch.float64, device=self.device)
+            self._rec_thr = torch.tensor(self.recall_thresholds, dtype=torch.float64, device=self.device)
+            self._gt_count = torch.zeros(self.nc, dtype=torch.int64, device=self.device)
+            self._status = torch.zeros(1, dtype=torch.int32, device=self.device)
+        self.reset()
+
+    def reset(self):
+        """Forget every batch seen so far."""
+        self._records = []
+        self._gt_total = 0   # upper bound on the ground truths seen: sum of B * max_gt (sizes the workspace)
+        with torch.cuda.device(self.device):
+            self._gt_count.zero_()
+            self._status.zero_()
+
+    def update(self, det, labels: PackedLabels):
+        """Match one batch: `det` is a detect_batch result (letterbox reversed, original-image pixels) and `labels`
+        the batch's PackedLabels (labels normalised to the original image, letterbox rows [orig_w, orig_h, ...])."""
+        boxes, keep = det["boxes"], det["keep"]
+        if boxes.device != self.device:
+            raise ValueError(f"detections on {boxes.device}, DetectionMAP on {self.device}")
+        B, cap = boxes.shape[0], boxes.shape[1]
+        if labels.labels.shape[0] != B or labels.labels.device != self.device:
+            raise ValueError("labels and detections disagree on the batch size or the device")
+        if labels.max_gt > _lib.MAP_MAX_GT:
+            raise ValueError(f"at most {_lib.MAP_MAX_GT} ground truths per image, got max_gt={labels.max_gt}")
+        slots = min(self.max_det, cap)
+        with torch.cuda.device(self.device):
+            rec = torch.empty(B * slots, 3, dtype=torch.int32, device=self.device)   # yb_map_record: score, class, tp
+            _lib.check(_lib.lib().yb_map_match(
+                boxes.data_ptr(), det["scores"].data_ptr(), det["classes"].data_ptr(), keep.data_ptr(),
+                det["n_keep"].data_ptr(), B, cap, self.max_det, labels.labels.data_ptr(), labels.n_gt.data_ptr(),
+                labels.letterbox.data_ptr(), labels.max_gt, self.nc, self._iou_thr.data_ptr(), len(self.iou_thresholds),
+                rec.data_ptr(), self._gt_count.data_ptr(), self._status.data_ptr(), _stream()), "yb_map_match")
+        self._records.append(rec)
+        self._gt_total += B * labels.max_gt
+
+    def compute(self):
+        """{map, map50, ap (nc,T), precision (T,R,nc), recall (T,nc), n_gt (nc), n_det (nc)} on the host (float64 /
+        int64; map50 is None when 0.5 is not a threshold).  Entries of a class without ground truth are -1, and
+        map / map50 are the means of the entries > -1 (-1 when there are none), as COCOeval.summarize."""
+        T, R, nc = len(self.iou_thresholds), len(self.recall_thresholds), self.nc
+        dev = self.device
+        with torch.cuda.device(dev):
+            rec = torch.cat(self._records) if self._records else torch.empty(0, 3, dtype=torch.int32, device=dev)
+            # key = class << 32 | order-reversed score bits: ascending key = class ascending, score descending;
+            # the stable sort keeps image and keep order among equal keys.  Unused slots (class -1) go last.
+            score = rec[:, 0].view(torch.float32) + 0.0          # -0.0 -> +0.0: equal scores must tie
+            bits = score.view(torch.int32).to(torch.int64)
+            asc = bits ^ ((bits >> 31) & 0x7FFFFFFF)              # monotone in the float value
+            cls = rec[:, 1].to(torch.int64)
+            key = torch.where(cls >= 0, cls, nc) * (1 << 32) + (0x7FFFFFFF - asc)
+            key, order = torch.sort(key, stable=True)
+            rec = rec.index_select(0, order).contiguous()
+            seg = torch.searchsorted(key, torch.arange(nc + 1, dtype=torch.int64, device=dev) * (1 << 32))
+            n = rec.shape[0]
+            ws_bytes = _lib.lib().yb_map_workspace_bytes(n, self._gt_total, T)
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            precision = torch.empty(T, R, nc, dtype=torch.float64, device=dev)
+            recall = torch.empty(T, nc, dtype=torch.float64, device=dev)
+            _lib.check(_lib.lib().yb_map_precision(rec.data_ptr(), seg.data_ptr(), self._gt_count.data_ptr(), nc, T,
+                                                   self._rec_thr.data_ptr(), R, precision.data_ptr(), recall.data_ptr(),
+                                                   ws.data_ptr(), ws_bytes, self._status.data_ptr(), _stream()),
+                       "yb_map_precision")
+            host = torch.cat([precision.reshape(-1), recall.reshape(-1), self._gt_count.double(), seg.double(),
+                              self._status.double()]).cpu().numpy()   # the one synchronisation
+        status = int(host[-1])
+        if status & _lib.MAP_BAD_CLASS:
+            raise IndexError("DetectionMAP: a ground-truth or detection class id is outside [0, num_classes)")
+        if status & _lib.MAP_NMS_FAILED:
+            raise RuntimeError("DetectionMAP: NMS failed for an image (n_keep < 0: bitmask algorithm with too small a "
+                               "workspace)")
+        if status & _lib.MAP_INCONSISTENT:
+            raise RuntimeError("DetectionMAP: a class has more true positives than ground truths")
+        o = 0
+        precision = host[o:o + T * R * nc].reshape(T, R, nc); o += T * R * nc
+        recall = host[o:o + T * nc].reshape(T, nc); o += T * nc
+        n_gt = host[o:o + nc].astype(np.int64); o += nc
+        n_det = np.diff(host[o:o + nc + 1]).astype(np.int64)
+        return dict(summarize_precision(precision, self.iou_thresholds), precision=precision, recall=recall,
+                    n_gt=n_gt, n_det=n_det)
+
+
+def summarize_precision(precision, iou_thresholds):
+    """map, map50 and ap (nc,T) from a (T,R,nc) precision table, as COCOeval.summarize averages it."""
+    def mean(s):
+        s = s[s > -1]
+        return float(np.mean(s)) if s.size else -1.0
+    hit = np.flatnonzero(np.asarray(iou_thresholds) == 0.5)
+    ap = np.where(precision.min(axis=1) > -1, precision.mean(axis=1), -1.0).T   # (nc,T)
+    return {"map": mean(precision), "map50": mean(precision[hit]) if hit.size else None, "ap": ap}
 
 
 # --------------------------------------------------------------------------------------------
