@@ -92,6 +92,16 @@ __device__ __forceinline__ int group_scale(const FilterArgs& a, uint32_t group) 
 // First half: one pass over the logits — maximum m, its first index mi, the runner-up m2 (largest value at any
 // other index).  The caller evaluates sigmoid(m) together with the row's other sigmoids and then calls
 // class_max_ties, which re-evaluates only when another logit can round to the same probability.
+// NaN: torch.max propagates it and returns the index of the first NaN.  A NaN at index 0 stays m (no v > NaN).  Any
+// later NaN fails v > m and reaches the runner-up through max.NaN, which keeps it: m2 is NaN after the pass
+// exactly when a NaN was seen at an index > 0.  Only then the logits are scanned again for the first NaN; m is
+// that NaN (so prob is NaN) and mi its index.  The pass costs what the plain runner-up update cost: one select
+// and one max per logit.
+__device__ __forceinline__ float fmax_nan(float a, float b) {
+    float d;
+    asm("max.NaN.f32 %0, %1, %2;" : "=f"(d) : "f"(a), "f"(b));
+    return d;
+}
 template <typename Load>
 __device__ __forceinline__ void class_max_logit(int nc, Load ld, float& m, float& m2, int& mi) {
     m = ld(0);
@@ -99,8 +109,9 @@ __device__ __forceinline__ void class_max_logit(int nc, Load ld, float& m, float
     mi = 0;
     int c = 1;
     auto step = [&](float v, int idx) {
-        if (v > m) { m2 = m; m = v; mi = idx; }
-        else m2 = v > m2 ? v : m2;
+        const bool gt = v > m;
+        m2 = fmax_nan(m2, gt ? m : v);
+        if (gt) { m = v; mi = idx; }
     };
     for (; c + 8 <= nc; c += 8) {  // 8 independent loads per step
         float v[8];
@@ -110,10 +121,21 @@ __device__ __forceinline__ void class_max_logit(int nc, Load ld, float& m, float
         for (int k = 0; k < 8; ++k) step(v[k], c + k);
     }
     for (; c < nc; ++c) step(ld(c), c);
+    if (m2 != m2) {
+        for (c = 0; c + 1 < nc && ld(c) == ld(c); ++c) {}
+        m = ld(c);
+        mi = c;
+    }
 }
 template <typename Load>
 __device__ __forceinline__ void class_max_ties(int nc, Load ld, float m, float m2, int mi, float& prob, int& id) {
     id = mi;   // prob = sigmoid(m) on entry
+    if (!(prob > 0.0f)) {
+        // NaN: mi is the first NaN.  0: m < -88.73, where expf(-m) overflows; every logit <= m has probability 0
+        // as well, so all of them tie and torch.max returns index 0.
+        if (prob == 0.0f) id = 0;
+        return;
+    }
     if (m <= 5.0f && !(m2 > m - 3.1e-4f)) return;  // 2e-6*(1+e^5) < 3.1e-4: the common case without the exponential
     const float lo = (m <= 14.0f) ? m - 2e-6f * (1.0f + expf(m)) : 13.0f;
     if (!(m2 > lo)) return;  // nothing else is close enough to round to the same probability
@@ -312,7 +334,8 @@ __global__ void __launch_bounds__(kFTile) filter_onepass_kernel(const FilterArgs
     // phase A: objectness test of this thread's row in every tile of the group (the only pass over the column).
     // sigmoid(x) > conf is decided from the logit when x is clearly on one side of logit(conf) (the fp32
     // sigmoid is within a few ulp of the real one, so a margin of obj_margin in x cannot flip the comparison);
-    // rows inside the margin evaluate the reference expression.
+    // rows inside the margin evaluate the reference expression.  The lower test is inclusive: without a margin
+    // (obj_lo = -inf) a row with x = -inf still evaluates sigmoid(-inf) = 0 > conf, which holds for conf < 0.
     float xo[kFMaxGroup];
 #pragma unroll
     for (int k = 0; k < kFMaxGroup; ++k) {
@@ -326,7 +349,7 @@ __global__ void __launch_bounds__(kFTile) filter_onepass_kernel(const FilterArgs
         mybal[k] = 0u;
         if (k < G) {
             bool pass = xo[k] > a.obj_hi;
-            if (!pass && xo[k] > a.obj_lo) pass = sigmoidf_ref(xo[k]) > a.conf;   // :1157,:1166-1167 objectness only
+            if (!pass && xo[k] >= a.obj_lo) pass = sigmoidf_ref(xo[k]) > a.conf;   // :1157,:1166-1167 objectness only
             const unsigned bal = __ballot_sync(0xffffffffu, pass);
             mybal[k] = bal;
             if (lane == 0) s_wcnt[k][warp] = __popc(bal);
