@@ -311,6 +311,57 @@ int yb_map_precision(const yb_map_record* records, const long long* seg, const l
                      int T, const double* recall_thr, int R, double* precision, double* recall, void* ws,
                      size_t ws_bytes, int* status, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * COCO bbox summary (pycocotools 2.0 COCOeval.evaluateImg + accumulate with area ranges and per-(image, category)
+ *   maxDets, no crowd).  Detections, ground truths, classes, status bits and the IoU are yb_map_match's.
+ *   area of a ground truth = (x2-x1)*(y2-y1) of its fp64 corners; of a detection the same on its fp32 corners
+ *     widened to fp64.  An object is outside range a iff area < area_rng[2a] || area > area_rng[2a+1]
+ *     (an area equal to a bound is inside; a NaN area is never outside).
+ * Stage 1, yb_coco_match, once per batch, one CTA per (image, area range):
+ *   per image, class, range a and threshold t (thr = min(iou_thr[t], 1-1e-10)): a ground truth outside range a
+ *     is ignored; each detection in keep order takes the not yet taken ground truth of its class that is best by
+ *     (not ignored first, higher IoU, later index) among those with IoU >= thr (COCO's ignored-last order with its
+ *     `break` and `iou < best: continue`).  Matched to an ignored one -> ignored, else TP; unmatched -> ignored
+ *     when the detection is outside range a, else FP.  A NaN IoU never matches (pycocotools' `iou < best` would let
+ *     it through: the one deliberate departure).
+ *   rank = number of earlier detections of the same image and class (saturating at 65535); COCO's dt[:maxDet] is
+ *     rank < maxDet, since a detection's matching depends only on earlier ones of its image and class.
+ *   records (B, min(max_det,cap)) receive {score, class, rank, TP bit t of tp[a], ignored bit t of ig[a]}; unused
+ *     slots have class -1; tp/ig of ranges >= A are 0.
+ *   gt_count (A, nc) int64 += ground truths per range and class that are not ignored (zeroed by the caller).
+ *   area_rng: HOST array of A <= YB_COCO_MAX_A (lo, hi) pairs; nc * 4 bytes of class counters, the ground truths
+ *   and the thresholds' taken bitmaps must fit one CTA's shared memory (YB_EINVAL otherwise).
+ * Between the stages the CALLER sorts the records as for yb_map_precision (seg (nc+1) as there).
+ * Stage 2, yb_coco_precision, once per evaluation, one CTA per (class, range), the M maxDets side by side:
+ *   a record counts for maxDets[m] iff rank < maxDets[m]; npig = gt_count[a][c]; ignored records count as neither TP
+ *   nor FP; tp, fp cumulative (doubles), rc = tp / npig, pr = tp / (fp + tp + 2^-52);
+ *   precision[t][r][c][a][m] = max of pr over positions with rc >= recall_thr[r] (0 if none),
+ *   recall[t][c][a][m] = rc at the end (0 without detections); both -1 when npig == 0 (COCOeval.eval's layout).
+ *   max_dets: HOST array of 1 <= M <= YB_COCO_MAX_M values in [1, 65535].  recall_thr must be ascending;
+ *   T*R*M*8 + R*8 bytes of shared memory must fit one CTA.
+ *   *status |= YB_MAP_INCONSISTENT when a class and range has more TPs than ground truths.
+ * ---------------------------------------------------------------------------------------- */
+#define YB_COCO_MAX_A 4
+#define YB_COCO_MAX_M 4
+typedef struct yb_coco_record {
+    float score;
+    int32_t cls;      /* -1: unused slot */
+    uint16_t rank;    /* among the image's detections of the same class, saturating */
+    uint16_t pad;
+    uint16_t tp[YB_COCO_MAX_A];   /* bit t: TP at iou_thr[t] in area range a */
+    uint16_t ig[YB_COCO_MAX_A];   /* bit t: ignored at iou_thr[t] in area range a */
+    uint32_t pad2;    /* 32 bytes */
+} yb_coco_record;
+
+int yb_coco_match(const float* boxes, const float* scores, const int64_t* classes, const int64_t* keep,
+                  const int* n_keep, int B, int cap, int max_det, const double* labels, const int* n_gt,
+                  const double* letterbox, int max_gt, int nc, const double* iou_thr, int T,
+                  const double* area_rng, int A, yb_coco_record* records, long long* gt_count, int* status,
+                  void* stream);
+int yb_coco_precision(const yb_coco_record* records, const long long* seg, const long long* gt_count, int nc,
+                      int A, int T, const double* recall_thr, int R, const int* max_dets, int M,
+                      double* precision, double* recall, int* status, void* stream);
+
 /* Per-launch CUDA-event timing for bench.py: when enabled every kernel launch of the library is
  * bracketed by two events on its stream; yb_timing_collect synchronises them, writes
  * "name count total_ms" lines into buf (NUL terminated, truncated to n) and resets. */

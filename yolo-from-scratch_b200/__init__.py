@@ -6,7 +6,8 @@ the reference's own Python function signatures on top (ops.py) and an installer 
 into the reference's `train` module (install.py).
 """
 from . import _lib
-from .ops import (COCO_IOU_THRESHOLDS, COCO_RECALL_THRESHOLDS, DetectionMAP, batched_nms, batched_nms_padded, build_targets, ciou_loss, compute_anchor_iou,
+from .ops import (COCO_AREA_LABELS, COCO_AREA_RANGES, COCO_IOU_THRESHOLDS, COCO_MAX_DETS, COCO_RECALL_THRESHOLDS,
+                  COCODetectionEval, DetectionMAP, format_coco_stats, batched_nms, batched_nms_padded, build_targets, ciou_loss, compute_anchor_iou,
                   decode_predictions, default_anchors, detect_batch, detect_batch_nchw, detections_to_lists, heads_from_nchw, eval_counts, eval_epoch,
                   filter_candidates,
                   loss_forward_backward, nms, nms_retry_overflow, pack_detections, predict_heads,
@@ -20,4 +21,5 @@ __all__ = [
     "PackedLabels", "pack_labels", "pack_labels_host", "eval_counts", "eval_epoch", "yolo_loss_multiscale_nchw",
     "detect_batch_nchw", "heads_from_nchw", "predict_heads", "HotPathGraph", "LAYOUT_BHWAC", "LAYOUT_NCHW", "default_anchors",
     "DetectionMAP", "COCO_IOU_THRESHOLDS", "COCO_RECALL_THRESHOLDS",
+    "COCODetectionEval", "COCO_AREA_RANGES", "COCO_AREA_LABELS", "COCO_MAX_DETS", "format_coco_stats",
 ]

@@ -15,6 +15,7 @@ NMS_GRAPH, NMS_BITMASK = 0, 1
 LAYOUT_BHWAC, LAYOUT_NCHW = 0, 1
 MAP_MAX_T, MAP_MAX_GT = 16, 4096
 MAP_BAD_CLASS, MAP_NMS_FAILED, MAP_INCONSISTENT = 1, 2, 4
+COCO_MAX_A, COCO_MAX_M = 4, 4
 LIB_NAME = "libyolo_b200.so"
 LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), LIB_NAME)
 
@@ -83,6 +84,11 @@ SIGNATURES = {
     "yb_map_workspace_bytes": (c_size_t, [c_longlong, c_longlong, c_int]),
     "yb_map_precision": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p,
                                  c_void_p, c_size_t, c_void_p, c_void_p]),
+    "yb_coco_match": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
+                              c_void_p, c_int, c_int, c_void_p, c_int, POINTER(c_double), c_int, c_void_p, c_void_p,
+                              c_void_p, c_void_p]),
+    "yb_coco_precision": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, POINTER(c_int),
+                                  c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
 }
 
 _lib = None

@@ -9,23 +9,11 @@
 // position, then the suffix maximum gives the (T,R,nc) precision table and the (T,nc) recall table.
 // Every fp64 expression is the oracle's (oracle/map_ref.py) operation for operation (-fmad=false).
 #include "yb_common.cuh"
+#include "yb_iou.cuh"
 
 namespace yb {
 
 constexpr int kPrecThreads = 256;
-
-struct GtBox {
-    double x1, y1, x2, y2;
-};
-
-// compute_iou_corners (train.py:1064-1084): 0 when the union is not positive
-__device__ __forceinline__ double corner_iou(const GtBox& a, const GtBox& b) {
-    const double iw = fmax(0.0, fmin(a.x2, b.x2) - fmax(a.x1, b.x1));
-    const double ih = fmax(0.0, fmin(a.y2, b.y2) - fmax(a.y1, b.y1));
-    const double inter = iw * ih;
-    const double uni = (a.x2 - a.x1) * (a.y2 - a.y1) + (b.x2 - b.x1) * (b.y2 - b.y1) - inter;
-    return uni > 0.0 ? inter / uni : 0.0;
-}
 
 struct MatchArgs {
     const float4* boxes;

@@ -99,37 +99,59 @@ def _make_predict(train_module):
     return predict, predict_batch
 
 
+def _evaluate_dataset(train_module, metric, model, dataset, device, num_classes, conf_threshold, iou_threshold,
+                      batch_size):
+    """Feed `metric` (DetectionMAP or COCODetectionEval) the detections of `model` on `dataset` (its imgs and labels
+    lists) batch by batch and return metric.compute().  Images are loaded and letterboxed by the module's own Image
+    and letterbox_resize, as predict() does (train.py:1134-1138)."""
+    import numpy as np
+    import torch
+    g = train_module.__dict__
+    model.eval()
+    img_size = model.img_size
+    n = len(dataset.imgs)
+    with torch.no_grad():
+        for i0 in range(0, n, batch_size):
+            imgs, letterbox, labels = [], [], []
+            for i in range(i0, min(i0 + batch_size, n)):
+                pil_img = g["Image"].open(dataset.imgs[i]).convert("RGB")
+                orig_w, orig_h = pil_img.size
+                pil_img, scale, pad_top, pad_left = g["letterbox_resize"](pil_img, img_size)
+                imgs.append(torch.from_numpy(np.array(pil_img)).permute(2, 0, 1).float() / 255.0)
+                letterbox.append((orig_w, orig_h, scale, pad_top, pad_left))
+                labels.append(_read_labels(train_module, dataset.labels[i]))
+            preds = model(torch.stack(imgs).to(device))
+            det = ops.detect_batch(list(preds), model.anchors, img_size, num_classes, conf_threshold, iou_threshold,
+                                   letterbox=[lb[2:] for lb in letterbox])
+            metric.update(det, ops.pack_labels(labels, img_size, letterbox))
+    return metric.compute()
+
+
 def _make_evaluate_map(train_module):
     """`evaluate_map`, a name the reference does not have: COCO-style mAP of a model over a YOLODataset's images
-    and label files (ops.DetectionMAP).  Images are loaded and letterboxed by the module's own Image and
-    letterbox_resize, as predict() does (train.py:1134-1138)."""
+    and label files (ops.DetectionMAP)."""
     def evaluate_map(model, dataset, device, num_classes=1, conf_threshold=0.001, iou_threshold=0.4, batch_size=8,
                      max_det=300):
         """mAP@[.5:.95] / mAP@0.5 of `model` on `dataset` (its imgs and labels lists).  Returns DetectionMAP.compute()'s
         dict: map, map50, ap (nc,T), precision (T,R,nc), recall (T,nc), n_gt (nc), n_det (nc)."""
-        import numpy as np
-        import torch
-        g = train_module.__dict__
-        model.eval()
-        img_size = model.img_size
         metric = ops.DetectionMAP(num_classes, max_det=max_det)
-        n = len(dataset.imgs)
-        with torch.no_grad():
-            for i0 in range(0, n, batch_size):
-                imgs, letterbox, labels = [], [], []
-                for i in range(i0, min(i0 + batch_size, n)):
-                    pil_img = g["Image"].open(dataset.imgs[i]).convert("RGB")
-                    orig_w, orig_h = pil_img.size
-                    pil_img, scale, pad_top, pad_left = g["letterbox_resize"](pil_img, img_size)
-                    imgs.append(torch.from_numpy(np.array(pil_img)).permute(2, 0, 1).float() / 255.0)
-                    letterbox.append((orig_w, orig_h, scale, pad_top, pad_left))
-                    labels.append(_read_labels(train_module, dataset.labels[i]))
-                preds = model(torch.stack(imgs).to(device))
-                det = ops.detect_batch(list(preds), model.anchors, img_size, num_classes, conf_threshold, iou_threshold,
-                                       letterbox=[lb[2:] for lb in letterbox])
-                metric.update(det, ops.pack_labels(labels, img_size, letterbox))
-        return metric.compute()
+        return _evaluate_dataset(train_module, metric, model, dataset, device, num_classes, conf_threshold,
+                                 iou_threshold, batch_size)
     return evaluate_map
+
+
+def _make_evaluate_coco(train_module):
+    """`evaluate_coco`, a name the reference does not have: COCO's twelve bbox stats of a model over a YOLODataset's
+    images and label files (ops.COCODetectionEval)."""
+    def evaluate_coco(model, dataset, device, num_classes=1, conf_threshold=0.001, iou_threshold=0.4, batch_size=8,
+                      max_det=300, max_dets=ops.COCO_MAX_DETS):
+        """COCO's bbox summary of `model` on `dataset` (its imgs and labels lists).  Returns
+        COCODetectionEval.compute()'s dict: stats (12,), precision (T,R,nc,A,M), recall (T,nc,A,M), n_gt (nc,A),
+        n_det (nc), ap (nc,T), map, map50; ops.format_coco_stats(stats) gives pycocotools' printed lines."""
+        metric = ops.COCODetectionEval(num_classes, max_det=max_det, max_dets=max_dets)
+        return _evaluate_dataset(train_module, metric, model, dataset, device, num_classes, conf_threshold,
+                                 iou_threshold, batch_size)
+    return evaluate_coco
 
 
 def channels_last_heads(model):
@@ -179,8 +201,8 @@ def install(train_module, patch_torchvision=False, patch_dataset=True, patch_eva
     channels_last (default: environment YOLO_B200_CHANNELS_LAST=1) makes every `train.YOLO` built afterwards
     run in NHWC, so that the head layout conversion of train.py:608-609 costs nothing (channels_last_heads).
     patch_eval also swaps `eval_epoch` (SURVEY 8f-1: its per-anchor python loop becomes one kernel);
-    patch_predict swaps `predict` and adds `predict_batch` (SURVEY 8f-3); `evaluate_map` (COCO-style mAP, a name
-    the reference does not have) is always added; patch_torchvision additionally
+    patch_predict swaps `predict` and adds `predict_batch` (SURVEY 8f-3); `evaluate_map` (COCO-style mAP) and
+    `evaluate_coco` (COCO's twelve bbox stats), names the reference does not have, are always added; patch_torchvision additionally
     rebinds torchvision.ops.batched_nms process-wide (off by default: predict no longer needs it)."""
     if getattr(train_module, _MARK, False):
         return train_module
@@ -197,6 +219,9 @@ def install(train_module, patch_torchvision=False, patch_dataset=True, patch_eva
     if not hasattr(train_module, "evaluate_map"):
         saved["evaluate_map"] = None
         train_module.evaluate_map = _make_evaluate_map(train_module)
+    if not hasattr(train_module, "evaluate_coco"):
+        saved["evaluate_coco"] = None
+        train_module.evaluate_coco = _make_evaluate_coco(train_module)
     if patch_dataset and hasattr(train_module, "YOLODataset"):
         cls = train_module.YOLODataset
         saved["YOLODataset.__getitem__"] = cls.__getitem__
@@ -233,6 +258,8 @@ def uninstall(train_module):
             del train_module.predict_batch
     if "evaluate_map" in saved:
         del train_module.evaluate_map
+    if "evaluate_coco" in saved:
+        del train_module.evaluate_coco
     if "YOLODataset.__getitem__" in saved:
         train_module.YOLODataset.__getitem__ = saved["YOLODataset.__getitem__"]
         train_module.YOLODataset.compute_anchor_iou = saved["YOLODataset.compute_anchor_iou"]

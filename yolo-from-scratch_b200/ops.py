@@ -827,6 +827,34 @@ COCO_IOU_THRESHOLDS = tuple(np.linspace(0.5, 0.95, 10).tolist())      # COCOeval
 COCO_RECALL_THRESHOLDS = tuple(np.linspace(0.0, 1.0, 101).tolist())   # COCOeval Params.recThrs
 
 
+def _sort_records(rec, nc):
+    """Records (N, words) int32 whose first two words are (score f32, class i32) -> (records sorted by class
+    ascending, then score descending, stably; seg (nc+1) int64: class c is rows [seg[c], seg[c+1])).  Unused slots
+    (class -1) go last."""
+    # key = class << 32 | order-reversed score bits: ascending key = class ascending, score descending;
+    # the stable sort keeps image and keep order among equal keys.
+    score = rec[:, 0].view(torch.float32) + 0.0          # -0.0 -> +0.0: equal scores must tie
+    bits = score.view(torch.int32).to(torch.int64)
+    asc = bits ^ ((bits >> 31) & 0x7FFFFFFF)              # monotone in the float value
+    cls = rec[:, 1].to(torch.int64)
+    key = torch.where(cls >= 0, cls, nc) * (1 << 32) + (0x7FFFFFFF - asc)
+    key, order = torch.sort(key, stable=True)
+    rec = rec.index_select(0, order).contiguous()
+    seg = torch.searchsorted(key, torch.arange(nc + 1, dtype=torch.int64, device=rec.device) * (1 << 32))
+    return rec, seg
+
+
+def _raise_status(status, who):
+    """The errors of the mAP kernels' status bits (YB_MAP_*)."""
+    if status & _lib.MAP_BAD_CLASS:
+        raise IndexError(f"{who}: a ground-truth or detection class id is outside [0, num_classes)")
+    if status & _lib.MAP_NMS_FAILED:
+        raise RuntimeError(f"{who}: NMS failed for an image (n_keep < 0: bitmask algorithm with too small a "
+                           "workspace)")
+    if status & _lib.MAP_INCONSISTENT:
+        raise RuntimeError(f"{who}: a class has more true positives than ground truths")
+
+
 class DetectionMAP:
     """mAP@[.5:.95] and mAP@0.5 of the kept detections of `detect_batch`, accumulated over batches on the device.
     COCO's bbox protocol (evaluateImg + accumulate, area range "all", no crowd) with one overall cap of `max_det`
@@ -895,16 +923,7 @@ class DetectionMAP:
         dev = self.device
         with torch.cuda.device(dev):
             rec = torch.cat(self._records) if self._records else torch.empty(0, 3, dtype=torch.int32, device=dev)
-            # key = class << 32 | order-reversed score bits: ascending key = class ascending, score descending;
-            # the stable sort keeps image and keep order among equal keys.  Unused slots (class -1) go last.
-            score = rec[:, 0].view(torch.float32) + 0.0          # -0.0 -> +0.0: equal scores must tie
-            bits = score.view(torch.int32).to(torch.int64)
-            asc = bits ^ ((bits >> 31) & 0x7FFFFFFF)              # monotone in the float value
-            cls = rec[:, 1].to(torch.int64)
-            key = torch.where(cls >= 0, cls, nc) * (1 << 32) + (0x7FFFFFFF - asc)
-            key, order = torch.sort(key, stable=True)
-            rec = rec.index_select(0, order).contiguous()
-            seg = torch.searchsorted(key, torch.arange(nc + 1, dtype=torch.int64, device=dev) * (1 << 32))
+            rec, seg = _sort_records(rec, nc)
             n = rec.shape[0]
             ws_bytes = _lib.lib().yb_map_workspace_bytes(n, self._gt_total, T)
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
@@ -916,14 +935,7 @@ class DetectionMAP:
                        "yb_map_precision")
             host = torch.cat([precision.reshape(-1), recall.reshape(-1), self._gt_count.double(), seg.double(),
                               self._status.double()]).cpu().numpy()   # the one synchronisation
-        status = int(host[-1])
-        if status & _lib.MAP_BAD_CLASS:
-            raise IndexError("DetectionMAP: a ground-truth or detection class id is outside [0, num_classes)")
-        if status & _lib.MAP_NMS_FAILED:
-            raise RuntimeError("DetectionMAP: NMS failed for an image (n_keep < 0: bitmask algorithm with too small a "
-                               "workspace)")
-        if status & _lib.MAP_INCONSISTENT:
-            raise RuntimeError("DetectionMAP: a class has more true positives than ground truths")
+        _raise_status(int(host[-1]), "DetectionMAP")
         o = 0
         precision = host[o:o + T * R * nc].reshape(T, R, nc); o += T * R * nc
         recall = host[o:o + T * nc].reshape(T, nc); o += T * nc
@@ -941,6 +953,152 @@ def summarize_precision(precision, iou_thresholds):
     hit = np.flatnonzero(np.asarray(iou_thresholds) == 0.5)
     ap = np.where(precision.min(axis=1) > -1, precision.mean(axis=1), -1.0).T   # (nc,T)
     return {"map": mean(precision), "map50": mean(precision[hit]) if hit.size else None, "ap": ap}
+
+
+COCO_AREA_RANGES = ((0.0, 1e5 ** 2), (0.0, 32.0 ** 2), (32.0 ** 2, 96.0 ** 2), (96.0 ** 2, 1e5 ** 2))   # Params.areaRng
+COCO_AREA_LABELS = ("all", "small", "medium", "large")                                                # Params.areaRngLbl
+COCO_MAX_DETS = (1, 10, 100)                                                                          # Params.maxDets
+
+
+class COCODetectionEval:
+    """COCO's bbox summary of the kept detections of `detect_batch`, accumulated over batches on the device: the
+    twelve numbers pycocotools prints (AP, AP50, AP75, AP_S/M/L, AR@maxDets, AR_S/M/L) and COCOeval.eval's
+    precision (T,R,nc,A,M) and recall (T,nc,A,M) tables.  COCO's protocol (evaluateImg + accumulate + summarize,
+    area ranges all/small/medium/large, per-(image, category) maxDets, no crowd) on the first `max_det` kept
+    detections of each image; include/yolo_b200.h states the semantics.  A NaN IoU never matches, where
+    pycocotools' `iou < best` test would let it through.
+
+    max_det caps the detections of an image (the records kept per image, YOLOv5's NMS cap); max_dets are COCO's
+    three per-(image, category) limits.  stats[0] (AP) reads maxDets = 100 literally, as pycocotools does, so it is
+    -1 when max_dets lacks 100; every other stat uses max_dets[0..2].
+
+    update(det, labels) enqueues one matching kernel per batch and keeps its records; it never synchronises.
+    compute() sorts the records once, runs the precision kernel and synchronises once."""
+
+    def __init__(self, num_classes, iou_thresholds=COCO_IOU_THRESHOLDS, recall_thresholds=COCO_RECALL_THRESHOLDS,
+                 max_det=300, max_dets=COCO_MAX_DETS):
+        self.nc = int(num_classes)
+        self.iou_thresholds = np.asarray(iou_thresholds, dtype=np.float64).reshape(-1)
+        self.recall_thresholds = np.asarray(recall_thresholds, dtype=np.float64).reshape(-1)
+        self.max_det = int(max_det)
+        self.max_dets = tuple(int(m) for m in max_dets)
+        self.area_ranges = np.asarray(COCO_AREA_RANGES, dtype=np.float64)
+        if self.nc < 1:
+            raise ValueError("num_classes must be >= 1")
+        if not 1 <= len(self.iou_thresholds) <= _lib.MAP_MAX_T:
+            raise ValueError(f"1..{_lib.MAP_MAX_T} IoU thresholds supported, got {len(self.iou_thresholds)}")
+        if len(self.recall_thresholds) < 1 or not np.all(np.diff(self.recall_thresholds) >= 0):
+            raise ValueError("recall_thresholds must be a non-empty ascending sequence")
+        if self.max_det < 0:
+            raise ValueError("max_det must be >= 0")
+        if len(self.max_dets) != 3 or not all(1 <= m <= 65535 for m in self.max_dets):
+            raise ValueError(f"max_dets must be three values in [1, 65535], got {max_dets}")
+        self.device = _device()
+        with torch.cuda.device(self.device):
+            self._iou_thr = torch.tensor(self.iou_thresholds, dtype=torch.float64, device=self.device)
+            self._rec_thr = torch.tensor(self.recall_thresholds, dtype=torch.float64, device=self.device)
+            self._gt_count = torch.zeros(len(self.area_ranges), self.nc, dtype=torch.int64, device=self.device)
+            self._status = torch.zeros(1, dtype=torch.int32, device=self.device)
+        self._rng_host = (ctypes.c_double * self.area_ranges.size)(*self.area_ranges.reshape(-1).tolist())
+        self._md_host = (ctypes.c_int * len(self.max_dets))(*self.max_dets)
+        self.reset()
+
+    def reset(self):
+        """Forget every batch seen so far."""
+        self._records = []
+        with torch.cuda.device(self.device):
+            self._gt_count.zero_()
+            self._status.zero_()
+
+    def update(self, det, labels: PackedLabels):
+        """Match one batch: `det` is a detect_batch result (letterbox reversed, original-image pixels) and `labels`
+        the batch's PackedLabels (labels normalised to the original image, letterbox rows [orig_w, orig_h, ...])."""
+        boxes, keep = det["boxes"], det["keep"]
+        if boxes.device != self.device:
+            raise ValueError(f"detections on {boxes.device}, COCODetectionEval on {self.device}")
+        B, cap = boxes.shape[0], boxes.shape[1]
+        if labels.labels.shape[0] != B or labels.labels.device != self.device:
+            raise ValueError("labels and detections disagree on the batch size or the device")
+        if labels.max_gt > _lib.MAP_MAX_GT:
+            raise ValueError(f"at most {_lib.MAP_MAX_GT} ground truths per image, got max_gt={labels.max_gt}")
+        slots = min(self.max_det, cap)
+        with torch.cuda.device(self.device):
+            rec = torch.empty(B * slots, 8, dtype=torch.int32, device=self.device)   # yb_coco_record, 32 bytes
+            _lib.check(_lib.lib().yb_coco_match(
+                boxes.data_ptr(), det["scores"].data_ptr(), det["classes"].data_ptr(), keep.data_ptr(),
+                det["n_keep"].data_ptr(), B, cap, self.max_det, labels.labels.data_ptr(), labels.n_gt.data_ptr(),
+                labels.letterbox.data_ptr(), labels.max_gt, self.nc, self._iou_thr.data_ptr(), len(self.iou_thresholds),
+                self._rng_host, len(self.area_ranges), rec.data_ptr(), self._gt_count.data_ptr(),
+                self._status.data_ptr(), _stream()), "yb_coco_match")
+        self._records.append(rec)
+
+    def compute(self):
+        """{stats (12,), precision (T,R,nc,A,M), recall (T,nc,A,M), n_gt (nc,A), n_det (nc), and ap (nc,T), map,
+        map50 at area "all" and max_dets[-1]} on the host (float64 / int64).  Entries of a (class, area) without
+        ground truth are -1; stats are pycocotools' _summarizeDets, map / map50 DetectionMAP's means.  n_gt counts
+        the ground truths inside each area range, n_det the records of each class (at most max_det per image)."""
+        T, R, nc = len(self.iou_thresholds), len(self.recall_thresholds), self.nc
+        A, M = len(self.area_ranges), len(self.max_dets)
+        dev = self.device
+        with torch.cuda.device(dev):
+            rec = torch.cat(self._records) if self._records else torch.empty(0, 8, dtype=torch.int32, device=dev)
+            rec, seg = _sort_records(rec, nc)
+            precision = torch.empty(T, R, nc, A, M, dtype=torch.float64, device=dev)
+            recall = torch.empty(T, nc, A, M, dtype=torch.float64, device=dev)
+            _lib.check(_lib.lib().yb_coco_precision(rec.data_ptr(), seg.data_ptr(), self._gt_count.data_ptr(), nc, A, T,
+                                                    self._rec_thr.data_ptr(), R, self._md_host, M, precision.data_ptr(),
+                                                    recall.data_ptr(), self._status.data_ptr(), _stream()),
+                       "yb_coco_precision")
+            host = torch.cat([precision.reshape(-1), recall.reshape(-1), self._gt_count.reshape(-1).double(),
+                              seg.double(), self._status.double()]).cpu().numpy()   # the one synchronisation
+        _raise_status(int(host[-1]), "COCODetectionEval")
+        o = 0
+        precision = host[o:o + T * R * nc * A * M].reshape(T, R, nc, A, M); o += T * R * nc * A * M
+        recall = host[o:o + T * nc * A * M].reshape(T, nc, A, M); o += T * nc * A * M
+        n_gt = host[o:o + A * nc].reshape(A, nc).T.astype(np.int64); o += A * nc
+        n_det = np.diff(host[o:o + nc + 1]).astype(np.int64)
+        stats = summarize_coco(precision, recall, self.iou_thresholds, self.max_dets)
+        return dict(summarize_precision(precision[..., 0, M - 1], self.iou_thresholds), stats=stats,
+                    precision=precision, recall=recall, n_gt=n_gt, n_det=n_det)
+
+
+def _coco_mean(s):
+    s = s[s > -1]
+    return float(np.mean(s)) if s.size else -1.0
+
+
+def summarize_coco(precision, recall, iou_thresholds, max_dets, area_labels=COCO_AREA_LABELS):
+    """pycocotools' COCOeval.summarize / _summarizeDets on COCOeval.eval's tables: the 12 stats.  Thresholds are
+    selected by exact float equality and maxDets by value, as there; stats[0] reads maxDets = 100 literally."""
+    iou_thresholds = np.asarray(iou_thresholds)
+
+    def summ(ap, iou_thr=None, area="all", md=100):
+        aind = [i for i, lbl in enumerate(area_labels) if lbl == area]
+        mind = [i for i, m in enumerate(max_dets) if m == md]
+        s = precision if ap else recall
+        if iou_thr is not None:
+            s = s[np.where(iou_thr == iou_thresholds)[0]]
+        s = s[:, :, :, aind, mind] if ap else s[:, :, aind, mind]
+        return _coco_mean(s)
+
+    md = max_dets
+    return np.array([summ(1), summ(1, .5, md=md[2]), summ(1, .75, md=md[2]), summ(1, area="small", md=md[2]),
+                     summ(1, area="medium", md=md[2]), summ(1, area="large", md=md[2]), summ(0, md=md[0]),
+                     summ(0, md=md[1]), summ(0, md=md[2]), summ(0, area="small", md=md[2]),
+                     summ(0, area="medium", md=md[2]), summ(0, area="large", md=md[2])])
+
+
+def format_coco_stats(stats, iou_thresholds=COCO_IOU_THRESHOLDS, max_dets=COCO_MAX_DETS):
+    """The twelve lines pycocotools' summarize() prints for `stats` (COCODetectionEval.compute()["stats"])."""
+    line = " {:<18} {} @[ IoU={:<9} | area={:>6s} | maxDets={:>3d} ] = {:0.3f}"
+    every = "{:0.2f}:{:0.2f}".format(iou_thresholds[0], iou_thresholds[-1])
+    md = max_dets
+    rows = [(1, None, "all", 100), (1, .5, "all", md[2]), (1, .75, "all", md[2]), (1, None, "small", md[2]),
+            (1, None, "medium", md[2]), (1, None, "large", md[2]), (0, None, "all", md[0]), (0, None, "all", md[1]),
+            (0, None, "all", md[2]), (0, None, "small", md[2]), (0, None, "medium", md[2]), (0, None, "large", md[2])]
+    return [line.format("Average Precision" if ap else "Average Recall", "(AP)" if ap else "(AR)",
+                        every if thr is None else "{:0.2f}".format(thr), area, m, float(v))
+            for (ap, thr, area, m), v in zip(rows, stats)]
 
 
 # --------------------------------------------------------------------------------------------
