@@ -18,7 +18,8 @@
  *   - return value 0 = success, otherwise a cudaError_t or a negative YB_E* code;
  *     yb_last_error() returns a thread-local, human readable message for the last failure;
  *   - head tensors use the model-output layout of train.py:608-609: contiguous fp32
- *     (B, H, W, A, 5+nc), row = [tx, ty, tw, th, obj, cls...] raw logits;
+ *     (B, H, W, A, 5+nc), row = [tx, ty, tw, th, obj, cls...] raw logits; the loss, decode and
+ *     filter entry points also take bf16 or fp16 heads (YB_DTYPE_*, below);
  *   - `anchors` are fp32 (A,2) = [w,h] in pixels (train.py:372-374, 386-388);
  *   - tensors must be 16-byte aligned (every torch allocation is).
  */
@@ -43,6 +44,15 @@ extern "C" {
 #define YB_LAYOUT_BHWAC 0
 #define YB_LAYOUT_NCHW 1
 
+/* Element type of head tensors (pred / grad / decode output).  A zero-filled descriptor means fp32.
+ * Half heads are read as they are: every value widens exactly to fp32 and all arithmetic is the fp32
+ * path's, so every result equals the fp32 path on the upcast heads.  Half results (decode output,
+ * loss gradients) are the fp32 values rounded to nearest even (__float2bfloat16_rn / __float2half_rn;
+ * overflow in fp16 gives +-inf).  Targets, anchors, candidates and boxes stay fp32. */
+#define YB_DTYPE_F32 0
+#define YB_DTYPE_BF16 1
+#define YB_DTYPE_F16 2
+
 #define YB_EINVAL (-1)   /* bad argument (shape, null pointer, alignment) */
 #define YB_EWORKSPACE (-2) /* workspace too small */
 
@@ -63,6 +73,13 @@ int yb_decode_fwd(const float* pred, const float* anchors, float* out,
                   int B, int H, int W, int A, int nc, float img_size, void* stream);
 int yb_decode_bwd(const float* pred, const float* anchors, const float* grad_out, float* grad_in,
                   int B, int H, int W, int A, int nc, float img_size, void* stream);
+/* The same on heads of element type `dtype` (YB_DTYPE_*): pred, out, grad_out and grad_in all have that
+ * type.  out = round(fp32 decode of the widened pred); grad_in = round(fp32 vector-Jacobian product of the
+ * widened pred and grad_out).  yb_decode_fwd / yb_decode_bwd are the fp32 case. */
+int yb_decode_fwd_t(const void* pred, const float* anchors, void* out, int B, int H, int W, int A, int nc,
+                    float img_size, int dtype, void* stream);
+int yb_decode_bwd_t(const void* pred, const float* anchors, const void* grad_out, void* grad_in, int B, int H,
+                    int W, int A, int nc, float img_size, int dtype, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * a-2  ciou_loss(pred_boxes, target_boxes, eps=1e-7)                    train.py:634-710
@@ -114,7 +131,23 @@ typedef struct yb_loss_desc {
     const float* anchors[YB_MAX_SCALES];
     float* grad[YB_MAX_SCALES];     /* nullable: forward only (torch.no_grad callers) */
     int layout;                     /* YB_LAYOUT_* of pred and grad */
+    int dtype;                      /* YB_DTYPE_* of pred and grad (tgt stays fp32) */
 } yb_loss_desc;
+
+/* Half heads (dtype bf16 / fp16).  The gradient of `total` depends on its upstream gradient s, which is
+ * known only at backward, and s has to be applied BEFORE the rounding to half (fp16 objectness gradients,
+ * ~coef/(B*H*W*A), are subnormal or zero in fp16 until a GradScaler's s lifts them).  So stage 1 writes
+ * no dense gradient for half heads (grad[] is ignored there): it keeps the fp32 objectness gradient, one
+ * float per row, and the positive lists in `ws` (the workspace is rows*4 bytes larger than for fp32).
+ * yb_loss_grad_emit then writes grad[s] completely, after stage 2, from the same workspace and the
+ * same reduced partials (max_gt: the value given to yb_loss_partials_sparse, or -1 after yb_loss_partials):
+ *   grad = round(s == 1 ? G : round_f32(G * s)),  s = *grad_scale (device fp32),
+ * where G is the fp32 path's gradient for upstream 1 (positive rows: g, then g * coef/P, each rounded
+ * to fp32) and round() rounds to nearest even in the head dtype — exactly what the fp32 path followed by
+ * yb_scale_inplace and a cast to the head dtype gives, for every s.  It may be called again (the
+ * workspace is read only) and is capturable; *grad_scale is read when the kernels run. */
+int yb_loss_grad_emit(const yb_loss_desc* d, const double* partials /* S*4, reduced */,
+                      const float* grad_scale, int max_gt, void* ws, size_t ws_bytes, void* stream);
 
 size_t yb_loss_workspace_bytes(const yb_loss_desc* d);
 int yb_loss_partials(const yb_loss_desc* d, double* partials /* S*4 */,
@@ -187,6 +220,7 @@ typedef struct yb_heads_desc {
     const float* pred[YB_MAX_SCALES];
     const float* anchors[YB_MAX_SCALES];
     int layout;                     /* YB_LAYOUT_* of pred (filter: both; decode/eval: BHWAC only) */
+    int dtype;                      /* YB_DTYPE_* of pred (filter: all three; eval: fp32 only) */
 } yb_heads_desc;
 
 size_t yb_filter_workspace_bytes(const yb_heads_desc* d);

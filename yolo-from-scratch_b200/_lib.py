@@ -13,6 +13,7 @@ MAX_SCALES = 4
 MAX_ANCHORS = 8
 NMS_GRAPH, NMS_BITMASK = 0, 1
 LAYOUT_BHWAC, LAYOUT_NCHW = 0, 1
+DTYPE_F32, DTYPE_BF16, DTYPE_F16 = 0, 1, 2
 MAP_MAX_T, MAP_MAX_GT = 16, 4096
 MAP_BAD_CLASS, MAP_NMS_FAILED, MAP_INCONSISTENT = 1, 2, 4
 COCO_MAX_A, COCO_MAX_M = 4, 4
@@ -30,7 +31,7 @@ class LossDesc(Structure):
         ("coef_obj", c_float * MAX_SCALES), ("coef_cls", c_float * MAX_SCALES),
         ("pred", c_void_p * MAX_SCALES), ("tgt", c_void_p * MAX_SCALES),
         ("anchors", c_void_p * MAX_SCALES), ("grad", c_void_p * MAX_SCALES),
-        ("layout", c_int),
+        ("layout", c_int), ("dtype", c_int),
     ]
 
 
@@ -40,7 +41,7 @@ class HeadsDesc(Structure):
         ("S", c_int), ("B", c_int), ("A", c_int), ("nc", c_int),
         ("H", c_int * MAX_SCALES), ("W", c_int * MAX_SCALES), ("img_size", c_float),
         ("pred", c_void_p * MAX_SCALES), ("anchors", c_void_p * MAX_SCALES),
-        ("layout", c_int),
+        ("layout", c_int), ("dtype", c_int),
     ]
 
 
@@ -53,6 +54,10 @@ SIGNATURES = {
     "yb_timing_collect": (c_int, [c_char_p, c_size_t]),
     "yb_decode_fwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p]),
     "yb_decode_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p]),
+    "yb_decode_fwd_t": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_float, c_int,
+                                c_void_p]),
+    "yb_decode_bwd_t": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_float,
+                                c_int, c_void_p]),
     "yb_ciou_scratch_bytes": (c_size_t, [c_longlong]),
     "yb_ciou_fwd_bwd": (c_int, [c_void_p, c_void_p, c_longlong, c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "yb_loss_workspace_bytes": (c_size_t, [POINTER(LossDesc)]),
@@ -61,6 +66,7 @@ SIGNATURES = {
     "yb_loss_sparse_workspace_bytes": (c_size_t, [POINTER(LossDesc), c_int]),
     "yb_loss_partials_sparse": (c_int, [POINTER(LossDesc), c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
                                         c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "yb_loss_grad_emit": (c_int, [POINTER(LossDesc), c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
     "yb_scale_inplace": (c_int, [c_void_p, c_longlong, c_void_p, c_void_p]),
     "yb_anchor_iou": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "yb_build_targets": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, POINTER(c_void_p), c_int, c_int, c_int,

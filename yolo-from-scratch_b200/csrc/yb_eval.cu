@@ -127,6 +127,7 @@ extern "C" int yb_eval_counts(const yb_heads_desc* d, const float* const* target
     a.conf = conf_threshold;
     a.counts = reinterpret_cast<unsigned long long*>(counts3);
     unsigned long long total = 0;
+    YB_CHECK_ARG(d->dtype == YB_DTYPE_F32, "eval_counts: heads must be fp32");
     for (int s = 0; s < d->S; ++s) {
         YB_CHECK_ARG(d->H[s] > 0 && d->W[s] > 0 && d->pred[s] && targets_host[s] && d->anchors[s],
                      "eval_counts: bad scale %d", s);

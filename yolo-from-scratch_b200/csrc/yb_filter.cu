@@ -27,7 +27,7 @@ constexpr int kFTile = 128;    // rows per tile == threads per CTA
 constexpr int kFMaxGroup = 8;  // tiles per CTA, at most
 
 struct FilterScale {
-    const float* pred;
+    const void* pred;      // element type T of the kernels
     const float* anchors;
     uint32_t rows;         // rows per image at this scale = H*W*A
     uint32_t hw;           // H*W
@@ -273,9 +273,10 @@ __device__ __forceinline__ void filter_emit_row(const FilterArgs& a, const Filte
 //               loads per tile), then streams the dense tiles (a quarter of the rows or more pass) through ONE
 //               shared-memory tile buffer, so that five CTAs per SM keep >200 KB of bulk copies in flight.  When the
 //               batch has been dense so far (lb_seen) the first copy starts before phase A.
-template <bool LONG>
+template <bool LONG, typename T>
 __global__ void __launch_bounds__(kFTile) filter_onepass_kernel(const FilterArgs a) {
     extern __shared__ __align__(128) float s_tile[];
+    T* s_t = reinterpret_cast<T*>(s_tile);   // staged rows
     __shared__ __align__(8) uint64_t s_bar[2];
     __shared__ int s_wcnt[kFMaxGroup][kFTile / 32];
     __shared__ int s_prefix, s_hint;
@@ -306,28 +307,30 @@ __global__ void __launch_bounds__(kFTile) filter_onepass_kernel(const FilterArgs
     const int G = (int)min((uint32_t)a.G, ntiles - tile0);  // tiles of this group
     const uint32_t row0 = tile0 * kFTile;
     const uint32_t nrows = min((uint32_t)(G * kFTile), L.rows - row0);
-    const size_t base = ((size_t)b * L.rows + row0) * a.row;  // float offset of the group
-    const float* g = L.pred + base;
+    const size_t base = ((size_t)b * L.rows + row0) * a.row;  // element offset of the group
+    const T* g = reinterpret_cast<const T*>(L.pred) + base;
     unsigned long long* st = a.lb_state + (size_t)b * a.groups_per_img;
-    const uint32_t tile_fl = (uint32_t)kFTile * a.row;        // floats of a full tile
+    const uint32_t tile_fl = (uint32_t)kFTile * a.row;        // elements of a full tile
+    constexpr uint32_t VM = kVec<T> - 1u;                     // 16-byte alignment mask, in elements
+    constexpr uint32_t ES = sizeof(T);
 
     // tile k of the group as a bulk-copy job: rows, floats, source, 16-byte alignment
     auto tile_rows = [&](int k) { return min((uint32_t)kFTile, nrows - (uint32_t)k * kFTile); };
-    auto tile_bulk_ok = [&](int k) { return ((base + (size_t)k * tile_fl) & 3) == 0 && ((tile_rows(k) * a.row) & 3u) == 0; };
+    auto tile_bulk_ok = [&](int k) { return ((base + (size_t)k * tile_fl) & VM) == 0 && ((tile_rows(k) * a.row) & VM) == 0; };
     int pending = -1;               // tile whose bulk copy is in flight / has landed in the buffer (all threads agree)
     uint32_t parity = 0u;
 
     if (!LONG) {   // the whole group up front
         const uint32_t nfl = nrows * a.row;
-        if ((base & 3) == 0 && (nfl & 3) == 0) {
-            if (threadIdx.x == 0) bulk_load(s_tile, g, nfl * 4u, &s_bar[0]);
+        if ((base & VM) == 0 && (nfl & VM) == 0) {
+            if (threadIdx.x == 0) bulk_load(s_t, g, nfl * ES, &s_bar[0]);
             mbar_wait(&s_bar[0], 0);
         } else {
-            for (uint32_t e = threadIdx.x; e < nfl; e += kFTile) s_tile[e] = g[e];
+            for (uint32_t e = threadIdx.x; e < nfl; e += kFTile) s_t[e] = g[e];
             __syncthreads();
         }
     } else if (s_hint && tile_bulk_ok(0)) {   // speculative: the first tile
-        if (threadIdx.x == 0) bulk_load(s_tile, g, tile_rows(0) * a.row * 4u, &s_bar[0]);
+        if (threadIdx.x == 0) bulk_load(s_t, g, tile_rows(0) * a.row * ES, &s_bar[0]);
         pending = 0;
     }
 
@@ -341,7 +344,7 @@ __global__ void __launch_bounds__(kFTile) filter_onepass_kernel(const FilterArgs
     for (int k = 0; k < kFMaxGroup; ++k) {
         const uint32_t rl = k * kFTile + threadIdx.x;
         xo[k] = __int_as_float(0x7fc00000);   // NaN: fails both quick tests and the exact one
-        if (k < G && rl < nrows) xo[k] = LONG ? __ldg(g + (size_t)rl * a.row + 4) : s_tile[rl * a.row + 4];
+        if (k < G && rl < nrows) xo[k] = LONG ? ldg_f(g + (size_t)rl * a.row + 4) : to_f32(s_t[rl * a.row + 4]);
     }
     unsigned mybal[kFMaxGroup];
 #pragma unroll
@@ -385,7 +388,7 @@ __global__ void __launch_bounds__(kFTile) filter_onepass_kernel(const FilterArgs
         if (LONG && k < G && a.stage_ok && tcnt[k] > 0 && tcnt[k] * 4 >= (int)tile_rows(k) && tile_bulk_ok(k)) dense_mask |= 1u << k;
     if (LONG && pending < 0 && dense_mask) {
         const int k = __ffs(dense_mask) - 1;
-        if (threadIdx.x == 0) bulk_load(s_tile, g + (size_t)k * tile_fl, tile_rows(k) * a.row * 4u, &s_bar[0]);
+        if (threadIdx.x == 0) bulk_load(s_t, g + (size_t)k * tile_fl, tile_rows(k) * a.row * ES, &s_bar[0]);
         pending = k;
     }
 #pragma unroll
@@ -418,8 +421,8 @@ __global__ void __launch_bounds__(kFTile) filter_onepass_kernel(const FilterArgs
 #pragma unroll 1
         for (int c = threadIdx.x; c < n_emit; c += kFTile) {
             const uint32_t rl = s_list[c];
-            const float* x = s_tile + rl * a.row;
-            filter_emit_row(a, L, row0 + rl, (size_t)b * a.cap + prefix + c, [&](int ch) { return x[ch]; }, inv_s, pt, pl);
+            const T* x = s_t + rl * a.row;
+            filter_emit_row(a, L, row0 + rl, (size_t)b * a.cap + prefix + c, [&](int ch) { return to_f32(x[ch]); }, inv_s, pt, pl);
         }
         return;
     }
@@ -429,8 +432,8 @@ __global__ void __launch_bounds__(kFTile) filter_onepass_kernel(const FilterArgs
     for (int c = threadIdx.x; c < n_emit; c += kFTile) {
         const uint32_t rl = s_list[c];
         if ((dense_mask >> (rl / kFTile)) & 1u) continue;
-        const float* x = g + (size_t)rl * a.row;
-        filter_emit_row(a, L, row0 + rl, (size_t)b * a.cap + prefix + c, [&](int ch) { return __ldg(x + ch); }, inv_s, pt, pl);
+        const T* x = g + (size_t)rl * a.row;
+        filter_emit_row(a, L, row0 + rl, (size_t)b * a.cap + prefix + c, [&](int ch) { return ldg_f(x + ch); }, inv_s, pt, pl);
     }
     // dense tiles: one bulk copy at a time through the tile buffer
     int off = 0;   // list offset of tile k
@@ -444,23 +447,23 @@ __global__ void __launch_bounds__(kFTile) filter_onepass_kernel(const FilterArgs
                 pending = -1;
             }
             if (pending != k) {
-                if (threadIdx.x == 0) bulk_load(s_tile, g + (size_t)k * tile_fl, tile_rows(k) * a.row * 4u, &s_bar[0]);
+                if (threadIdx.x == 0) bulk_load(s_t, g + (size_t)k * tile_fl, tile_rows(k) * a.row * ES, &s_bar[0]);
             }
             mbar_wait(&s_bar[0], parity);
             parity ^= 1u;
             pending = -1;
-            const float* xb = s_tile - (size_t)k * tile_fl;
+            const T* xb = s_t - (size_t)k * tile_fl;
 #pragma unroll 1
             for (int c = threadIdx.x; c < n_k; c += kFTile) {
                 const uint32_t rl = s_list[off + c];
-                const float* x = xb + (size_t)rl * a.row;
-                filter_emit_row(a, L, row0 + rl, (size_t)b * a.cap + prefix + off + c, [&](int ch) { return x[ch]; }, inv_s, pt, pl);
+                const T* x = xb + (size_t)rl * a.row;
+                filter_emit_row(a, L, row0 + rl, (size_t)b * a.cap + prefix + off + c, [&](int ch) { return to_f32(x[ch]); }, inv_s, pt, pl);
             }
             __syncthreads();   // the buffer is free again
             const unsigned rest = dense_mask >> (k + 1);
             if (rest) {          // next dense tile: start its copy right away
                 const int k2 = k + __ffs(rest);
-                if (threadIdx.x == 0) bulk_load(s_tile, g + (size_t)k2 * tile_fl, tile_rows(k2) * a.row * 4u, &s_bar[0]);
+                if (threadIdx.x == 0) bulk_load(s_t, g + (size_t)k2 * tile_fl, tile_rows(k2) * a.row * ES, &s_bar[0]);
                 pending = k2;
             }
         }
@@ -488,6 +491,7 @@ __device__ __forceinline__ int nchw_tile_scale(const FilterArgs& a, const Filter
     return s;
 }
 
+template <typename T>
 __global__ void __launch_bounds__(kFTile) filter_count_nchw_kernel(const FilterArgs a, const FilterNchw n) {
     __shared__ int s_red[kFTile / 32];
     const uint32_t tile = blockIdx.x, b = blockIdx.y;
@@ -499,7 +503,7 @@ __global__ void __launch_bounds__(kFTile) filter_count_nchw_kernel(const FilterA
         float x[YB_MAX_ANCHORS];
 #pragma unroll
         for (int an = 0; an < YB_MAX_ANCHORS; ++an)
-            if (an < a.A) x[an] = __ldg(L.pred + ((size_t)(b * (uint32_t)a.A + an) * a.row + 4) * L.hw + cell);
+            if (an < a.A) x[an] = ldg_f(reinterpret_cast<const T*>(L.pred) + ((size_t)(b * (uint32_t)a.A + an) * a.row + 4) * L.hw + cell);
 #pragma unroll
         for (int an = 0; an < YB_MAX_ANCHORS; ++an)
             if (an < a.A) cnt += sigmoidf_ref(x[an]) > a.conf ? 1 : 0;  // :1157,:1166-1167 objectness only
@@ -515,6 +519,7 @@ __global__ void __launch_bounds__(kFTile) filter_count_nchw_kernel(const FilterA
     }
 }
 
+template <typename T>
 __global__ void __launch_bounds__(kFTile) filter_emit_nchw_kernel(const FilterArgs a, const FilterNchw n) {
     __shared__ int s_red[kFTile / 32];
     __shared__ int s_wsum[kFTile / 32];
@@ -540,7 +545,7 @@ __global__ void __launch_bounds__(kFTile) filter_emit_nchw_kernel(const FilterAr
     const FilterScale& L = a.sc[s];
     const uint32_t cell = (tile - n.tile_begin[s]) * kFTile + threadIdx.x;
     const bool valid = cell < L.hw;
-    const float* plane0 = L.pred + (size_t)b * a.A * a.row * L.hw + (valid ? cell : 0u);  // channel 0, anchor 0
+    const T* plane0 = reinterpret_cast<const T*>(L.pred) + (size_t)b * a.A * a.row * L.hw + (valid ? cell : 0u);  // channel 0, anchor 0
     const size_t hw = L.hw;
 
     // phase A: objectness of this cell for every anchor
@@ -549,7 +554,7 @@ __global__ void __launch_bounds__(kFTile) filter_emit_nchw_kernel(const FilterAr
 #pragma unroll
     for (int an = 0; an < YB_MAX_ANCHORS; ++an) {
         so[an] = 0.0f;
-        if (an < a.A && valid) so[an] = __ldg(plane0 + ((size_t)an * a.row + 4) * hw);
+        if (an < a.A && valid) so[an] = ldg_f(plane0 + ((size_t)an * a.row + 4) * hw);
     }
 #pragma unroll
     for (int an = 0; an < YB_MAX_ANCHORS; ++an) {
@@ -584,12 +589,12 @@ __global__ void __launch_bounds__(kFTile) filter_emit_nchw_kernel(const FilterAr
     for (int an = 0; an < YB_MAX_ANCHORS; ++an) {
         if (an >= a.A || !((passmask >> an) & 1u)) continue;
         if (pos >= a.cap) break;
-        const float* x = plane0 + (size_t)an * a.row * hw;
+        const T* x = plane0 + (size_t)an * a.row * hw;
         const float aw = __ldg(L.anchors + an * 2), ah = __ldg(L.anchors + an * 2 + 1);
-        const float x0 = __ldg(x), x1r = __ldg(x + hw), x2r = __ldg(x + 2 * hw), x3r = __ldg(x + 3 * hw);
+        const float x0 = ldg_f(x), x1r = ldg_f(x + hw), x2r = ldg_f(x + 2 * hw), x3r = ldg_f(x + 3 * hw);
         float cprob;
         int cid;
-        class_max(a.nc, [&](int c) { return __ldg(x + (size_t)(5 + c) * hw); }, cprob, cid);
+        class_max(a.nc, [&](int c) { return ldg_f(x + (size_t)(5 + c) * hw); }, cprob, cid);
         const float bx = decode_xy(x0, (float)gx, L.inv_w);
         const float by = decode_xy(x1r, (float)gy, L.inv_h);
         const float bw = decode_wh(x2r, aw, a.inv_img);
@@ -614,6 +619,8 @@ static int filter_fill(const yb_heads_desc* d, FilterArgs& a) {
                  "filter: bad S/B/A/nc (nc must be >= 1, train.py:1184-1189)");
     a.S = d->S; a.A = d->A; a.nc = d->nc; a.row = 5 + d->nc;
     YB_CHECK_ARG(d->layout == YB_LAYOUT_BHWAC || d->layout == YB_LAYOUT_NCHW, "filter: unknown layout %d", d->layout);
+    YB_CHECK_ARG(d->dtype == YB_DTYPE_F32 || d->dtype == YB_DTYPE_BF16 || d->dtype == YB_DTYPE_F16,
+                 "filter: unknown dtype %d", d->dtype);
     a.nchw = d->layout == YB_LAYOUT_NCHW ? 1 : 0;
     a.img = d->img_size; a.inv_img = 1.0f / d->img_size;
     // tiles per CTA: kFMaxGroup in the reference layout (short rows stage the whole group, long rows stream tile by
@@ -641,6 +648,52 @@ static int filter_fill(const yb_heads_desc* d, FilterArgs& a) {
     return 0;
 }
 
+}  // namespace yb
+
+namespace yb {
+template <typename T>
+static int filter_launch(const yb_heads_desc* d, FilterArgs& a, void* ws, cudaStream_t st) {
+    // staging sizes follow the element size: half rows take half the bytes, so rows of up to 24 halves stage the
+    // whole group and a long-row tile buffer takes half the shared memory (more CTAs per SM)
+    const size_t es = sizeof(T);
+    const size_t tile_fl = ((size_t)kFTile * a.row + 31) / 32 * 32;   // elements
+    const bool long_rows = (size_t)a.G * kFTile * a.row * es > 48 * 1024;
+    size_t smem = long_rows ? tile_fl * es : (size_t)a.G * kFTile * a.row * es;
+    a.stage_ok = smem <= 200 * 1024;   // else: rows so long that one tile does not fit; the emit reads global memory
+    if (!a.stage_ok) smem = 0;
+    smem = (smem + 127) / 128 * 128;
+    a.sobj_offset = (uint32_t)(smem / sizeof(float));
+    smem += (size_t)a.G * kFTile * sizeof(float);   // NCHW: sigmoid(obj) scratch; reference layout: u16 row list (half of it)
+    if (a.nchw) {
+        FilterNchw n;
+        uint32_t t = 0;
+        for (int s = 0; s < d->S; ++s) {
+            n.tile_begin[s] = t;
+            t += (a.sc[s].hw + kFTile - 1) / kFTile;
+        }
+        n.tiles_per_img = t;  // <= tiles_per_img of the row tiling: the workspace is large enough
+        dim3 ngrid(t, d->B);
+        YB_LAUNCH("filter_count_nchw_kernel", st, filter_count_nchw_kernel<T><<<ngrid, kFTile, 0, st>>>(a, n));
+        YB_LAUNCH("filter_emit_nchw_kernel", st, filter_emit_nchw_kernel<T><<<ngrid, kFTile, 0, st>>>(a, n));
+        return 0;
+    }
+    dim3 grid(a.groups_per_img, d->B);
+    a.lb_state = reinterpret_cast<unsigned long long*>(ws);
+    a.lb_ticket = reinterpret_cast<unsigned int*>(a.lb_state + (size_t)d->B * a.groups_per_img);
+    a.lb_seen = a.lb_ticket + d->B;
+    YB_CUDA(cudaMemsetAsync(ws, 0, (size_t)d->B * a.groups_per_img * sizeof(unsigned long long) + ((size_t)d->B + 2) * sizeof(unsigned int), st));
+    const size_t dyn = smem;
+    if (long_rows) {
+        if (dyn > 48 * 1024)
+            YB_CUDA(cudaFuncSetAttribute(filter_onepass_kernel<true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+        YB_LAUNCH("filter_onepass_kernel", st, (filter_onepass_kernel<true, T><<<grid, kFTile, dyn, st>>>(a)));
+    } else {
+        if (dyn > 48 * 1024)
+            YB_CUDA(cudaFuncSetAttribute(filter_onepass_kernel<false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+        YB_LAUNCH("filter_onepass_kernel", st, (filter_onepass_kernel<false, T><<<grid, kFTile, dyn, st>>>(a)));
+    }
+    return 0;
+}
 }  // namespace yb
 
 extern "C" size_t yb_filter_workspace_bytes(const yb_heads_desc* d) {
@@ -684,42 +737,7 @@ extern "C" int yb_filter_compact(const yb_heads_desc* d, float conf_thres, const
     }
     a.tile_counts = reinterpret_cast<int*>(ws);
     a.boxes = reinterpret_cast<float4*>(boxes); a.scores = scores; a.classes = classes; a.counts = counts;
-    const size_t tile_fl = ((size_t)kFTile * a.row + 31) / 32 * 32;
-    const bool long_rows = (size_t)a.G * kFTile * a.row * sizeof(float) > 48 * 1024;
-    size_t smem = long_rows ? tile_fl * sizeof(float) : (size_t)a.G * kFTile * a.row * sizeof(float);
-    a.stage_ok = smem <= 200 * 1024;   // else: rows so long that one tile does not fit; the emit reads global memory
-    if (!a.stage_ok) smem = 0;
-    smem = (smem + 127) / 128 * 128;
-    a.sobj_offset = (uint32_t)(smem / sizeof(float));
-    smem += (size_t)a.G * kFTile * sizeof(float);   // NCHW: sigmoid(obj) scratch; reference layout: u16 row list (half of it)
     cudaStream_t st = (cudaStream_t)stream;
-    if (a.nchw) {
-        FilterNchw n;
-        uint32_t t = 0;
-        for (int s = 0; s < d->S; ++s) {
-            n.tile_begin[s] = t;
-            t += (a.sc[s].hw + kFTile - 1) / kFTile;
-        }
-        n.tiles_per_img = t;  // <= tiles_per_img of the row tiling: the workspace is large enough
-        dim3 ngrid(t, d->B);
-        YB_LAUNCH("filter_count_nchw_kernel", st, filter_count_nchw_kernel<<<ngrid, kFTile, 0, st>>>(a, n));
-        YB_LAUNCH("filter_emit_nchw_kernel", st, filter_emit_nchw_kernel<<<ngrid, kFTile, 0, st>>>(a, n));
-        return 0;
-    }
-    dim3 grid(a.groups_per_img, d->B);
-    a.lb_state = reinterpret_cast<unsigned long long*>(ws);
-    a.lb_ticket = reinterpret_cast<unsigned int*>(a.lb_state + (size_t)d->B * a.groups_per_img);
-    a.lb_seen = a.lb_ticket + d->B;
-    YB_CUDA(cudaMemsetAsync(ws, 0, (size_t)d->B * a.groups_per_img * sizeof(unsigned long long) + ((size_t)d->B + 2) * sizeof(unsigned int), st));
-    const size_t dyn = smem;
-    if (long_rows) {
-        if (dyn > 48 * 1024)
-            YB_CUDA(cudaFuncSetAttribute(filter_onepass_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-        YB_LAUNCH("filter_onepass_kernel", st, filter_onepass_kernel<true><<<grid, kFTile, dyn, st>>>(a));
-    } else {
-        if (dyn > 48 * 1024)
-            YB_CUDA(cudaFuncSetAttribute(filter_onepass_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-        YB_LAUNCH("filter_onepass_kernel", st, filter_onepass_kernel<false><<<grid, kFTile, dyn, st>>>(a));
-    }
+    YB_DISPATCH_DTYPE(d->dtype, T, return filter_launch<T>(d, a, ws, st));
     return 0;
 }

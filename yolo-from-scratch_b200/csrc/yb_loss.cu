@@ -150,10 +150,11 @@ __global__ void ciou_mean_kernel(const double* __restrict__ acc, long long N, fl
 constexpr int kTileRows = 256;  // rows per tile == threads per CTA of loss_main_kernel
 
 struct LossScale {
-    const float* pred;
+    const void* pred;     // element type T of the kernels
     const float* tgt;
     const float* anchors;
-    float* grad;
+    void* grad;           // fp32: written by stage 1; half: written by yb_loss_grad_emit only
+    float* dobj;          // half heads: fp32 objectness gradient of every row (canonical order), else null
     const uint32_t* bits; // sparse targets: 1 bit per row (positive), else null
     uint32_t rows;        // B*H*W*A (local)
     uint32_t tile_begin;  // first global tile index of this scale
@@ -181,7 +182,9 @@ struct LossArgs {
     float coef_box[YB_MAX_SCALES], coef_cls[YB_MAX_SCALES];
     const uint32_t* pos_ent;     // sparse targets: entry id of each listed row
     const SparseEntry* entries;  // sparse targets: target rows
-    double* partials;    // S*4: {sum(1-ciou), n_pos, sum bce_obj, sum bce_cls}
+    double* partials;    // S*4: {sum(1-ciou), n_pos, sum bce_obj, sum bce_cls}; null in the half emit pass
+    const double* red;   // half emit pass: the reduced partials (P_s of the normalisation), else null
+    const float* gscale; // half emit pass: upstream gradient s of `total` (device), else null
 };
 
 // offset of channel 0 of canonical row r, and the distance between its channels
@@ -202,7 +205,7 @@ struct LossWs {
     int pad[12];
 };
 
-template <bool SPARSE>
+template <typename T, bool SPARSE>
 __global__ void __launch_bounds__(kTileRows) loss_main_kernel(const LossArgs a) {
     __shared__ float s_dobj[kTileRows];
     __shared__ float s_warp[kTileRows / 32];
@@ -226,7 +229,7 @@ __global__ void __launch_bounds__(kTileRows) loss_main_kernel(const LossArgs a) 
         bool pos = false;
         if (threadIdx.x < nrows) {
             const size_t off = (size_t)(row0 + threadIdx.x) * a.row + 4;
-            const float x = __ldg(L.pred + off);
+            const float x = ldg_f(reinterpret_cast<const T*>(L.pred) + off);
             float t;
             if (SPARSE) {
                 const uint32_t r = row0 + threadIdx.x;
@@ -235,7 +238,12 @@ __global__ void __launch_bounds__(kTileRows) loss_main_kernel(const LossArgs a) 
                 t = __ldg(L.tgt + off);
             }
             bce = bce_logits_ref(x, t);
-            s_dobj[threadIdx.x] = (sigmoidf_ref(x) - t) * L.obj_scale;
+            const float dobj = (sigmoidf_ref(x) - t) * L.obj_scale;
+            if constexpr (kHalf<T>) {   // no dense gradient here: the emit pass writes it once s is known
+                if (L.dobj) L.dobj[row0 + threadIdx.x] = dobj;
+            } else {
+                s_dobj[threadIdx.x] = dobj;
+            }
             pos = t > 0.5f;
         }
         // positives: warp-aggregated append
@@ -258,9 +266,9 @@ __global__ void __launch_bounds__(kTileRows) loss_main_kernel(const LossArgs a) 
                 if (k == s) cta_sum[k] += (double)tsum;
         }
         // phase 2: dense gradient tile, coalesced float4: zeros except the objectness column
-        if (L.grad) {
+        if (!kHalf<T> && L.grad) {
             const uint32_t nfl = nrows * a.row;
-            float* g = L.grad + (size_t)row0 * a.row;
+            float* g = reinterpret_cast<float*>(L.grad) + (size_t)row0 * a.row;
             float4* g4 = reinterpret_cast<float4*>(g);
             const uint32_t nvec = nfl >> 2;
             for (uint32_t v = threadIdx.x; v < nvec; v += kTileRows) {
@@ -296,7 +304,7 @@ __global__ void __launch_bounds__(kTileRows) loss_main_kernel(const LossArgs a) 
 // store of the gradient.
 constexpr int kNchwVecs = 4;  // float4 vectors per thread and tile: 256 threads x 4 x 16 B = 16 KB per tile
 
-template <bool SPARSE>
+template <typename T, bool SPARSE>
 __device__ __forceinline__ float nchw_obj_elem(const LossArgs& a, const LossScale& L, int s, uint32_t ba, uint32_t cell,
                                                float x, float& bce) {
     uint32_t b, an;
@@ -310,11 +318,18 @@ __device__ __forceinline__ float nchw_obj_elem(const LossArgs& a, const LossScal
         const int slot = atomicAdd(a.pos_count + s, 1);
         a.pos_list[L.list_begin + slot] = r;
     }
-    return (sigmoidf_ref(x) - t) * L.obj_scale;
+    const float dobj = (sigmoidf_ref(x) - t) * L.obj_scale;
+    if constexpr (kHalf<T>) {
+        if (L.dobj) L.dobj[r] = dobj;
+    }
+    return dobj;
 }
 
-template <bool SPARSE>
+template <typename T, bool SPARSE>
 __global__ void __launch_bounds__(kTileRows) loss_main_nchw_kernel(const LossArgs a) {
+    // 4 elements per step for every element type (16-byte fp32 vectors, 8-byte half vectors): each thread sums the
+    // same elements in the same order, so the half heads' loss is bit-identical to the fp32 path's
+    constexpr uint32_t V = 4;
     __shared__ double s_part[kTileRows / 32][YB_MAX_SCALES];
     double acc[YB_MAX_SCALES];
 #pragma unroll
@@ -330,29 +345,39 @@ __global__ void __launch_bounds__(kTileRows) loss_main_nchw_kernel(const LossArg
         float bce = 0.0f;
 #pragma unroll
         for (int k = 0; k < kNchwVecs; ++k) {
-            const uint32_t e0 = (((tile - L.tile_begin) * kNchwVecs + k) * kTileRows + threadIdx.x) * 4u;
+            const uint32_t e0 = (((tile - L.tile_begin) * kNchwVecs + k) * kTileRows + threadIdx.x) * V;
             if (e0 >= L.n_float) continue;
             uint32_t plane, within;
             L.d_HW.divmod(e0, plane, within);
-            float o[4] = {0.0f, 0.0f, 0.0f, 0.0f};
-            if (within + 4u <= L.HW && e0 + 4u <= L.n_float) {  // the common case: one channel plane
+            float o[V];
+#pragma unroll
+            for (int j = 0; j < (int)V; ++j) o[j] = 0.0f;
+            if (within + V <= L.HW && e0 + V <= L.n_float) {  // the common case: one channel plane
                 uint32_t ba, c;
                 a.d_row.divmod(plane, ba, c);
                 if (c == 4u) {
-                    const float4 x = __ldg(reinterpret_cast<const float4*>(L.pred + e0));
-                    o[0] = nchw_obj_elem<SPARSE>(a, L, s, ba, within, x.x, bce);
-                    o[1] = nchw_obj_elem<SPARSE>(a, L, s, ba, within + 1, x.y, bce);
-                    o[2] = nchw_obj_elem<SPARSE>(a, L, s, ba, within + 2, x.z, bce);
-                    o[3] = nchw_obj_elem<SPARSE>(a, L, s, ba, within + 3, x.w, bce);
+                    if constexpr (kHalf<T>) {
+                        const uint2 x2 = __ldg(reinterpret_cast<const uint2*>(reinterpret_cast<const T*>(L.pred) + e0));
+                        const T* x = reinterpret_cast<const T*>(&x2);
+#pragma unroll
+                        for (int j = 0; j < (int)V; ++j) o[j] = nchw_obj_elem<T, SPARSE>(a, L, s, ba, within + j, to_f32(x[j]), bce);
+                    } else {
+                        const float4 x4 = __ldg(reinterpret_cast<const float4*>(reinterpret_cast<const T*>(L.pred) + e0));
+                        o[0] = nchw_obj_elem<T, SPARSE>(a, L, s, ba, within, x4.x, bce);
+                        o[1] = nchw_obj_elem<T, SPARSE>(a, L, s, ba, within + 1, x4.y, bce);
+                        o[2] = nchw_obj_elem<T, SPARSE>(a, L, s, ba, within + 2, x4.z, bce);
+                        o[3] = nchw_obj_elem<T, SPARSE>(a, L, s, ba, within + 3, x4.w, bce);
+                    }
                 }
-                if (L.grad) *reinterpret_cast<float4*>(L.grad + e0) = make_float4(o[0], o[1], o[2], o[3]);
-            } else {  // a vector straddling two planes or the end of the tensor (H*W not a multiple of 4)
-                for (uint32_t j = 0; j < 4u && e0 + j < L.n_float; ++j) {
+                if (!kHalf<T> && L.grad)   // half: the emit pass writes the gradient
+                    *reinterpret_cast<float4*>(reinterpret_cast<float*>(L.grad) + e0) = make_float4(o[0], o[1], o[2], o[3]);
+            } else {  // a vector straddling two planes or the end of the tensor (H*W not a multiple of V)
+                for (uint32_t j = 0; j < V && e0 + j < L.n_float; ++j) {
                     uint32_t ba, c;
                     a.d_row.divmod(plane, ba, c);
                     float v = 0.0f;
-                    if (c == 4u) v = nchw_obj_elem<SPARSE>(a, L, s, ba, within, __ldg(L.pred + e0 + j), bce);
-                    if (L.grad) L.grad[e0 + j] = v;
+                    if (c == 4u) v = nchw_obj_elem<T, SPARSE>(a, L, s, ba, within, ldg_f(reinterpret_cast<const T*>(L.pred) + e0 + j), bce);
+                    if (!kHalf<T> && L.grad) reinterpret_cast<float*>(L.grad)[e0 + j] = v;
                     if (++within == L.HW) { within = 0; ++plane; }
                 }
             }
@@ -375,8 +400,9 @@ __global__ void __launch_bounds__(kTileRows) loss_main_nchw_kernel(const LossArg
     }
 }
 
-// one warp per positive row
-template <bool SPARSE>
+// one warp per positive row.  Half heads run it twice: in stage 1 for the loss sums only (grad null), and in the
+// emit pass (partials null, red/gscale set) for the gradient of the positive rows, fully normalised and scaled.
+template <typename T, bool SPARSE>
 __global__ void __launch_bounds__(256) loss_positive_kernel(const LossArgs a) {
     const int lane = threadIdx.x & 31;
     const int warps_per_cta = blockDim.x >> 5;
@@ -388,16 +414,29 @@ __global__ void __launch_bounds__(256) loss_positive_kernel(const LossArgs a) {
         double acc_box = 0.0, acc_cls = 0.0;
         // single rank: the local positive count IS the global one, so the normalisation that
         // loss_finalize_kernel would apply (same two roundings: unnormalised value, then * k) happens here
-        float k_box = 1.0f, k_cls = 1.0f;
-        if (a.fuse_norm && P > 0) {
+        float k_box = 1.0f, k_cls = 1.0f, gsc = 1.0f;
+        if constexpr (kHalf<T>) {   // emit pass: the normalisation of loss_finalize_kernel, from the reduced P_s
+            const double Pg = a.red ? a.red[s * 4 + 1] : 0.0;
+            if (Pg > 0.0) {
+                k_box = (float)((double)a.coef_box[s] / Pg);
+                k_cls = a.nc > 0 ? (float)((double)a.coef_cls[s] / (Pg * (double)a.nc)) : 0.0f;
+            }
+            if (a.gscale) gsc = __ldg(a.gscale);
+        } else if (a.fuse_norm && P > 0) {
             k_box = (float)((double)a.coef_box[s] / (double)P);
             k_cls = a.nc > 0 ? (float)((double)a.coef_cls[s] / ((double)P * (double)a.nc)) : 0.0f;
         }
+        // gradient entry i of the row: fp32 as before; half: round_D((g * k) * s), the fp32 path's two roundings,
+        // its scale_kernel product and the cast to the head dtype
+        auto put = [&](size_t i, float g, float k) {
+            if constexpr (kHalf<T>) reinterpret_cast<T*>(L.grad)[i] = from_f32<T>((g * k) * gsc);
+            else reinterpret_cast<float*>(L.grad)[i] = a.fuse_norm ? g * k : g;
+        };
         for (uint32_t k = gwarp; k < P; k += nwarps) {
             const uint32_t r = a.pos_list[L.list_begin + k];
             uint32_t cs;
             const size_t xb = row_base(a, L, r, cs);
-            const float* x = L.pred + xb;
+            const T* x = reinterpret_cast<const T*>(L.pred) + xb;
             const float* t = SPARSE ? nullptr : L.tgt + (size_t)r * a.row;  // dense targets keep the reference layout
             SparseEntry ent = {0.f, 0.f, 0.f, 0.f, 0, 0, 0, 0};
             if (SPARSE) ent = a.entries[a.pos_ent[L.list_begin + k]];
@@ -406,7 +445,7 @@ __global__ void __launch_bounds__(256) loss_positive_kernel(const LossArgs a) {
             L.d_W.divmod(cell, gy_b, gx);
             L.d_H.divmod(gy_b, bi, gy);
             const float aw = __ldg(L.anchors + an * 2), ah = __ldg(L.anchors + an * 2 + 1);
-            const float xr[4] = {x[0], x[(size_t)cs], x[2 * (size_t)cs], x[3 * (size_t)cs]};
+            const float xr[4] = {to_f32(x[0]), to_f32(x[(size_t)cs]), to_f32(x[2 * (size_t)cs]), to_f32(x[3 * (size_t)cs])};
             const float p[4] = {decode_xy(xr[0], (float)gx, L.inv_w), decode_xy(xr[1], (float)gy, L.inv_h),
                                 decode_wh(xr[2], aw, a.inv_img), decode_wh(xr[3], ah, a.inv_img)};
             const float tb[4] = {SPARSE ? ent.x : t[0], SPARSE ? ent.y : t[1], SPARSE ? ent.w : t[2],
@@ -416,12 +455,12 @@ __global__ void __launch_bounds__(256) loss_positive_kernel(const LossArgs a) {
             // class BCE, lanes stride over classes
             float cls = 0.0f;
             for (int c = lane; c < a.nc; c += 32) {
-                const float xc = x[(size_t)(5 + c) * cs];
+                const float xc = to_f32(x[(size_t)(5 + c) * cs]);
                 const float tc = SPARSE ? (c == ent.cls ? 1.0f : 0.0f) : t[5 + c];
                 cls += bce_logits_ref(xc, tc);
                 if (L.grad) {
                     const float g = sigmoidf_ref(xc) - tc;
-                    L.grad[xb + (size_t)(5 + c) * cs] = a.fuse_norm ? g * k_cls : g;
+                    put(xb + (size_t)(5 + c) * cs, g, k_cls);
                 }
             }
             cls = warp_sum(cls);
@@ -437,16 +476,18 @@ __global__ void __launch_bounds__(256) loss_positive_kernel(const LossArgs a) {
                     const float u = 2.0f * sgm;
                     g = (((gp[lane] * (anc * a.inv_img)) * (2.0f * u)) * 2.0f) * ds;
                 }
-                L.grad[xb + (size_t)lane * cs] = a.fuse_norm ? g * k_box : g;
+                put(xb + (size_t)lane * cs, g, k_box);
             }
             acc_box += (double)l;
             acc_cls += (double)cls;
         }
-        if (lane == 0 && gwarp < P) {
-            atomicAdd(a.partials + s * 4 + 0, acc_box);
-            if (a.nc > 0) atomicAdd(a.partials + s * 4 + 3, acc_cls);
+        if (!kHalf<T> || a.partials) {
+            if (lane == 0 && gwarp < P) {
+                atomicAdd(a.partials + s * 4 + 0, acc_box);
+                if (a.nc > 0) atomicAdd(a.partials + s * 4 + 3, acc_cls);
+            }
+            if (gwarp == 0 && lane == 0) a.partials[s * 4 + 1] = (double)P;
         }
-        if (gwarp == 0 && lane == 0) a.partials[s * 4 + 1] = (double)P;
     }
 }
 
@@ -477,7 +518,7 @@ __global__ void __launch_bounds__(256) loss_finalize_kernel(const FinalizeArgs f
         const float k_cls = a.nc > 0 ? (float)((double)f.coef_cls[s] / (Pg * (double)a.nc)) : 0.0f;
         for (uint32_t k = gwarp; k < P; k += nwarps) {
             uint32_t cs;
-            float* g = L.grad + row_base(a, L, a.pos_list[L.list_begin + k], cs);
+            float* g = reinterpret_cast<float*>(L.grad) + row_base(a, L, a.pos_list[L.list_begin + k], cs);
             if (lane < 4) g[(size_t)lane * cs] *= k_box;
             for (int c = lane; c < a.nc; c += 32) g[(size_t)(5 + c) * cs] *= k_cls;
         }
@@ -517,6 +558,59 @@ __global__ void __launch_bounds__(256) scale_kernel(float* __restrict__ x, long 
     if (blockIdx.x == 0 && threadIdx.x < (n & 3)) x[nvec * 4 + threadIdx.x] *= f;
 }
 
+// Half heads, backward: the dense gradient of every scale, zeros except the objectness channel, which is
+// round_D(dobj * s) (dobj: stage 1's fp32 value).  16-byte vector stores; loss_positive_kernel<T> overwrites the
+// box and class channels of the positive rows afterwards.  Zeros are 0 * s, as the fp32 path's scale_kernel gives.
+template <typename T>
+__global__ void __launch_bounds__(256) loss_grad_emit_kernel(const LossArgs a) {
+    constexpr uint32_t V = kVec<T>;
+    const float gsc = __ldg(a.gscale);
+    const float zero = 0.0f * gsc;
+    const uint32_t tid = blockIdx.x * blockDim.x + threadIdx.x, stride = gridDim.x * blockDim.x;
+    for (int s = 0; s < a.S; ++s) {
+        const LossScale& L = a.sc[s];
+        T* grad = reinterpret_cast<T*>(L.grad);
+        if (!grad) continue;
+        const float* dobj = L.dobj;
+        const uint32_t n = L.n_float, nv = (n + V - 1) / V;
+        for (uint32_t v = tid; v < nv; v += stride) {
+            const uint32_t e0 = v * V;
+            float o[V];
+            if (!a.nchw) {
+                uint32_t r, c;
+                a.d_row.divmod(e0, r, c);
+#pragma unroll
+                for (int j = 0; j < (int)V; ++j) {
+                    o[j] = (c == 4u && e0 + j < n) ? dobj[r] * gsc : zero;
+                    if (++c == a.row) { c = 0; ++r; }
+                }
+            } else {
+                uint32_t plane, within, ba, c;
+                L.d_HW.divmod(e0, plane, within);
+                a.d_row.divmod(plane, ba, c);
+#pragma unroll
+                for (int j = 0; j < (int)V; ++j) {
+                    o[j] = zero;
+                    if (c == 4u && e0 + j < n) {
+                        uint32_t b, an;
+                        L.d_A.divmod(ba, b, an);
+                        o[j] = dobj[(b * L.HW + within) * (uint32_t)a.A + an] * gsc;
+                    }
+                    if (++within == L.HW) {
+                        within = 0;
+                        if (++c == a.row) { c = 0; ++ba; }
+                    }
+                }
+            }
+            if (e0 + V <= n) {
+                *reinterpret_cast<float4*>(grad + e0) = pack16<T>(o);
+            } else {
+                for (uint32_t j = 0; e0 + j < n; ++j) grad[e0 + j] = from_f32<T>(o[j]);
+            }
+        }
+    }
+}
+
 // ---- host side ----------------------------------------------------------------------------
 static int loss_validate(const yb_loss_desc* d, bool need_ptrs, bool sparse = false) {
     YB_CHECK_ARG(d, "loss: null descriptor");
@@ -524,6 +618,8 @@ static int loss_validate(const yb_loss_desc* d, bool need_ptrs, bool sparse = fa
     YB_CHECK_ARG(d->B >= 0 && d->A > 0 && d->A <= YB_MAX_ANCHORS && d->nc >= 0, "loss: bad B/A/nc");
     YB_CHECK_ARG(d->B_global >= d->B, "loss: B_global < B");
     YB_CHECK_ARG(d->layout == YB_LAYOUT_BHWAC || d->layout == YB_LAYOUT_NCHW, "loss: unknown layout %d", d->layout);
+    YB_CHECK_ARG(d->dtype == YB_DTYPE_F32 || d->dtype == YB_DTYPE_BF16 || d->dtype == YB_DTYPE_F16,
+                 "loss: unknown dtype %d", d->dtype);
     unsigned long long tot = 0;
     for (int s = 0; s < d->S; ++s) {
         YB_CHECK_ARG(d->H[s] > 0 && d->W[s] > 0, "loss: bad grid at scale %d", s);
@@ -540,7 +636,17 @@ static int loss_validate(const yb_loss_desc* d, bool need_ptrs, bool sparse = fa
     return 0;
 }
 
+static size_t loss_rows(const yb_loss_desc* d) {
+    size_t rows = 0;
+    for (int s = 0; s < d->S; ++s) rows += (size_t)d->B * d->H[s] * d->W[s] * d->A;
+    return rows;
+}
+// half heads: the fp32 objectness gradient (rows floats) follows the positive list in the workspace
+static size_t dobj_offset(const yb_loss_desc* d) { return (sizeof(LossWs) + loss_rows(d) * sizeof(uint32_t) + 15) / 16 * 16; }
+static size_t dobj_bytes(const yb_loss_desc* d) { return d->dtype == YB_DTYPE_F32 ? 0 : loss_rows(d) * sizeof(float); }
+
 static void loss_fill_args(const yb_loss_desc* d, void* ws, LossArgs& a) {
+    const bool half = d->dtype != YB_DTYPE_F32;
     a.S = d->S; a.A = d->A; a.nc = d->nc; a.row = 5 + d->nc;
     a.nchw = d->layout == YB_LAYOUT_NCHW ? 1 : 0;
     a.inv_img = 1.0f / d->img_size; a.eps = d->eps;
@@ -551,14 +657,17 @@ static void loss_fill_args(const yb_loss_desc* d, void* ws, LossArgs& a) {
     uint32_t tile = 0, list = 0;
     for (int s = 0; s < d->S; ++s) {
         LossScale& L = a.sc[s];
-        L.pred = d->pred[s]; L.tgt = d->tgt[s]; L.anchors = d->anchors[s]; L.grad = d->grad[s];
+        L.pred = d->pred[s]; L.tgt = d->tgt[s]; L.anchors = d->anchors[s];
+        L.grad = half ? nullptr : d->grad[s];   // half: only yb_loss_grad_emit writes the gradient
+        L.dobj = half ? reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + dobj_offset(d)) + list : nullptr;
         L.bits = nullptr;
         L.rows = (uint32_t)((unsigned long long)d->B * d->H[s] * d->W[s] * d->A);
         L.tile_begin = tile; L.list_begin = list;
         L.HW = (uint32_t)d->H[s] * (uint32_t)d->W[s];
         L.n_float = L.rows * a.row;
         L.d_HW = FastDiv(L.HW);
-        // reference layout: one tile = kTileRows rows; NCHW: one tile = kTileRows*kNchwVecs float4 of the flat tensor
+        // reference layout: one tile = kTileRows rows; NCHW: one tile = kTileRows*kNchwVecs steps of 4 elements of the
+        // flat tensor
         tile += a.nchw ? (L.n_float + kTileRows * 4 * kNchwVecs - 1) / (kTileRows * 4 * kNchwVecs)
                        : (L.rows + kTileRows - 1) / kTileRows;
         list += L.rows;
@@ -572,10 +681,14 @@ static void loss_fill_args(const yb_loss_desc* d, void* ws, LossArgs& a) {
     a.pos_ent = nullptr;
     a.entries = nullptr;
     a.fuse_norm = d->B_global == (long long)d->B ? 1 : 0;
+    a.partials = nullptr;
+    a.red = nullptr;
+    a.gscale = nullptr;
     for (int s = 0; s < d->S; ++s) { a.coef_box[s] = d->coef_box[s]; a.coef_cls[s] = d->coef_cls[s]; }
 }
 
-// sparse-target workspace: [dense-layout workspace][pos_ent: rows u32][entries][bits]
+// sparse-target workspace: [dense-layout workspace][pos_ent: rows u32][entries][bits]; the dense-layout part holds
+// the objectness gradient of half heads, so pos_ent and entries do not depend on max_gt
 struct SparseLayout { size_t pos_ent, entries, bits, total; uint32_t bits_begin[YB_MAX_SCALES]; };
 static SparseLayout sparse_layout(const yb_loss_desc* d, int max_gt) {
     SparseLayout L;
@@ -586,7 +699,7 @@ static SparseLayout sparse_layout(const yb_loss_desc* d, int max_gt) {
         words += (r + 31) / 32;
         rows += r;
     }
-    size_t o = (sizeof(LossWs) + rows * sizeof(uint32_t) + 15) / 16 * 16;
+    size_t o = (dobj_offset(d) + dobj_bytes(d) + 15) / 16 * 16;
     L.pos_ent = o; o = (o + rows * sizeof(uint32_t) + 15) / 16 * 16;
     L.entries = o; o += (size_t)d->B * (max_gt > 0 ? max_gt : 1) * sizeof(SparseEntry);
     L.bits = o; o += (words + 4) * sizeof(uint32_t);
@@ -625,10 +738,21 @@ extern "C" int yb_ciou_fwd_bwd(const float* pred_boxes, const float* tgt_boxes, 
 
 extern "C" size_t yb_loss_workspace_bytes(const yb_loss_desc* d) {
     if (!d || d->S < 1 || d->S > YB_MAX_SCALES) return 0;
-    size_t rows = 0;
-    for (int s = 0; s < d->S; ++s) rows += (size_t)d->B * d->H[s] * d->W[s] * d->A;
-    return sizeof(yb::LossWs) + rows * sizeof(uint32_t) + 16;
+    if (d->dtype != YB_DTYPE_F32) return yb::dobj_offset(d) + yb::dobj_bytes(d) + 16;
+    return sizeof(yb::LossWs) + yb::loss_rows(d) * sizeof(uint32_t) + 16;
 }
+
+namespace yb {
+template <typename T, bool SPARSE>
+static int loss_stage1_launch(const LossArgs& a, cudaStream_t st) {
+    const int sms = sm_count();
+    int blocks = (int)(a.n_tiles < (uint32_t)(sms * 8) ? a.n_tiles : (uint32_t)(sms * 8));
+    if (a.nchw) YB_LAUNCH("loss_main_nchw_kernel", st, (loss_main_nchw_kernel<T, SPARSE><<<blocks, kTileRows, 0, st>>>(a)));
+    else YB_LAUNCH("loss_main_kernel", st, (loss_main_kernel<T, SPARSE><<<blocks, kTileRows, 0, st>>>(a)));
+    YB_LAUNCH("loss_positive_kernel", st, (loss_positive_kernel<T, SPARSE><<<sms * 2, 256, 0, st>>>(a)));
+    return 0;
+}
+}  // namespace yb
 
 extern "C" int yb_loss_partials(const yb_loss_desc* d, double* partials, void* ws, size_t ws_bytes,
                                 void* stream) {
@@ -647,11 +771,7 @@ extern "C" int yb_loss_partials(const yb_loss_desc* d, double* partials, void* w
     YB_CUDA(cudaMemsetAsync(ws, 0, sizeof(LossWs), st));
     YB_CUDA(cudaMemsetAsync(partials, 0, sizeof(double) * 4 * d->S, st));
     if (a.n_tiles == 0) return 0;
-    const int sms = sm_count();
-    int blocks = (int)(a.n_tiles < (uint32_t)(sms * 8) ? a.n_tiles : (uint32_t)(sms * 8));
-    if (a.nchw) YB_LAUNCH("loss_main_nchw_kernel", st, loss_main_nchw_kernel<false><<<blocks, kTileRows, 0, st>>>(a));
-    else YB_LAUNCH("loss_main_kernel", st, loss_main_kernel<false><<<blocks, kTileRows, 0, st>>>(a));
-    YB_LAUNCH("loss_positive_kernel", st, loss_positive_kernel<false><<<sms * 2, 256, 0, st>>>(a));
+    YB_DISPATCH_DTYPE(d->dtype, T, return loss_stage1_launch<T, false>(a, st));
     return 0;
 }
 
@@ -703,11 +823,7 @@ extern "C" int yb_loss_partials_sparse(const yb_loss_desc* d, const double* labe
     rc = launch_assign_sparse(labels, n_gt, letterbox, anchors_all, d->B, max_gt, d->S, G, d->A, d->nc, assign_img_size,
                               status, o, st);
     if (rc) return rc;
-    const int sms = sm_count();
-    int blocks = (int)(a.n_tiles < (uint32_t)(sms * 8) ? a.n_tiles : (uint32_t)(sms * 8));
-    if (a.nchw) YB_LAUNCH("loss_main_nchw_kernel", st, loss_main_nchw_kernel<true><<<blocks, kTileRows, 0, st>>>(a));
-    else YB_LAUNCH("loss_main_kernel", st, loss_main_kernel<true><<<blocks, kTileRows, 0, st>>>(a));
-    YB_LAUNCH("loss_positive_kernel", st, loss_positive_kernel<true><<<sms * 2, 256, 0, st>>>(a));
+    YB_DISPATCH_DTYPE(d->dtype, T, return loss_stage1_launch<T, true>(a, st));
     return 0;
 }
 
@@ -732,11 +848,55 @@ extern "C" int yb_loss_finalize(const yb_loss_desc* d, const double* partials, f
         f.w_obj[s] = d->w_obj[s];
         f.coef_box[s] = d->coef_box[s];
         f.coef_cls[s] = d->coef_cls[s];
-        any_grad |= d->grad[s] != nullptr;
+        any_grad |= f.a.sc[s].grad != nullptr;
     }
     const int blocks = (any_grad && f.a.n_tiles > 0 && !f.a.fuse_norm) ? sm_count() : 1;
     cudaStream_t st = (cudaStream_t)stream;
     YB_LAUNCH("loss_finalize_kernel", st, loss_finalize_kernel<<<blocks, 256, 0, st>>>(f));
+    return 0;
+}
+
+namespace yb {
+template <typename T>
+static int loss_emit_launch(const LossArgs& a, bool sparse, cudaStream_t st) {
+    const int sms = sm_count();
+    YB_LAUNCH("loss_grad_emit_kernel", st, loss_grad_emit_kernel<T><<<sms * 8, 256, 0, st>>>(a));
+    if (sparse) YB_LAUNCH("loss_positive_kernel", st, (loss_positive_kernel<T, true><<<sms * 2, 256, 0, st>>>(a)));
+    else YB_LAUNCH("loss_positive_kernel", st, (loss_positive_kernel<T, false><<<sms * 2, 256, 0, st>>>(a)));
+    return 0;
+}
+}  // namespace yb
+
+extern "C" int yb_loss_grad_emit(const yb_loss_desc* d, const double* partials, const float* grad_scale, int max_gt,
+                                 void* ws, size_t ws_bytes, void* stream) {
+    using namespace yb;
+    const bool sparse = max_gt >= 0;
+    int rc = loss_validate(d, true, sparse);
+    if (rc) return rc;
+    YB_CHECK_ARG(d->dtype != YB_DTYPE_F32, "loss_grad_emit: fp32 heads get their gradient from yb_loss_partials");
+    YB_CHECK_ARG(partials && grad_scale && ws, "loss_grad_emit: null pointer");
+    const size_t need = sparse ? yb_loss_sparse_workspace_bytes(d, max_gt) : yb_loss_workspace_bytes(d);
+    if (ws_bytes < need) {
+        set_error("loss_grad_emit: workspace %zu < %zu", ws_bytes, need);
+        return YB_EWORKSPACE;
+    }
+    LossArgs a;
+    loss_fill_args(d, ws, a);
+    bool any = false;
+    for (int s = 0; s < d->S; ++s) {
+        a.sc[s].grad = d->grad[s];
+        any |= d->grad[s] != nullptr;
+    }
+    if (!any || a.n_tiles == 0) return 0;
+    a.red = partials;
+    a.gscale = grad_scale;
+    if (sparse) {
+        const SparseLayout SL = sparse_layout(d, max_gt);
+        a.pos_ent = reinterpret_cast<const uint32_t*>(reinterpret_cast<const char*>(ws) + SL.pos_ent);
+        a.entries = reinterpret_cast<const SparseEntry*>(reinterpret_cast<const char*>(ws) + SL.entries);
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    YB_DISPATCH_DTYPE(d->dtype, T, if constexpr (kHalf<T>) return loss_emit_launch<T>(a, sparse, st));
     return 0;
 }
 

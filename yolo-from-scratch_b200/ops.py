@@ -78,6 +78,29 @@ def _f32c(t: torch.Tensor, dev: torch.device) -> torch.Tensor:
     return t
 
 
+_HEAD_DTYPES = {torch.float32: _lib.DTYPE_F32, torch.bfloat16: _lib.DTYPE_BF16, torch.float16: _lib.DTYPE_F16}
+
+
+def _headc(t: torch.Tensor, dev: torch.device) -> torch.Tensor:
+    """A head tensor as the kernels read it: fp32, bf16 and fp16 keep their dtype (a CPU half tensor is staged as
+    half), any other dtype becomes fp32; contiguous, on `dev`, 16-byte aligned (differentiable)."""
+    if t.device != dev:
+        t = t.to(dev)
+    if t.dtype not in _HEAD_DTYPES:
+        t = t.float()
+    t = t.contiguous()
+    if t.data_ptr() % 16:
+        t = t.clone()
+    return t
+
+
+def _same_dtype(ts: List[torch.Tensor]) -> List[torch.Tensor]:
+    """Heads of mixed dtypes are all read as fp32."""
+    if len({t.dtype for t in ts}) > 1:
+        ts = [t.float() for t in ts]
+    return ts
+
+
 _anchor_cache = {}
 
 
@@ -122,8 +145,8 @@ class _DecodeFn(torch.autograd.Function):
     def forward(ctx, pred, anchors, img_size):
         B, H, W, A, row = pred.shape
         out = torch.empty_like(pred)
-        _lib.check(_lib.lib().yb_decode_fwd(pred.data_ptr(), anchors.data_ptr(), out.data_ptr(),
-                                            B, H, W, A, row - 5, float(img_size), _stream()), "yb_decode_fwd")
+        _lib.check(_lib.lib().yb_decode_fwd_t(pred.data_ptr(), anchors.data_ptr(), out.data_ptr(), B, H, W, A, row - 5,
+                                              float(img_size), _HEAD_DTYPES[pred.dtype], _stream()), "yb_decode_fwd_t")
         ctx.save_for_backward(pred, anchors)
         ctx.img_size = float(img_size)
         return out
@@ -132,22 +155,23 @@ class _DecodeFn(torch.autograd.Function):
     def backward(ctx, grad_out):
         pred, anchors = ctx.saved_tensors
         B, H, W, A, row = pred.shape
-        grad_out = _f32c(grad_out, pred.device)
+        grad_out = _headc(grad_out.to(pred.dtype), pred.device)
         grad_in = torch.empty_like(pred)
-        _lib.check(_lib.lib().yb_decode_bwd(pred.data_ptr(), anchors.data_ptr(), grad_out.data_ptr(),
-                                            grad_in.data_ptr(), B, H, W, A, row - 5, ctx.img_size, _stream()),
-                   "yb_decode_bwd")
+        _lib.check(_lib.lib().yb_decode_bwd_t(pred.data_ptr(), anchors.data_ptr(), grad_out.data_ptr(),
+                                              grad_in.data_ptr(), B, H, W, A, row - 5, ctx.img_size,
+                                              _HEAD_DTYPES[pred.dtype], _stream()), "yb_decode_bwd_t")
         return grad_in, None, None
 
 
 def decode_predictions(raw_preds: torch.Tensor, anchors, img_size=640) -> torch.Tensor:
     """train.py:712-779.  (B,H,W,A,5+nc) raw logits -> same shape with xywh decoded to
-    normalised coordinates; objectness/class logits unchanged.  Differentiable."""
+    normalised coordinates; objectness/class logits unchanged.  Differentiable.  bf16 / fp16 heads are
+    decoded natively: the result is the fp32 decode of the upcast heads rounded to the head dtype."""
     _check_head(raw_preds, "raw_preds")
     dev = _device()
     orig_dev, orig_dtype = raw_preds.device, raw_preds.dtype
     with torch.cuda.device(dev):
-        pred = _f32c(raw_preds, dev)
+        pred = _headc(raw_preds, dev)
         anc = _anchors_dev(anchors, dev)
         if anc.shape[0] != pred.shape[3]:
             raise ValueError("anchors must be (num_anchors, 2)")
@@ -225,6 +249,7 @@ def _fill_loss_desc(preds, tgts, ancs, grads, nc, obj_weights, coef, B_global=No
     d.nc = nc
     d.img_size = img_size
     d.eps = CIOU_EPS
+    d.dtype = _HEAD_DTYPES[preds[0].dtype]
     d.w_box, d.w_cls = BOX_WEIGHT, CLS_WEIGHT
     for s in range(S):
         d.H[s], d.W[s] = _grid(preds[s], layout)
@@ -238,20 +263,37 @@ def _fill_loss_desc(preds, tgts, ancs, grads, nc, obj_weights, coef, B_global=No
 
 
 def loss_forward_backward(preds, tgts, ancs, nc, obj_weights, want_grad, coef=None, group=None, equal_shards=True,
-                          b_global=None, reduce_fn=None, sparse=None, layout=LAYOUT_BHWAC):
+                          b_global=None, reduce_fn=None, sparse=None, layout=LAYOUT_BHWAC, grad_scale=None):
     """Run the fused kernels on device tensors.  Returns (out4, per_scale(S,3), grads list).
 
     `group`: optional torch.distributed process group; the batch is then a shard of a global
     batch and the S*4 partial sums are all-reduced once (SURVEY 8e) between the two stages.
     `sparse`: a `PackedLabels` — targets are assigned on the device from the label lists and handed
     to the loss in sparse form (SURVEY 8f-4); `tgts` is then ignored (pass None).
+    `grad_scale`: bf16 / fp16 heads only, an optional (1,) fp32 device tensor s; the gradients are then those
+    of s * total (what `GradScaler.scale(total).backward()` gives), rounded to the head dtype after the scaling.
     """
+    out4, per_scale, grads, emit = _loss_run(preds, tgts, ancs, nc, obj_weights, want_grad, coef, group, equal_shards,
+                                             b_global, reduce_fn, sparse, layout)
+    if emit is not None:
+        if grad_scale is None:
+            grad_scale = torch.ones(1, dtype=torch.float32, device=preds[0].device)
+        grads = _loss_emit(emit, grad_scale)
+    return out4, per_scale, grads
+
+
+def _loss_run(preds, tgts, ancs, nc, obj_weights, want_grad, coef=None, group=None, equal_shards=True, b_global=None,
+              reduce_fn=None, sparse=None, layout=LAYOUT_BHWAC):
+    """Both stages.  fp32 heads: (out4, per_scale, grads, None), the gradient written by stage 1.  Half heads:
+    (out4, per_scale, [None]*S, emit) where `emit` holds what `_loss_emit` needs to write the gradients later, once
+    the upstream gradient is known (None when no gradient is wanted)."""
     L = _lib.lib()
     S = len(preds)
     dev = preds[0].device
+    half = preds[0].dtype != torch.float32
     if coef is None:
         coef = [(BOX_WEIGHT, obj_weights[s], CLS_WEIGHT) for s in range(S)]
-    grads = [torch.empty_like(p) if w else None for p, w in zip(preds, want_grad)]
+    grads = [torch.empty_like(p) if w and not half else None for p, w in zip(preds, want_grad)]
     world = 1
     explicit = b_global
     b_global = preds[0].shape[0]
@@ -291,7 +333,22 @@ def loss_forward_backward(preds, tgts, ancs, nc, obj_weights, want_grad, coef=No
         allreduce_partials(partials, group)
     _lib.check(L.yb_loss_finalize(ctypes.byref(d), partials.data_ptr(), out4.data_ptr(), per_scale.data_ptr(),
                                   ws.data_ptr(), ws_bytes, st), "yb_loss_finalize")
-    return out4, per_scale, grads
+    emit = None
+    if half and any(want_grad):
+        # the tensors the emit pass reads (heads, dense targets, anchors) are referenced by d's pointers: keep them
+        emit = (d, partials, ws, -1 if sparse is None else sparse.max_gt, list(want_grad), (preds, tgts, ancs))
+    return out4, per_scale, grads, emit
+
+
+def _loss_emit(emit, grad_scale):
+    """Half heads: the gradients of grad_scale * total (grad_scale: (1,) fp32 on the device, read by the kernels)."""
+    d, partials, ws, max_gt, want, (preds, _, _) = emit
+    grads = [torch.empty_like(p) if w else None for p, w in zip(preds, want)]
+    for s, g in enumerate(grads):
+        d.grad[s] = _ptr(g)
+    _lib.check(_lib.lib().yb_loss_grad_emit(ctypes.byref(d), partials.data_ptr(), grad_scale.data_ptr(), max_gt,
+                                            ws.data_ptr(), ws.numel(), _stream()), "yb_loss_grad_emit")
+    return grads
 
 
 class _YoloLossFn(torch.autograd.Function):
@@ -306,12 +363,13 @@ class _YoloLossFn(torch.autograd.Function):
             group, sparse, layout = group
         preds, tgts, ancs = tensors[:S], tensors[S:2 * S], tensors[2 * S:3 * S]
         want = [ctx.needs_input_grad[4 + s] for s in range(S)]
-        out4, per_scale, grads = loss_forward_backward(preds, tgts, ancs, nc, obj_weights, want, group=group,
-                                                       sparse=sparse, layout=layout)
+        out4, per_scale, grads, emit = _loss_run(preds, tgts, ancs, nc, obj_weights, want, group=group, sparse=sparse,
+                                                 layout=layout)
         ctx.set_materialize_grads(False)
         ctx.sparse, ctx.layout = sparse, layout
         ctx.cfg = (nc, obj_weights, group, S, want)
-        ctx.fused_grads = grads
+        ctx.fused_grads = grads if emit is None else None
+        ctx.emit = emit   # half heads: the gradient is written in backward, after the upstream gradient is applied
         ctx.save_for_backward(*tensors)
         return out4[0], out4[1], out4[2], out4[3]
 
@@ -321,7 +379,13 @@ class _YoloLossFn(torch.autograd.Function):
         none = (None,) * 4
         if not any(want):
             return none + (None,) * (3 * S)
-        if g_bbox is None and g_obj is None and g_cls is None and ctx.fused_grads is not None:
+        if g_bbox is None and g_obj is None and g_cls is None and ctx.emit is not None:
+            tensors = ctx.saved_tensors
+            if g_total is None:
+                grads = [torch.zeros_like(p) if w else None for p, w in zip(tensors[:S], want)]
+            else:   # read on the device: no synchronisation
+                grads = _loss_emit(ctx.emit, g_total.detach().to(torch.float32).reshape(1).contiguous())
+        elif g_bbox is None and g_obj is None and g_cls is None and ctx.fused_grads is not None:
             grads = ctx.fused_grads
             if g_total is None:
                 grads = [None if g is None else torch.zeros_like(g) for g in grads]
@@ -342,7 +406,7 @@ class _YoloLossFn(torch.autograd.Function):
             coef = [(BOX_WEIGHT * gt_ + gb_, obj_weights[s] * gt_ + go_, CLS_WEIGHT * gt_ + gc_) for s in range(S)]
             _, _, grads = loss_forward_backward(preds, tgts, ancs, nc, obj_weights, want, coef=coef, group=group,
                                                 sparse=ctx.sparse, layout=ctx.layout)
-        ctx.fused_grads = None
+        ctx.fused_grads = ctx.emit = None
         return none + tuple(grads) + (None,) * (2 * S)
 
 
@@ -368,10 +432,13 @@ def _loss_common(predictions, targets, anchors_list, num_classes, obj_weights, g
                     raise ValueError(f"scale {s}: predictions {tuple(predictions[s].shape)} vs targets {tuple(targets[s].shape)}")
                 if predictions[s].shape[4] != 5 + num_classes:
                     raise ValueError(f"scale {s}: last dim {predictions[s].shape[4]} != 5+num_classes")
-            preds.append(_f32c(predictions[s], dev))
+            preds.append(_headc(predictions[s], dev))
             # sparse targets: a placeholder keeps the autograd signature (preds, targets, anchors) x S
             tgts.append(_f32c(targets[s].detach(), dev) if sparse is None else preds[-1].detach())
             ancs.append(_anchors_dev(anchors_list[s], dev))
+        preds = _same_dtype(preds)
+        if sparse is not None:
+            tgts = [p.detach() for p in preds]
         packed_cfg = group if (sparse is None and layout == LAYOUT_BHWAC) else (group, sparse, layout)
         outs = _YoloLossFn.apply(int(num_classes), tuple(float(w) for w in obj_weights), packed_cfg, S,
                                  *preds, *tgts, *ancs)
@@ -606,6 +673,7 @@ def _heads_desc(preds, ancs, img_size, nc, layout=LAYOUT_BHWAC):
     d.S, d.B, d.A, d.nc = len(preds), preds[0].shape[0], ancs[0].shape[0], nc
     d.img_size = float(img_size)
     d.layout = layout
+    d.dtype = _HEAD_DTYPES[preds[0].dtype]
     for s, p in enumerate(preds):
         d.H[s], d.W[s] = _grid(p, layout)
         d.pred[s] = p.data_ptr()
@@ -617,6 +685,7 @@ def filter_candidates(predictions, anchors_list, img_size, num_classes=1, conf_t
                       layout=LAYOUT_BHWAC):
     """Per-scale body of predict() (train.py:1152-1229) for a batch: decode, sigmoid, objectness
     filter, class max, pixel xyxy with letterbox reverse, score; P3->P4->P5 order preserved.
+    bf16 / fp16 heads are read natively; the candidates are those of the fp32 filter on the upcast heads.
 
     letterbox: (B,3) [scale, pad_top, pad_left] or None.
     Returns (boxes (B,cap,4), scores (B,cap), classes (B,cap) int64, counts (B,) int32) on the GPU,
@@ -625,7 +694,7 @@ def filter_candidates(predictions, anchors_list, img_size, num_classes=1, conf_t
     dev = _device()
     S = len(predictions)
     with torch.cuda.device(dev):
-        preds = [_f32c(p.detach(), dev) for p in predictions]
+        preds = _same_dtype([_headc(p.detach(), dev) for p in predictions])
         ancs = [_anchors_dev(a, dev) for a in anchors_list[:S]]
         for s, p in enumerate(preds):
             if layout == LAYOUT_NCHW:
@@ -1115,16 +1184,28 @@ class HotPathGraph:
       targets[s] dense (B,G,G,A,5+nc) (targets="dense": the reference's call signature)
     Static outputs: losses (4,) [total, bbox, obj, cls], grads[s] (gradient of `total`), det (the
     detect_batch dict), rows (B*cap,6) + offsets (B+1,) from pack_detections.
-    An image whose NMS graph overflows the edge list is resolved exactly inside the same launch."""
+    An image whose NMS graph overflows the edge list is resolved exactly inside the same launch.
+
+    dtype: element type of the static heads and gradients, torch.float32, torch.bfloat16 or torch.float16.  A half
+    graph also owns `grad_scale`, a (1,) fp32 device tensor (1.0 at first) that the captured kernels read at every
+    replay: grads[s] are the gradients of grad_scale * total, rounded to dtype after the scaling — what
+    `scaler.scale(total).backward()` gives.  Copy a GradScaler's scale into it between replays."""
 
     def __init__(self, batch, img_size, num_classes, anchors_list, conf_threshold=0.5, iou_threshold=0.4, max_gt=50,
                  targets="labels", layout=LAYOUT_BHWAC, num_anchors=3, device=None, adopt_heads=None,
-                 adopt_targets=None, group=None, overlap_loss=True, fork_loss="auto"):
+                 adopt_targets=None, group=None, overlap_loss=True, fork_loss="auto", dtype=torch.float32):
         """adopt_heads / adopt_targets: existing device tensors (or a PackedLabels) to use as the static
         inputs instead of allocating new ones.  group: torch.distributed process group of an image-sharded
         job; the all-reduce of the loss partials is then captured inside the graph (NCCL).
         overlap_loss: the loss kernels (HBM-bound, few resident warps) and the filter/NMS kernels (issue-bound)
         are independent readers of the heads; they are captured as two parallel branches of the graph."""
+        if dtype not in _HEAD_DTYPES:
+            raise ValueError(f"dtype must be torch.float32, torch.bfloat16 or torch.float16, got {dtype}")
+        if adopt_heads is not None:
+            for s, h in enumerate(adopt_heads):
+                if h.dtype != dtype:
+                    raise ValueError(f"adopt_heads[{s}] is {h.dtype}, the graph's dtype is {dtype}")
+        self.dtype = dtype
         self.group = group
         self.overlap_loss = bool(overlap_loss)
         if fork_loss not in ("auto", "start", "after_filter"):
@@ -1140,9 +1221,10 @@ class HotPathGraph:
             if adopt_heads is not None:
                 self.heads = list(adopt_heads)
             elif layout == LAYOUT_NCHW:
-                self.heads = [torch.zeros(batch, A * row, g, g, device=dev) for g in grids]
+                self.heads = [torch.zeros(batch, A * row, g, g, device=dev, dtype=dtype) for g in grids]
             else:
-                self.heads = [torch.zeros(batch, g, g, A, row, device=dev) for g in grids]
+                self.heads = [torch.zeros(batch, g, g, A, row, device=dev, dtype=dtype) for g in grids]
+            self.grad_scale = None if dtype == torch.float32 else torch.ones(1, dtype=torch.float32, device=dev)
             self.labels = self.targets = None
             if adopt_targets is not None:
                 if isinstance(adopt_targets, PackedLabels):
@@ -1182,7 +1264,7 @@ class HotPathGraph:
     def _loss(self):
         out4, _, grads = loss_forward_backward(self.heads, self.targets, self.anchors, self.nc, MULTISCALE_OBJ_WEIGHTS,
                                                [True] * len(self.heads), sparse=self.labels, layout=self.layout,
-                                               group=self.group)
+                                               group=self.group, grad_scale=self.grad_scale)
         return out4, grads
 
     def _step(self):
