@@ -396,6 +396,35 @@ int yb_coco_precision(const yb_coco_record* records, const long long* seg, const
                       int A, int T, const double* recall_thr, int R, const int* max_dets, int M,
                       double* precision, double* recall, int* status, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Validation report (confusion matrix, images per class, confidence histograms of the P/R/F1 curves)
+ *   yb_report_match, once per batch, after yb_map_match on the same batch and stream, one CTA per image.
+ *   Detections, ground truths (corners, classes, nc == 1 -> class 0), the IoU and the status bits are yb_map_match's;
+ *   records are the (B, min(max_det,cap)) records yb_map_match just wrote for this batch.
+ *   Confusion matrix (nc+1, nc+1) int64, row = predicted class, column = true class, index nc = background:
+ *     D = the first min(n_keep[b], max_det) keep entries with a class in [0,nc) and (double)score > cm_conf (a NaN
+ *       score never passes); G = the ground truths with a class in [0,nc).  The matching is class-agnostic:
+ *     step 1: each d in D picks the g with the largest IoU among those with IoU > cm_iou (strict; a NaN IoU never
+ *       matches), the lower g on equal IoU;
+ *     step 2: each g picked by some d keeps the d with the largest IoU, the earlier keep position on equal IoU;
+ *     confusion[cls_d][cls_g] += 1 per kept pair, [nc][cls_g] += 1 per g nobody picked, [cls_d][nc] += 1 per d not
+ *       kept.  (The Ultralytics ConfusionMatrix's layout and two-step unique matching; the tie rules and the
+ *       counting of unmatched detections are defined here, not claimed equal to any Ultralytics release.)
+ *   images (nc) int64 += 1 per class with at least one ground truth in the image.
+ *   det_hist / tp_hist (nc, K) int64: each record with class c >= 0 and a non-NaN score s, with
+ *     j = #{k : grid[k] < (double)s} - 1 >= 0, adds 1 to det_hist[c][j], and to tp_hist[c][j] when its TP bit t_curve
+ *     is set.  The suffix sum over j >= k is the number of detections (TPs) with score > grid[k].
+ *   grid: DEVICE array of K strictly ascending finite doubles (not checked here); cm_conf, cm_iou finite.
+ *   The caller zeroes every output once per evaluation; they accumulate over batches.
+ *   The ground truths (48 B each), 16 B per detection slot and nc * 4 bytes must fit one CTA's shared memory
+ *   (YB_EINVAL otherwise).  *status |= YB_MAP_BAD_CLASS, YB_MAP_NMS_FAILED as yb_map_match.
+ * ---------------------------------------------------------------------------------------- */
+int yb_report_match(const float* boxes, const float* scores, const int64_t* classes, const int64_t* keep,
+                    const int* n_keep, int B, int cap, int max_det, const double* labels, const int* n_gt,
+                    const double* letterbox, int max_gt, int nc, const yb_map_record* records, int t_curve,
+                    const double* grid, int K, double cm_conf, double cm_iou, long long* confusion,
+                    long long* images, long long* det_hist, long long* tp_hist, int* status, void* stream);
+
 /* Per-launch CUDA-event timing for bench.py: when enabled every kernel launch of the library is
  * bracketed by two events on its stream; yb_timing_collect synchronises them, writes
  * "name count total_ms" lines into buf (NUL terminated, truncated to n) and resets. */

@@ -7,7 +7,7 @@ into the reference's `train` module (install.py).
 """
 from . import _lib
 from .ops import (COCO_AREA_LABELS, COCO_AREA_RANGES, COCO_IOU_THRESHOLDS, COCO_MAX_DETS, COCO_RECALL_THRESHOLDS,
-                  COCODetectionEval, DetectionMAP, format_coco_stats, batched_nms, batched_nms_padded, build_targets, ciou_loss, compute_anchor_iou,
+                  COCODetectionEval, DetectionMAP, DetectionReport, format_coco_stats, format_detection_report, batched_nms, batched_nms_padded, build_targets, ciou_loss, compute_anchor_iou,
                   decode_predictions, default_anchors, detect_batch, detect_batch_nchw, detections_to_lists, heads_from_nchw, eval_counts, eval_epoch,
                   filter_candidates,
                   loss_forward_backward, nms, nms_retry_overflow, pack_detections, predict_heads,
@@ -22,4 +22,5 @@ __all__ = [
     "detect_batch_nchw", "heads_from_nchw", "predict_heads", "HotPathGraph", "LAYOUT_BHWAC", "LAYOUT_NCHW", "default_anchors",
     "DetectionMAP", "COCO_IOU_THRESHOLDS", "COCO_RECALL_THRESHOLDS",
     "COCODetectionEval", "COCO_AREA_RANGES", "COCO_AREA_LABELS", "COCO_MAX_DETS", "format_coco_stats",
+    "DetectionReport", "format_detection_report",
 ]

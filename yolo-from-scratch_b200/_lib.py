@@ -95,6 +95,9 @@ SIGNATURES = {
                               c_void_p, c_void_p]),
     "yb_coco_precision": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, POINTER(c_int),
                                   c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "yb_report_match": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p,
+                                c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_int, c_double, c_double,
+                                c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
 }
 
 _lib = None

@@ -318,13 +318,6 @@ __global__ void __launch_bounds__(kCocoPrecThreads) coco_precision_kernel(const 
     }
 }
 
-static int max_smem_optin() {
-    int dev = 0, v = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&v, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess)
-        return 48 * 1024;
-    return v;
-}
-
 }  // namespace yb
 
 extern "C" int yb_coco_match(const float* boxes, const float* scores, const int64_t* classes, const int64_t* keep,

@@ -1,8 +1,17 @@
-// yb_iou.cuh — the fp64 ground-truth box and corner IoU shared by the mAP (yb_map.cu) and COCO (yb_coco.cu) kernels.
+// yb_iou.cuh — the fp64 ground-truth box and corner IoU shared by the mAP (yb_map.cu), COCO (yb_coco.cu) and
+// validation report (yb_report.cu) kernels, and the shared-memory limit their hosts check the staging against.
 #pragma once
 #include "yb_common.cuh"
 
 namespace yb {
+
+// the current device's opt-in shared memory per block (48 KB if it cannot be read)
+static inline int max_smem_optin() {
+    int dev = 0, v = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&v, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess)
+        return 48 * 1024;
+    return v;
+}
 
 struct GtBox {
     double x1, y1, x2, y2;

@@ -101,7 +101,7 @@ def _make_predict(train_module):
 
 def _evaluate_dataset(train_module, metric, model, dataset, device, num_classes, conf_threshold, iou_threshold,
                       batch_size):
-    """Feed `metric` (DetectionMAP or COCODetectionEval) the detections of `model` on `dataset` (its imgs and labels
+    """Feed `metric` (DetectionMAP, COCODetectionEval or DetectionReport) the detections of `model` on `dataset` (its imgs and labels
     lists) batch by batch and return metric.compute().  Images are loaded and letterboxed by the module's own Image
     and letterbox_resize, as predict() does (train.py:1134-1138)."""
     import numpy as np
@@ -154,6 +154,20 @@ def _make_evaluate_coco(train_module):
     return evaluate_coco
 
 
+def _make_evaluate_report(train_module):
+    """`evaluate_report`, a name the reference does not have: the validation report of a model over a YOLODataset's
+    images and label files (ops.DetectionReport)."""
+    def evaluate_report(model, dataset, device, num_classes=1, conf_threshold=0.001, iou_threshold=0.4, batch_size=8,
+                        max_det=300):
+        """Confusion matrix, P/R/F1 curves over the confidence threshold, best-F1 threshold and the AP columns of
+        `model` on `dataset` (its imgs and labels lists).  Returns DetectionReport.compute()'s dict;
+        ops.format_detection_report(out) gives the per-class table."""
+        metric = ops.DetectionReport(num_classes, max_det=max_det)
+        return _evaluate_dataset(train_module, metric, model, dataset, device, num_classes, conf_threshold,
+                                 iou_threshold, batch_size)
+    return evaluate_report
+
+
 def channels_last_heads(model):
     """SURVEY 8f-2 for the UNCHANGED model: run the network in NHWC (`torch.channels_last`).  The head convs
     then write (B, H, W, A*(5+nc)) in memory, on which train.py:608-609's view/permute is a pure stride change and
@@ -201,8 +215,9 @@ def install(train_module, patch_torchvision=False, patch_dataset=True, patch_eva
     channels_last (default: environment YOLO_B200_CHANNELS_LAST=1) makes every `train.YOLO` built afterwards
     run in NHWC, so that the head layout conversion of train.py:608-609 costs nothing (channels_last_heads).
     patch_eval also swaps `eval_epoch` (SURVEY 8f-1: its per-anchor python loop becomes one kernel);
-    patch_predict swaps `predict` and adds `predict_batch` (SURVEY 8f-3); `evaluate_map` (COCO-style mAP) and
-    `evaluate_coco` (COCO's twelve bbox stats), names the reference does not have, are always added; patch_torchvision additionally
+    patch_predict swaps `predict` and adds `predict_batch` (SURVEY 8f-3); `evaluate_map` (COCO-style mAP),
+    `evaluate_coco` (COCO's twelve bbox stats) and `evaluate_report` (confusion matrix, P/R/F1 curves, per-class
+    table), names the reference does not have, are always added; patch_torchvision additionally
     rebinds torchvision.ops.batched_nms process-wide (off by default: predict no longer needs it)."""
     if getattr(train_module, _MARK, False):
         return train_module
@@ -222,6 +237,9 @@ def install(train_module, patch_torchvision=False, patch_dataset=True, patch_eva
     if not hasattr(train_module, "evaluate_coco"):
         saved["evaluate_coco"] = None
         train_module.evaluate_coco = _make_evaluate_coco(train_module)
+    if not hasattr(train_module, "evaluate_report"):
+        saved["evaluate_report"] = None
+        train_module.evaluate_report = _make_evaluate_report(train_module)
     if patch_dataset and hasattr(train_module, "YOLODataset"):
         cls = train_module.YOLODataset
         saved["YOLODataset.__getitem__"] = cls.__getitem__
@@ -260,6 +278,8 @@ def uninstall(train_module):
         del train_module.evaluate_map
     if "evaluate_coco" in saved:
         del train_module.evaluate_coco
+    if "evaluate_report" in saved:
+        del train_module.evaluate_report
     if "YOLODataset.__getitem__" in saved:
         train_module.YOLODataset.__getitem__ = saved["YOLODataset.__getitem__"]
         train_module.YOLODataset.compute_anchor_iou = saved["YOLODataset.compute_anchor_iou"]

@@ -14,6 +14,7 @@ include/yolo_b200.h).  PyTorch is used only for device memory, streams and autog
   nms / batched_nms       torchvision.ops as called at train.py:1232-1233
   detect_batch            filter_candidates + batched_nms + gather (predict :1152-1238 for a batch)
   DetectionMAP            COCO-style mAP of detect_batch's detections (new; no reference equivalent)
+  DetectionReport         confusion matrix, P/R/F1 over confidence, best-F1 threshold, per-class table (new)
 
 CPU tensors are accepted (the reference's tests pass CPU tensors): they are staged to the GPU,
 computed there, and staged back.  That is staging, not a fallback: without CUDA every function
@@ -988,23 +989,38 @@ class DetectionMAP:
         """{map, map50, ap (nc,T), precision (T,R,nc), recall (T,nc), n_gt (nc), n_det (nc)} on the host (float64 /
         int64; map50 is None when 0.5 is not a threshold).  Entries of a class without ground truth are -1, and
         map / map50 are the means of the entries > -1 (-1 when there are none), as COCOeval.summarize."""
+        with torch.cuda.device(self.device):
+            host = torch.cat(self._compute_device()).cpu().numpy()   # the one synchronisation
+        return self._compute_host(host, "DetectionMAP")
+
+    def _compute_device(self):
+        """Device half of compute(): sort the records and run the precision kernel.  Returns the flat float64 device
+        tensors compute() copies back, in the order _compute_host reads them (the status word last)."""
         T, R, nc = len(self.iou_thresholds), len(self.recall_thresholds), self.nc
         dev = self.device
-        with torch.cuda.device(dev):
-            rec = torch.cat(self._records) if self._records else torch.empty(0, 3, dtype=torch.int32, device=dev)
-            rec, seg = _sort_records(rec, nc)
-            n = rec.shape[0]
-            ws_bytes = _lib.lib().yb_map_workspace_bytes(n, self._gt_total, T)
-            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-            precision = torch.empty(T, R, nc, dtype=torch.float64, device=dev)
-            recall = torch.empty(T, nc, dtype=torch.float64, device=dev)
-            _lib.check(_lib.lib().yb_map_precision(rec.data_ptr(), seg.data_ptr(), self._gt_count.data_ptr(), nc, T,
-                                                   self._rec_thr.data_ptr(), R, precision.data_ptr(), recall.data_ptr(),
-                                                   ws.data_ptr(), ws_bytes, self._status.data_ptr(), _stream()),
-                       "yb_map_precision")
-            host = torch.cat([precision.reshape(-1), recall.reshape(-1), self._gt_count.double(), seg.double(),
-                              self._status.double()]).cpu().numpy()   # the one synchronisation
-        _raise_status(int(host[-1]), "DetectionMAP")
+        rec = torch.cat(self._records) if self._records else torch.empty(0, 3, dtype=torch.int32, device=dev)
+        rec, seg = _sort_records(rec, nc)
+        n = rec.shape[0]
+        ws_bytes = _lib.lib().yb_map_workspace_bytes(n, self._gt_total, T)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        precision = torch.empty(T, R, nc, dtype=torch.float64, device=dev)
+        recall = torch.empty(T, nc, dtype=torch.float64, device=dev)
+        _lib.check(_lib.lib().yb_map_precision(rec.data_ptr(), seg.data_ptr(), self._gt_count.data_ptr(), nc, T,
+                                               self._rec_thr.data_ptr(), R, precision.data_ptr(), recall.data_ptr(),
+                                               ws.data_ptr(), ws_bytes, self._status.data_ptr(), _stream()),
+                   "yb_map_precision")
+        return [precision.reshape(-1), recall.reshape(-1), self._gt_count.double(), seg.double(), self._status.double()]
+
+    def _host_size(self):
+        """Number of doubles _compute_device's tensors hold."""
+        T, R, nc = len(self.iou_thresholds), len(self.recall_thresholds), self.nc
+        return T * R * nc + T * nc + nc + nc + 1 + 1
+
+    def _compute_host(self, host, who):
+        """Host half of compute(): raise on the status bits, unpack the first _host_size() doubles of `host` and
+        summarise them."""
+        T, R, nc = len(self.iou_thresholds), len(self.recall_thresholds), self.nc
+        _raise_status(int(host[self._host_size() - 1]), who)
         o = 0
         precision = host[o:o + T * R * nc].reshape(T, R, nc); o += T * R * nc
         recall = host[o:o + T * nc].reshape(T, nc); o += T * nc
@@ -1168,6 +1184,151 @@ def format_coco_stats(stats, iou_thresholds=COCO_IOU_THRESHOLDS, max_dets=COCO_M
     return [line.format("Average Precision" if ap else "Average Recall", "(AP)" if ap else "(AR)",
                         every if thr is None else "{:0.2f}".format(thr), area, m, float(v))
             for (ap, thr, area, m), v in zip(rows, stats)]
+
+
+# --------------------------------------------------------------------------------------------
+# validation report: confusion matrix, P/R/F1 over the confidence threshold, per-class table
+# --------------------------------------------------------------------------------------------
+DEFAULT_CONF_GRID = tuple(np.linspace(0.0, 1.0, 1000).tolist())
+
+
+class DetectionReport:
+    """The validation report YOLO tools print, of the kept detections of `detect_batch`, accumulated over batches on
+    the device: a confusion matrix with a background row and column, precision / recall / F1 curves over the
+    confidence threshold at IoU `curve_iou`, the threshold with the best mean F1, and DetectionMAP's AP columns for a
+    per-class table (format_detection_report).  include/yolo_b200.h states the matrix and histogram semantics.
+
+    conf_grid: the thresholds of the curves, strictly ascending and finite; a detection counts at grid[k] when its
+    score is > grid[k].  cm_conf / cm_iou: the matrix's score and IoU thresholds (both strict).
+
+    update(det, labels) runs DetectionMAP.update and one report kernel on the records it wrote; it never
+    synchronises.  compute() runs DetectionMAP's compute path plus the histograms' suffix sums and synchronises
+    once."""
+
+    def __init__(self, num_classes, max_det=300, iou_thresholds=COCO_IOU_THRESHOLDS, conf_grid=DEFAULT_CONF_GRID,
+                 curve_iou=0.5, cm_conf=0.25, cm_iou=0.45):
+        self.map = DetectionMAP(num_classes, iou_thresholds=iou_thresholds, max_det=max_det)
+        self.nc = self.map.nc
+        self.conf_grid = np.asarray(conf_grid, dtype=np.float64).reshape(-1)
+        self.curve_iou, self.cm_conf, self.cm_iou = float(curve_iou), float(cm_conf), float(cm_iou)
+        hit = np.flatnonzero(self.map.iou_thresholds == self.curve_iou)
+        if hit.size == 0:
+            raise ValueError(f"curve_iou={curve_iou} is not one of iou_thresholds {self.map.iou_thresholds.tolist()}")
+        self._t_curve = int(hit[0])
+        if (self.conf_grid.size < 1 or not np.all(np.isfinite(self.conf_grid))
+                or not np.all(np.diff(self.conf_grid) > 0)):
+            raise ValueError("conf_grid must be a non-empty, strictly ascending sequence of finite values")
+        if not (np.isfinite(self.cm_conf) and np.isfinite(self.cm_iou)):
+            raise ValueError("cm_conf and cm_iou must be finite")
+        nc, K, dev = self.nc, self.conf_grid.size, self.map.device
+        with torch.cuda.device(dev):
+            self._grid = torch.tensor(self.conf_grid, dtype=torch.float64, device=dev)
+            # one buffer, zeroed at once: confusion (nc+1)^2, images (nc), det_hist (nc,K), tp_hist (nc,K)
+            self._counts = torch.zeros((nc + 1) ** 2 + nc + 2 * nc * K, dtype=torch.int64, device=dev)
+        # compute()'s one copy back goes to page-locked memory: about 16 bytes per class and grid point
+        self._host = torch.empty(self.map._host_size() + (nc + 1) ** 2 + nc + 2 * nc * K, dtype=torch.float64,
+                                 pin_memory=True)
+        o = 0
+        self._confusion = self._counts[o:o + (nc + 1) ** 2].view(nc + 1, nc + 1); o += (nc + 1) ** 2
+        self._images = self._counts[o:o + nc]; o += nc
+        self._det_hist = self._counts[o:o + nc * K].view(nc, K); o += nc * K
+        self._tp_hist = self._counts[o:o + nc * K].view(nc, K)
+        self.reset()
+
+    def reset(self):
+        """Forget every batch seen so far."""
+        self.map.reset()
+        self.images_total = 0
+        with torch.cuda.device(self.map.device):
+            self._counts.zero_()
+
+    def update(self, det, labels: PackedLabels):
+        """Match one batch: the arguments of DetectionMAP.update.  After an error, reset() before the next update."""
+        self.map.update(det, labels)
+        boxes, keep = det["boxes"], det["keep"]
+        B, cap = boxes.shape[0], boxes.shape[1]
+        with torch.cuda.device(self.map.device):
+            _lib.check(_lib.lib().yb_report_match(
+                boxes.data_ptr(), det["scores"].data_ptr(), det["classes"].data_ptr(), keep.data_ptr(),
+                det["n_keep"].data_ptr(), B, cap, self.map.max_det, labels.labels.data_ptr(), labels.n_gt.data_ptr(),
+                labels.letterbox.data_ptr(), labels.max_gt, self.nc, self.map._records[-1].data_ptr(), self._t_curve,
+                self._grid.data_ptr(), self.conf_grid.size, self.cm_conf, self.cm_iou, self._confusion.data_ptr(),
+                self._images.data_ptr(), self._det_hist.data_ptr(), self._tp_hist.data_ptr(),
+                self.map._status.data_ptr(), _stream()), "yb_report_match")
+        self.images_total += B
+
+    def compute(self):
+        """DetectionMAP.compute()'s dict plus, on the host:
+        px (K,) the grid; p_curve, r_curve, f1_curve (nc,K) at curve_iou (P = TP/D, 1 where D = 0; R = TP/n_gt;
+        F1 = 2PR/(P+R), 0 where P+R = 0; rows of classes without ground truth -1); best_conf = px[k*] with k* the
+        first arg-max of the mean F1 over the classes with ground truth (None when there are none); p, r, f1 (nc,)
+        at k*; confusion (nc+1,nc+1) and images (nc) int64; images_total; iou_thresholds (the columns of ap)."""
+        nc, K = self.nc, self.conf_grid.size
+        m = self.map._host_size()
+        with torch.cuda.device(self.map.device):
+            hist = self._counts[(nc + 1) ** 2 + nc:].view(2, nc, K)   # det_hist, tp_hist
+            rev = hist.flip(2).cumsum(2)   # [.., K-1-k] = detections / TPs with score > grid[k]
+            dev = torch.cat(self.map._compute_device() + [self._counts[:(nc + 1) ** 2 + nc].double(),
+                                                          rev.reshape(-1).double()])
+            self._host.copy_(dev, non_blocking=True)
+            torch.cuda.current_stream().synchronize()   # the one synchronisation
+        host = self._host.numpy()
+        out = self.map._compute_host(host[:m].copy(), "DetectionReport")   # its tables are returned as views
+        o = m
+        confusion = host[o:o + (nc + 1) ** 2].astype(np.int64).reshape(nc + 1, nc + 1); o += (nc + 1) ** 2
+        images = host[o:o + nc].astype(np.int64); o += nc
+        n_det = host[o:o + nc * K].astype(np.int64).reshape(nc, K)[:, ::-1]; o += nc * K
+        n_tp = host[o:o + nc * K].astype(np.int64).reshape(nc, K)[:, ::-1]
+        out.update(report_curves(n_det, n_tp, out["n_gt"], self.conf_grid), confusion=confusion, images=images,
+                   images_total=self.images_total, iou_thresholds=self.map.iou_thresholds.copy())
+        return out
+
+
+def report_curves(n_det, n_tp, n_gt, px):
+    """px, p_curve, r_curve, f1_curve, best_conf, p, r, f1 (DetectionReport.compute's fields) from the detections
+    n_det (nc,K) and TPs n_tp (nc,K) with score > px[k] and the ground truths n_gt (nc) per class."""
+    tp, d = n_tp.astype(np.float64), n_det.astype(np.float64)
+    n = np.asarray(n_gt, dtype=np.float64)[:, None]
+    has_gt = np.asarray(n_gt) > 0
+    with np.errstate(divide="ignore", invalid="ignore"):   # 0/0 where D = 0, P + R = 0 or n_gt = 0: replaced
+        p = tp / d
+        p[d == 0] = 1.0
+        r = tp / n
+        s = p + r
+        f1 = 2 * p * r / s
+    f1[s == 0] = 0.0
+    p[~has_gt], r[~has_gt], f1[~has_gt] = -1.0, -1.0, -1.0
+    if has_gt.any():
+        k = int(np.argmax(f1[has_gt].mean(axis=0)))
+        best_conf = float(px[k])
+        at = (p[:, k].copy(), r[:, k].copy(), f1[:, k].copy())
+    else:
+        best_conf = None
+        at = tuple(np.full(len(has_gt), -1.0) for _ in range(3))
+    return {"px": np.asarray(px, dtype=np.float64).copy(), "p_curve": p, "r_curve": r, "f1_curve": f1,
+            "best_conf": best_conf, "p": at[0], "r": at[1], "f1": at[2]}
+
+
+def format_detection_report(out, names=None):
+    """The per-class table of DetectionReport.compute()'s dict `out`, as YOLO validators print it: a header, an
+    `all` row (images, ground truths, mean P and R at best_conf over the classes with ground truth, map50, map) and
+    one row per class with ground truth (its images, ground truths, P, R, AP50, AP50-95).  names: class names
+    (default: the class indices).  A value that does not exist (no class with ground truth, no 0.5 threshold) is
+    printed as -1."""
+    n_gt, ap = np.asarray(out["n_gt"]), np.asarray(out["ap"])
+    has_gt = n_gt > 0
+    mean = lambda v: float(np.mean(v[has_gt])) if has_gt.any() else -1.0
+    hit = np.flatnonzero(np.asarray(out["iou_thresholds"]) == 0.5)
+    neg = lambda v: -1.0 if v is None else v
+    row = "%22s" + "%11i" * 2 + "%11.3g" * 4
+    lines = [("%22s" + "%11s" * 6) % ("Class", "Images", "Instances", "P", "R", "mAP50", "mAP50-95"),
+             row % ("all", out["images_total"], int(n_gt.sum()), mean(out["p"]), mean(out["r"]), neg(out["map50"]),
+                    out["map"])]
+    for c in np.flatnonzero(has_gt):
+        name = str(names[c]) if names is not None else str(c)
+        lines.append(row % (name, out["images"][c], n_gt[c], out["p"][c], out["r"][c],
+                            ap[c, hit[0]] if hit.size else -1.0, ap[c].mean()))
+    return lines
 
 
 # --------------------------------------------------------------------------------------------
