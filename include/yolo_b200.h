@@ -317,6 +317,12 @@ int yb_eval_counts(const yb_heads_desc* d, const float* const* targets_host, dou
  *   descending), keeping image order (batch after batch, then batch position) and keep order among equal
  *   scores — COCO's argsort(-scores, kind="mergesort") over the images in order; class -1 last.  ops.py does it
  *   with one torch.sort(stable=True) on an int64 key.  seg (nc+1) int64: class c is records [seg[c], seg[c+1]).
+ *   Image-sharded runs (ops' compute(group), dist.gather_eval_state): each rank runs stage 1 on its images, and
+ *   the records of ranks 0, 1, ... are concatenated before the sort, gt_count summed and status ORed.  When rank r
+ *   holds the r-th contiguous block of images in image order this is exactly one process's order, so the tables
+ *   are bit-identical.  With any other assignment (an interleaving sampler) the counts are still identical and the
+ *   precision table can differ only through the order of equal-score records of different images.  The same holds
+ *   for yb_coco_precision's records and yb_report_match's counts below.
  * Stage 2, yb_map_precision, once per evaluation, one CTA per class:
  *   tp, fp = cumulative counts (doubles), rc = tp / n_gt_c, pr = tp / (fp + tp + 2^-52);
  *   precision[t][r][c] = max of pr over positions with rc >= recall_thr[r] (0 if none), recall[t][c] = rc at the

@@ -6,10 +6,20 @@ produces S x {sum(1-CIoU), n_pos, sum BCE_obj, sum BCE_cls} for its images and o
 of those S*4 doubles (96 bytes for three scales) gives the global values; the objectness normaliser
 B_global*H*W*A is known without communication and the positive rows' gradients are scaled by the
 reduced 1/n_pos afterwards (yb_loss_finalize).  One process per GPU, torch.distributed / NCCL.
+
+Evaluation shards the same way: every rank matches its own images (DetectionMAP / COCODetectionEval /
+DetectionReport.update), and compute(group) merges the ranks' records and counts with gather_eval_state before
+the one sort and precision pass (DESIGN §3.11).
 """
 from typing import Tuple
 
 import torch
+
+# The configuration words of gather_eval_state's header, which must be equal on every rank.  gather_eval_state
+# appends the record width and the number of counts, which size its own collectives.
+FINGERPRINT_FIELDS = ("metric", "nc", "T", "R", "A", "M", "K", "max_det", "crc")
+_CHECKED = FINGERPRINT_FIELDS + ("record width", "counts")
+_ROWS, _GT_TOTAL, _IMAGES_TOTAL, _STATUS = range(len(_CHECKED), len(_CHECKED) + 4)
 
 
 def shard_range(n_images: int, rank: int, world: int) -> Tuple[int, int]:
@@ -48,3 +58,59 @@ def yolo_loss_multiscale_sharded(predictions, targets, anchors_list, num_classes
     S = min(len(predictions), len(targets), len(anchors_list), len(ops.MULTISCALE_OBJ_WEIGHTS))
     return ops._loss_common(list(predictions[:S]), list(targets[:S]), list(anchors_list[:S]), num_classes,
                             ops.MULTISCALE_OBJ_WEIGHTS[:S], group=group)
+
+
+def gather_eval_state(fingerprint, records, counts, gt_total, images_total, status, group=None):
+    """Merge an evaluation metric's accumulated state over the ranks of `group`.  A collective: every rank calls it.
+
+    fingerprint: len(FINGERPRINT_FIELDS) ints describing the metric's configuration; records (n, W) int32, the local
+    records in image order (word 1 is the class, -1 for an unused row); counts: the fixed-size int64 counts (any
+    shape); gt_total, images_total: host ints; status: (1,) int32 status word.  The tensors live on one device, CUDA
+    for NCCL, CUDA or CPU for gloo.
+
+    Step 1 gathers a fixed-size int64 header (the fingerprint, W, counts.numel(), n, gt_total, images_total, status)
+    and reads it on the host, the one synchronisation here.  If any rank's configuration words differ from rank 0's,
+    every rank raises ValueError before any variable-size collective, so none is left waiting.  Step 2 gathers the
+    counts and, unless every rank has n = 0, the records padded to the largest n with rows of -1 (class -1).
+
+    Returns (records, counts, gt_total, images_total, status) as one process holding every rank's updates would
+    hold them: the records of rank 0, 1, ... concatenated without the padding, counts summed (counts' shape),
+    gt_total and images_total summed, status the OR of the words, as a (1,) tensor like `status`.  The inputs are
+    not changed."""
+    import torch.distributed as dist
+    fingerprint = [int(v) for v in fingerprint]
+    if len(fingerprint) != len(FINGERPRINT_FIELDS):
+        raise ValueError(f"fingerprint needs the {len(FINGERPRINT_FIELDS)} words {FINGERPRINT_FIELDS}, "
+                         f"got {len(fingerprint)}")
+    if records.dim() != 2 or records.dtype != torch.int32 or counts.dtype != torch.int64:
+        raise TypeError("records must be (n, W) int32 and counts int64")
+    world = dist.get_world_size(group)
+    n, width = records.shape
+    header = torch.tensor(fingerprint + [width, counts.numel(), n, int(gt_total), int(images_total), 0],
+                          dtype=torch.int64).to(records.device)
+    header[_STATUS:].copy_(status.reshape(1))   # on the device: the status word is not read before the exchange
+    headers = [torch.empty_like(header) for _ in range(world)]
+    dist.all_gather(headers, header, group=group)
+    h = torch.stack(headers).cpu()
+    for r in range(1, world):
+        diff = [name for i, name in enumerate(_CHECKED) if h[r, i] != h[0, i]]
+        if diff:
+            raise ValueError(f"evaluation configurations differ across ranks: rank {r} and rank 0 disagree on "
+                             f"{', '.join(diff)}; every rank must build the metric with the same arguments")
+    parts = [torch.empty_like(counts) for _ in range(world)]
+    dist.all_gather(parts, counts.contiguous(), group=group)
+    counts = torch.stack(parts).sum(0)
+    rows = h[:, _ROWS].tolist()
+    if max(rows) == 0:
+        merged = records.new_empty((0, width))
+    else:
+        padded = records.new_full((max(rows), width), -1)
+        padded[:n] = records
+        parts = [torch.empty_like(padded) for _ in range(world)]
+        dist.all_gather(parts, padded, group=group)
+        merged = torch.cat([p[:r] for p, r in zip(parts, rows)])
+    word = 0
+    for s in h[:, _STATUS].tolist():
+        word |= s
+    return (merged, counts, int(h[:, _GT_TOTAL].sum()), int(h[:, _IMAGES_TOTAL].sum()),
+            torch.tensor([word], dtype=status.dtype).to(status.device))

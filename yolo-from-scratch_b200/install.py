@@ -100,20 +100,26 @@ def _make_predict(train_module):
 
 
 def _evaluate_dataset(train_module, metric, model, dataset, device, num_classes, conf_threshold, iou_threshold,
-                      batch_size):
+                      batch_size, group):
     """Feed `metric` (DetectionMAP, COCODetectionEval or DetectionReport) the detections of `model` on `dataset` (its imgs and labels
     lists) batch by batch and return metric.compute().  Images are loaded and letterboxed by the module's own Image
-    and letterbox_resize, as predict() does (train.py:1134-1138)."""
+    and letterbox_resize, as predict() does (train.py:1134-1138).  With a torch.distributed `group` this rank takes
+    only its contiguous block of images, dist.shard_range(len(dataset.imgs), rank, world), and returns
+    metric.compute(group): every rank of the group must call it, and every rank gets the result over all images."""
     import numpy as np
     import torch
+    from .dist import shard_range
     g = train_module.__dict__
     model.eval()
     img_size = model.img_size
-    n = len(dataset.imgs)
+    lo, hi = 0, len(dataset.imgs)
+    if group is not None:
+        import torch.distributed as dist
+        lo, hi = shard_range(hi, dist.get_rank(group), dist.get_world_size(group))
     with torch.no_grad():
-        for i0 in range(0, n, batch_size):
+        for i0 in range(lo, hi, batch_size):
             imgs, letterbox, labels = [], [], []
-            for i in range(i0, min(i0 + batch_size, n)):
+            for i in range(i0, min(i0 + batch_size, hi)):
                 pil_img = g["Image"].open(dataset.imgs[i]).convert("RGB")
                 orig_w, orig_h = pil_img.size
                 pil_img, scale, pad_top, pad_left = g["letterbox_resize"](pil_img, img_size)
@@ -124,19 +130,21 @@ def _evaluate_dataset(train_module, metric, model, dataset, device, num_classes,
             det = ops.detect_batch(list(preds), model.anchors, img_size, num_classes, conf_threshold, iou_threshold,
                                    letterbox=[lb[2:] for lb in letterbox])
             metric.update(det, ops.pack_labels(labels, img_size, letterbox))
-    return metric.compute()
+    return metric.compute(group)
 
 
 def _make_evaluate_map(train_module):
     """`evaluate_map`, a name the reference does not have: COCO-style mAP of a model over a YOLODataset's images
     and label files (ops.DetectionMAP)."""
     def evaluate_map(model, dataset, device, num_classes=1, conf_threshold=0.001, iou_threshold=0.4, batch_size=8,
-                     max_det=300):
+                     max_det=300, group=None):
         """mAP@[.5:.95] / mAP@0.5 of `model` on `dataset` (its imgs and labels lists).  Returns DetectionMAP.compute()'s
-        dict: map, map50, ap (nc,T), precision (T,R,nc), recall (T,nc), n_gt (nc), n_det (nc)."""
+        dict: map, map50, ap (nc,T), precision (T,R,nc), recall (T,nc), n_gt (nc), n_det (nc).  group: a
+        torch.distributed process group; every rank calls evaluate_map, scores only its block of the images
+        (dist.shard_range) and gets the result over all of them (DetectionMAP.compute(group))."""
         metric = ops.DetectionMAP(num_classes, max_det=max_det)
         return _evaluate_dataset(train_module, metric, model, dataset, device, num_classes, conf_threshold,
-                                 iou_threshold, batch_size)
+                                 iou_threshold, batch_size, group)
     return evaluate_map
 
 
@@ -144,13 +152,14 @@ def _make_evaluate_coco(train_module):
     """`evaluate_coco`, a name the reference does not have: COCO's twelve bbox stats of a model over a YOLODataset's
     images and label files (ops.COCODetectionEval)."""
     def evaluate_coco(model, dataset, device, num_classes=1, conf_threshold=0.001, iou_threshold=0.4, batch_size=8,
-                      max_det=300, max_dets=ops.COCO_MAX_DETS):
+                      max_det=300, max_dets=ops.COCO_MAX_DETS, group=None):
         """COCO's bbox summary of `model` on `dataset` (its imgs and labels lists).  Returns
         COCODetectionEval.compute()'s dict: stats (12,), precision (T,R,nc,A,M), recall (T,nc,A,M), n_gt (nc,A),
-        n_det (nc), ap (nc,T), map, map50; ops.format_coco_stats(stats) gives pycocotools' printed lines."""
+        n_det (nc), ap (nc,T), map, map50; ops.format_coco_stats(stats) gives pycocotools' printed lines.  group: as
+        evaluate_map's."""
         metric = ops.COCODetectionEval(num_classes, max_det=max_det, max_dets=max_dets)
         return _evaluate_dataset(train_module, metric, model, dataset, device, num_classes, conf_threshold,
-                                 iou_threshold, batch_size)
+                                 iou_threshold, batch_size, group)
     return evaluate_coco
 
 
@@ -158,13 +167,13 @@ def _make_evaluate_report(train_module):
     """`evaluate_report`, a name the reference does not have: the validation report of a model over a YOLODataset's
     images and label files (ops.DetectionReport)."""
     def evaluate_report(model, dataset, device, num_classes=1, conf_threshold=0.001, iou_threshold=0.4, batch_size=8,
-                        max_det=300):
+                        max_det=300, group=None):
         """Confusion matrix, P/R/F1 curves over the confidence threshold, best-F1 threshold and the AP columns of
         `model` on `dataset` (its imgs and labels lists).  Returns DetectionReport.compute()'s dict;
-        ops.format_detection_report(out) gives the per-class table."""
+        ops.format_detection_report(out) gives the per-class table.  group: as evaluate_map's."""
         metric = ops.DetectionReport(num_classes, max_det=max_det)
         return _evaluate_dataset(train_module, metric, model, dataset, device, num_classes, conf_threshold,
-                                 iou_threshold, batch_size)
+                                 iou_threshold, batch_size, group)
     return evaluate_report
 
 

@@ -21,6 +21,7 @@ computed there, and staged back.  That is staging, not a fallback: without CUDA 
 raises.
 """
 import ctypes
+import zlib
 from typing import List, Optional, Sequence
 
 import numpy as np
@@ -914,6 +915,16 @@ def _sort_records(rec, nc):
     return rec, seg
 
 
+def _eval_fingerprint(kind, nc, T, R, A, M, K, max_det, arrays):
+    """The configuration words compute(group) requires to be equal on every rank (dist.FINGERPRINT_FIELDS; kind 1
+    DetectionMAP, 2 COCODetectionEval, 3 DetectionReport): the sizes, and one CRC-32 over the float64 bytes of every
+    threshold, grid, area range and limit."""
+    crc = 0
+    for a in arrays:
+        crc = zlib.crc32(np.ascontiguousarray(a, dtype=np.float64).tobytes(), crc)
+    return kind, nc, T, R, A, M, K, max_det, crc
+
+
 def _raise_status(status, who):
     """The errors of the mAP kernels' status bits (YB_MAP_*)."""
     if status & _lib.MAP_BAD_CLASS:
@@ -931,7 +942,15 @@ class DetectionMAP:
     detections per image instead of COCO's per-category maxDets; include/yolo_b200.h states the semantics.
 
     update(det, labels) enqueues one matching kernel per batch and keeps its records; it never synchronises.
-    compute() sorts the records once, runs the precision kernel and synchronises once."""
+    compute() sorts the records once, runs the precision kernel and synchronises once.
+
+    compute(group) evaluates an image-sharded run: a collective over the torch.distributed process group `group`
+    (every rank calls it) that returns on every rank the dict one process would return after update() with every
+    rank's batches in rank order (DESIGN §3.11).  It synchronises twice and leaves the local state unchanged.  The
+    result is bit-identical to that process when rank r updated the r-th contiguous block of images
+    (dist.shard_range) in image order.  With any other assignment, such as DistributedSampler's interleaving,
+    n_gt, n_det and recall are still identical, and the precision table (with the AP values taken from it) can
+    differ only through the order of equal-score detections of different images."""
 
     def __init__(self, num_classes, iou_thresholds=COCO_IOU_THRESHOLDS, recall_thresholds=COCO_RECALL_THRESHOLDS,
                  max_det=300):
@@ -985,31 +1004,45 @@ class DetectionMAP:
         self._records.append(rec)
         self._gt_total += B * labels.max_gt
 
-    def compute(self):
+    def compute(self, group=None):
         """{map, map50, ap (nc,T), precision (T,R,nc), recall (T,nc), n_gt (nc), n_det (nc)} on the host (float64 /
         int64; map50 is None when 0.5 is not a threshold).  Entries of a class without ground truth are -1, and
-        map / map50 are the means of the entries > -1 (-1 when there are none), as COCOeval.summarize."""
+        map / map50 are the means of the entries > -1 (-1 when there are none), as COCOeval.summarize.
+        group: a torch.distributed process group to merge over (see the class docstring)."""
         with torch.cuda.device(self.device):
-            host = torch.cat(self._compute_device()).cpu().numpy()   # the one synchronisation
+            state = self._local_state()
+            if group is not None:
+                from .dist import gather_eval_state
+                fp = _eval_fingerprint(1, self.nc, len(self.iou_thresholds), len(self.recall_thresholds), 0, 0, 0,
+                                       self.max_det, (self.iou_thresholds, self.recall_thresholds))
+                rec, gt_count, gt_total, _, status = gather_eval_state(fp, *state[:3], 0, state[3], group)
+                state = (rec, gt_count, gt_total, status)
+            host = torch.cat(self._compute_device(*state)).cpu().numpy()   # the one synchronisation (2nd with a group)
         return self._compute_host(host, "DetectionMAP")
 
-    def _compute_device(self):
-        """Device half of compute(): sort the records and run the precision kernel.  Returns the flat float64 device
-        tensors compute() copies back, in the order _compute_host reads them (the status word last)."""
+    def _local_state(self):
+        """(records in image order, gt_count, gt_total, status): what _compute_device reads of one process."""
+        rec = (torch.cat(self._records) if self._records
+               else torch.empty(0, 3, dtype=torch.int32, device=self.device))
+        return rec, self._gt_count, self._gt_total, self._status
+
+    def _compute_device(self, rec, gt_count, gt_total, status):
+        """Device half of compute() on the state _local_state returns or a merge of it: sort the records and run the
+        precision kernel.  Returns the flat float64 device tensors compute() copies back, in the order _compute_host
+        reads them (the status word last)."""
         T, R, nc = len(self.iou_thresholds), len(self.recall_thresholds), self.nc
         dev = self.device
-        rec = torch.cat(self._records) if self._records else torch.empty(0, 3, dtype=torch.int32, device=dev)
         rec, seg = _sort_records(rec, nc)
         n = rec.shape[0]
-        ws_bytes = _lib.lib().yb_map_workspace_bytes(n, self._gt_total, T)
+        ws_bytes = _lib.lib().yb_map_workspace_bytes(n, gt_total, T)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         precision = torch.empty(T, R, nc, dtype=torch.float64, device=dev)
         recall = torch.empty(T, nc, dtype=torch.float64, device=dev)
-        _lib.check(_lib.lib().yb_map_precision(rec.data_ptr(), seg.data_ptr(), self._gt_count.data_ptr(), nc, T,
+        _lib.check(_lib.lib().yb_map_precision(rec.data_ptr(), seg.data_ptr(), gt_count.data_ptr(), nc, T,
                                                self._rec_thr.data_ptr(), R, precision.data_ptr(), recall.data_ptr(),
-                                               ws.data_ptr(), ws_bytes, self._status.data_ptr(), _stream()),
+                                               ws.data_ptr(), ws_bytes, status.data_ptr(), _stream()),
                    "yb_map_precision")
-        return [precision.reshape(-1), recall.reshape(-1), self._gt_count.double(), seg.double(), self._status.double()]
+        return [precision.reshape(-1), recall.reshape(-1), gt_count.double(), seg.double(), status.double()]
 
     def _host_size(self):
         """Number of doubles _compute_device's tensors hold."""
@@ -1058,7 +1091,13 @@ class COCODetectionEval:
     -1 when max_dets lacks 100; every other stat uses max_dets[0..2].
 
     update(det, labels) enqueues one matching kernel per batch and keeps its records; it never synchronises.
-    compute() sorts the records once, runs the precision kernel and synchronises once."""
+    compute() sorts the records once, runs the precision kernel and synchronises once.
+
+    compute(group) evaluates an image-sharded run as DetectionMAP.compute(group) does: a collective over `group` that
+    returns on every rank the dict of one process that saw every rank's batches in rank order, bit-identical when
+    rank r updated the r-th contiguous block of images in image order.  With any other assignment n_gt, n_det and
+    recall are still identical, and precision (with the stats and AP values taken from it) can differ only through
+    the order of equal-score detections of different images."""
 
     def __init__(self, num_classes, iou_thresholds=COCO_IOU_THRESHOLDS, recall_thresholds=COCO_RECALL_THRESHOLDS,
                  max_det=300, max_dets=COCO_MAX_DETS):
@@ -1117,25 +1156,32 @@ class COCODetectionEval:
                 self._status.data_ptr(), _stream()), "yb_coco_match")
         self._records.append(rec)
 
-    def compute(self):
+    def compute(self, group=None):
         """{stats (12,), precision (T,R,nc,A,M), recall (T,nc,A,M), n_gt (nc,A), n_det (nc), and ap (nc,T), map,
         map50 at area "all" and max_dets[-1]} on the host (float64 / int64).  Entries of a (class, area) without
         ground truth are -1; stats are pycocotools' _summarizeDets, map / map50 DetectionMAP's means.  n_gt counts
-        the ground truths inside each area range, n_det the records of each class (at most max_det per image)."""
+        the ground truths inside each area range, n_det the records of each class (at most max_det per image).
+        group: a torch.distributed process group to merge over (see the class docstring)."""
         T, R, nc = len(self.iou_thresholds), len(self.recall_thresholds), self.nc
         A, M = len(self.area_ranges), len(self.max_dets)
         dev = self.device
         with torch.cuda.device(dev):
             rec = torch.cat(self._records) if self._records else torch.empty(0, 8, dtype=torch.int32, device=dev)
+            gt_count, status = self._gt_count, self._status
+            if group is not None:
+                from .dist import gather_eval_state
+                fp = _eval_fingerprint(2, nc, T, R, A, M, 0, self.max_det,
+                                       (self.iou_thresholds, self.recall_thresholds, self.area_ranges, self.max_dets))
+                rec, gt_count, _, _, status = gather_eval_state(fp, rec, gt_count, 0, 0, status, group)
             rec, seg = _sort_records(rec, nc)
             precision = torch.empty(T, R, nc, A, M, dtype=torch.float64, device=dev)
             recall = torch.empty(T, nc, A, M, dtype=torch.float64, device=dev)
-            _lib.check(_lib.lib().yb_coco_precision(rec.data_ptr(), seg.data_ptr(), self._gt_count.data_ptr(), nc, A, T,
+            _lib.check(_lib.lib().yb_coco_precision(rec.data_ptr(), seg.data_ptr(), gt_count.data_ptr(), nc, A, T,
                                                     self._rec_thr.data_ptr(), R, self._md_host, M, precision.data_ptr(),
-                                                    recall.data_ptr(), self._status.data_ptr(), _stream()),
+                                                    recall.data_ptr(), status.data_ptr(), _stream()),
                        "yb_coco_precision")
-            host = torch.cat([precision.reshape(-1), recall.reshape(-1), self._gt_count.reshape(-1).double(),
-                              seg.double(), self._status.double()]).cpu().numpy()   # the one synchronisation
+            host = torch.cat([precision.reshape(-1), recall.reshape(-1), gt_count.reshape(-1).double(),
+                              seg.double(), status.double()]).cpu().numpy()   # the one sync (2nd with a group)
         _raise_status(int(host[-1]), "COCODetectionEval")
         o = 0
         precision = host[o:o + T * R * nc * A * M].reshape(T, R, nc, A, M); o += T * R * nc * A * M
@@ -1203,7 +1249,14 @@ class DetectionReport:
 
     update(det, labels) runs DetectionMAP.update and one report kernel on the records it wrote; it never
     synchronises.  compute() runs DetectionMAP's compute path plus the histograms' suffix sums and synchronises
-    once."""
+    once.
+
+    compute(group) evaluates an image-sharded run as DetectionMAP.compute(group) does: a collective over `group` that
+    returns on every rank the dict of one process that saw every rank's batches in rank order, bit-identical when
+    rank r updated the r-th contiguous block of images in image order.  With any other assignment the counts (n_gt,
+    n_det, confusion, images, images_total, the histograms and so the curves and best_conf) and recall are still
+    identical, and precision (with the AP values taken from it) can differ only through the order of equal-score
+    detections of different images."""
 
     def __init__(self, num_classes, max_det=300, iou_thresholds=COCO_IOU_THRESHOLDS, conf_grid=DEFAULT_CONF_GRID,
                  curve_iou=0.5, cm_conf=0.25, cm_iou=0.45):
@@ -1257,21 +1310,33 @@ class DetectionReport:
                 self.map._status.data_ptr(), _stream()), "yb_report_match")
         self.images_total += B
 
-    def compute(self):
+    def compute(self, group=None):
         """DetectionMAP.compute()'s dict plus, on the host:
         px (K,) the grid; p_curve, r_curve, f1_curve (nc,K) at curve_iou (P = TP/D, 1 where D = 0; R = TP/n_gt;
         F1 = 2PR/(P+R), 0 where P+R = 0; rows of classes without ground truth -1); best_conf = px[k*] with k* the
         first arg-max of the mean F1 over the classes with ground truth (None when there are none); p, r, f1 (nc,)
-        at k*; confusion (nc+1,nc+1) and images (nc) int64; images_total; iou_thresholds (the columns of ap)."""
+        at k*; confusion (nc+1,nc+1) and images (nc) int64; images_total; iou_thresholds (the columns of ap).
+        group: a torch.distributed process group to merge over (see the class docstring)."""
         nc, K = self.nc, self.conf_grid.size
         m = self.map._host_size()
         with torch.cuda.device(self.map.device):
-            hist = self._counts[(nc + 1) ** 2 + nc:].view(2, nc, K)   # det_hist, tp_hist
+            rec, gt_count, gt_total, status = self.map._local_state()
+            counts, images_total = self._counts, self.images_total
+            if group is not None:
+                from .dist import gather_eval_state
+                mp = self.map
+                fp = _eval_fingerprint(3, nc, len(mp.iou_thresholds), len(mp.recall_thresholds), 0, 0, K, mp.max_det,
+                                       (mp.iou_thresholds, mp.recall_thresholds, self.conf_grid,
+                                        (self.curve_iou, self.cm_conf, self.cm_iou)))
+                rec, both, gt_total, images_total, status = gather_eval_state(
+                    fp, rec, torch.cat([gt_count, counts]), gt_total, images_total, status, group)
+                gt_count, counts = both[:nc], both[nc:]
+            hist = counts[(nc + 1) ** 2 + nc:].view(2, nc, K)   # det_hist, tp_hist
             rev = hist.flip(2).cumsum(2)   # [.., K-1-k] = detections / TPs with score > grid[k]
-            dev = torch.cat(self.map._compute_device() + [self._counts[:(nc + 1) ** 2 + nc].double(),
-                                                          rev.reshape(-1).double()])
+            dev = torch.cat(self.map._compute_device(rec, gt_count, gt_total, status)
+                            + [counts[:(nc + 1) ** 2 + nc].double(), rev.reshape(-1).double()])
             self._host.copy_(dev, non_blocking=True)
-            torch.cuda.current_stream().synchronize()   # the one synchronisation
+            torch.cuda.current_stream().synchronize()   # the one synchronisation (the second with a group)
         host = self._host.numpy()
         out = self.map._compute_host(host[:m].copy(), "DetectionReport")   # its tables are returned as views
         o = m
@@ -1280,7 +1345,7 @@ class DetectionReport:
         n_det = host[o:o + nc * K].astype(np.int64).reshape(nc, K)[:, ::-1]; o += nc * K
         n_tp = host[o:o + nc * K].astype(np.int64).reshape(nc, K)[:, ::-1]
         out.update(report_curves(n_det, n_tp, out["n_gt"], self.conf_grid), confusion=confusion, images=images,
-                   images_total=self.images_total, iou_thresholds=self.map.iou_thresholds.copy())
+                   images_total=images_total, iou_thresholds=self.map.iou_thresholds.copy())
         return out
 
 
