@@ -229,6 +229,35 @@ int yb_filter_compact(const yb_heads_desc* d, float conf_thres, const float* let
                       void* ws, size_t ws_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Multi-label candidates with a per-image top-K cap (the candidate set of YOLO validation tools;
+ * no reference equivalent: predict() takes the arg-max class, train.py:1184-1189).
+ *   Rows of image b in yb_filter_compact's canonical order (P3->P4->P5, (gy,gx,a) row-major; NCHW heads the same).
+ *   A row is considered iff sigmoid(obj) > conf (yb_filter_compact's objectness test, 1/(1+expf(-x))).
+ *   For each class c ascending it emits a candidate iff score = fp32(sigmoid(obj) * sigmoid(cls_c)) > (float)conf
+ *   (nc == 1: slot 5 only, class 0).  A NaN class logit gives no candidate for that class, a NaN objectness none.
+ *   The box is the row's box of yb_filter_compact, bit for bit.  Candidate order = (row, class) lexicographic.
+ *   Scores are never negative or NaN, so their uint32 bit patterns are ordered like their values.
+ *   Cap, K = max_candidates >= 1, N_b = candidates of image b:
+ *     N_b <= K: every candidate is kept;
+ *     else: the first K of the stable order (score descending, candidate order ascending), i.e. argsort(-score,
+ *     stable)[:K]: ties at the K-th score go to the earlier candidates.
+ *   Kept candidates are written in candidate order: boxes (B,cap,4) fp32, scores (B,cap) fp32, classes (B,cap)
+ *   int64; counts[b] = min(N_b, K); totals[b] = N_b (int32, nullable; N_b <= rows * nc < 2^31 is checked).
+ *   cap >= min(max_candidates, rows * nc) (YB_EINVAL otherwise).
+ *   Workspace: 4 * B * (3*1024 + 8 + 258 * tiles) bytes, tiles = sum_s ceil(H_s*W_s / 128): three radix histograms
+ *   and the select state per image, two counts per 128-cell tile and per cell.  It does not grow with nc or K.
+ *   Nothing is synchronised and every launch runs unconditionally (images under the cap return at once), so the call
+ *   is capturable in a CUDA graph.
+ * NMS options of the callers, in terms of yb_batched_nms: class-agnostic = classes NULL (torchvision.ops.nms on the
+ *   candidates; the detections keep their classes); max_det = min(n_keep[b], max_det), the kept prefix
+ *   (torchvision's keep[:max_det]); a failed image's -1 stays -1.
+ * ---------------------------------------------------------------------------------------- */
+size_t yb_filter_multilabel_workspace_bytes(const yb_heads_desc* d, int max_candidates);
+int yb_filter_multilabel(const yb_heads_desc* d, float conf_thres, const float* letterbox, int max_candidates,
+                         float* boxes, float* scores, int64_t* classes, int* counts, int* totals /* nullable */,
+                         int cap, void* ws, size_t ws_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * a-7  torchvision.ops.batched_nms(boxes, scores, idxs, iou_threshold)       train.py:1232-1233
  *      (torchvision 0.26.0, torchvision/ops/boxes.py:51-120 and its CUDA nms kernel)
  *   Batched over B independent images with a fixed stride of `cap` candidates per image and

@@ -9,7 +9,7 @@ from . import _lib
 from .ops import (COCO_AREA_LABELS, COCO_AREA_RANGES, COCO_IOU_THRESHOLDS, COCO_MAX_DETS, COCO_RECALL_THRESHOLDS,
                   COCODetectionEval, DetectionMAP, DetectionReport, format_coco_stats, format_detection_report, batched_nms, batched_nms_padded, build_targets, ciou_loss, compute_anchor_iou,
                   decode_predictions, default_anchors, detect_batch, detect_batch_nchw, detections_to_lists, heads_from_nchw, eval_counts, eval_epoch,
-                  filter_candidates,
+                  filter_candidates, filter_candidates_multilabel, MAX_CANDIDATES,
                   loss_forward_backward, nms, nms_retry_overflow, pack_detections, predict_heads,
                   NMS_GRAPH, NMS_BITMASK, HotPathGraph, LAYOUT_BHWAC, LAYOUT_NCHW, PackedLabels, pack_labels, pack_labels_host, yolo_loss,
                   yolo_loss_multiscale, yolo_loss_multiscale_labels, yolo_loss_multiscale_nchw)
@@ -22,5 +22,5 @@ __all__ = [
     "detect_batch_nchw", "heads_from_nchw", "predict_heads", "HotPathGraph", "LAYOUT_BHWAC", "LAYOUT_NCHW", "default_anchors",
     "DetectionMAP", "COCO_IOU_THRESHOLDS", "COCO_RECALL_THRESHOLDS",
     "COCODetectionEval", "COCO_AREA_RANGES", "COCO_AREA_LABELS", "COCO_MAX_DETS", "format_coco_stats",
-    "DetectionReport", "format_detection_report",
+    "DetectionReport", "format_detection_report", "filter_candidates_multilabel", "MAX_CANDIDATES",
 ]

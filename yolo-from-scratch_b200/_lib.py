@@ -74,6 +74,9 @@ SIGNATURES = {
     "yb_filter_workspace_bytes": (c_size_t, [POINTER(HeadsDesc)]),
     "yb_filter_compact": (c_int, [POINTER(HeadsDesc), c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                   c_int, c_void_p, c_size_t, c_void_p]),
+    "yb_filter_multilabel_workspace_bytes": (c_size_t, [POINTER(HeadsDesc), c_int]),
+    "yb_filter_multilabel": (c_int, [POINTER(HeadsDesc), c_float, c_void_p, c_int, c_void_p, c_void_p, c_void_p,
+                                     c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
     "yb_nms_workspace_bytes": (c_size_t, [c_int, c_int]),
     "yb_nms_min_workspace_bytes": (c_size_t, [c_int, c_int]),
     "yb_nms_graph_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),

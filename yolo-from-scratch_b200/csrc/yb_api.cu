@@ -88,6 +88,6 @@ extern "C" int yb_timing_collect(char* buf, size_t n) {
     return (int)out.size();
 }
 
-extern "C" int yb_version(void) { return 101; }
+extern "C" int yb_version(void) { return 102; }
 extern "C" const char* yb_last_error(void) { return yb::g_err; }
 extern "C" unsigned long long yb_launch_count(void) { return yb::g_launches.load(); }

@@ -100,12 +100,13 @@ def _make_predict(train_module):
 
 
 def _evaluate_dataset(train_module, metric, model, dataset, device, num_classes, conf_threshold, iou_threshold,
-                      batch_size, group):
+                      batch_size, group, multi_label=False, agnostic=False, max_candidates=None):
     """Feed `metric` (DetectionMAP, COCODetectionEval or DetectionReport) the detections of `model` on `dataset` (its imgs and labels
     lists) batch by batch and return metric.compute().  Images are loaded and letterboxed by the module's own Image
     and letterbox_resize, as predict() does (train.py:1134-1138).  With a torch.distributed `group` this rank takes
     only its contiguous block of images, dist.shard_range(len(dataset.imgs), rank, world), and returns
-    metric.compute(group): every rank of the group must call it, and every rank gets the result over all images."""
+    metric.compute(group): every rank of the group must call it, and every rank gets the result over all images.
+    multi_label, agnostic and max_candidates go to ops.detect_batch."""
     import numpy as np
     import torch
     from .dist import shard_range
@@ -128,7 +129,8 @@ def _evaluate_dataset(train_module, metric, model, dataset, device, num_classes,
                 labels.append(_read_labels(train_module, dataset.labels[i]))
             preds = model(torch.stack(imgs).to(device))
             det = ops.detect_batch(list(preds), model.anchors, img_size, num_classes, conf_threshold, iou_threshold,
-                                   letterbox=[lb[2:] for lb in letterbox])
+                                   letterbox=[lb[2:] for lb in letterbox], multi_label=multi_label,
+                                   max_candidates=max_candidates, agnostic=agnostic)
             metric.update(det, ops.pack_labels(labels, img_size, letterbox))
     return metric.compute(group)
 
@@ -137,14 +139,17 @@ def _make_evaluate_map(train_module):
     """`evaluate_map`, a name the reference does not have: COCO-style mAP of a model over a YOLODataset's images
     and label files (ops.DetectionMAP)."""
     def evaluate_map(model, dataset, device, num_classes=1, conf_threshold=0.001, iou_threshold=0.4, batch_size=8,
-                     max_det=300, group=None):
+                     max_det=300, group=None, *, multi_label=False, agnostic=False, max_candidates=None):
         """mAP@[.5:.95] / mAP@0.5 of `model` on `dataset` (its imgs and labels lists).  Returns DetectionMAP.compute()'s
         dict: map, map50, ap (nc,T), precision (T,R,nc), recall (T,nc), n_gt (nc), n_det (nc).  group: a
         torch.distributed process group; every rank calls evaluate_map, scores only its block of the images
-        (dist.shard_range) and gets the result over all of them (DetectionMAP.compute(group))."""
+        (dist.shard_range) and gets the result over all of them (DetectionMAP.compute(group)).
+        multi_label=True scores the multi-label candidates of YOLO validation tools (one per (row, class) pair above
+        conf_threshold, at most max_candidates per image, None = ops.MAX_CANDIDATES); agnostic=True suppresses across
+        classes (ops.detect_batch)."""
         metric = ops.DetectionMAP(num_classes, max_det=max_det)
         return _evaluate_dataset(train_module, metric, model, dataset, device, num_classes, conf_threshold,
-                                 iou_threshold, batch_size, group)
+                                 iou_threshold, batch_size, group, multi_label, agnostic, max_candidates)
     return evaluate_map
 
 
@@ -152,14 +157,15 @@ def _make_evaluate_coco(train_module):
     """`evaluate_coco`, a name the reference does not have: COCO's twelve bbox stats of a model over a YOLODataset's
     images and label files (ops.COCODetectionEval)."""
     def evaluate_coco(model, dataset, device, num_classes=1, conf_threshold=0.001, iou_threshold=0.4, batch_size=8,
-                      max_det=300, max_dets=ops.COCO_MAX_DETS, group=None):
+                      max_det=300, max_dets=ops.COCO_MAX_DETS, group=None, *, multi_label=False, agnostic=False,
+                      max_candidates=None):
         """COCO's bbox summary of `model` on `dataset` (its imgs and labels lists).  Returns
         COCODetectionEval.compute()'s dict: stats (12,), precision (T,R,nc,A,M), recall (T,nc,A,M), n_gt (nc,A),
-        n_det (nc), ap (nc,T), map, map50; ops.format_coco_stats(stats) gives pycocotools' printed lines.  group: as
-        evaluate_map's."""
+        n_det (nc), ap (nc,T), map, map50; ops.format_coco_stats(stats) gives pycocotools' printed lines.  group,
+        multi_label, agnostic, max_candidates: as evaluate_map's."""
         metric = ops.COCODetectionEval(num_classes, max_det=max_det, max_dets=max_dets)
         return _evaluate_dataset(train_module, metric, model, dataset, device, num_classes, conf_threshold,
-                                 iou_threshold, batch_size, group)
+                                 iou_threshold, batch_size, group, multi_label, agnostic, max_candidates)
     return evaluate_coco
 
 
@@ -167,13 +173,14 @@ def _make_evaluate_report(train_module):
     """`evaluate_report`, a name the reference does not have: the validation report of a model over a YOLODataset's
     images and label files (ops.DetectionReport)."""
     def evaluate_report(model, dataset, device, num_classes=1, conf_threshold=0.001, iou_threshold=0.4, batch_size=8,
-                        max_det=300, group=None):
+                        max_det=300, group=None, *, multi_label=False, agnostic=False, max_candidates=None):
         """Confusion matrix, P/R/F1 curves over the confidence threshold, best-F1 threshold and the AP columns of
         `model` on `dataset` (its imgs and labels lists).  Returns DetectionReport.compute()'s dict;
-        ops.format_detection_report(out) gives the per-class table.  group: as evaluate_map's."""
+        ops.format_detection_report(out) gives the per-class table.  group, multi_label, agnostic, max_candidates: as
+        evaluate_map's."""
         metric = ops.DetectionReport(num_classes, max_det=max_det)
         return _evaluate_dataset(train_module, metric, model, dataset, device, num_classes, conf_threshold,
-                                 iou_threshold, batch_size, group)
+                                 iou_threshold, batch_size, group, multi_label, agnostic, max_candidates)
     return evaluate_report
 
 

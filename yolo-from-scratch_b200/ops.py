@@ -13,6 +13,7 @@ include/yolo_b200.h).  PyTorch is used only for device memory, streams and autog
   filter_candidates       train.py:1152-1229 (per-scale body of predict), batched
   nms / batched_nms       torchvision.ops as called at train.py:1232-1233
   detect_batch            filter_candidates + batched_nms + gather (predict :1152-1238 for a batch)
+  filter_candidates_multilabel  multi-label candidates with a per-image top-K cap (new; YOLO validation's candidate set)
   DetectionMAP            COCO-style mAP of detect_batch's detections (new; no reference equivalent)
   DetectionReport         confusion matrix, P/R/F1 over confidence, best-F1 threshold, per-class table (new)
 
@@ -683,6 +684,27 @@ def _heads_desc(preds, ancs, img_size, nc, layout=LAYOUT_BHWAC):
     return d
 
 
+def _stage_heads(predictions, anchors_list, num_classes, layout, dev):
+    """The heads and anchors as the filter kernels read them, checked: (preds, ancs, rows per image)."""
+    S = len(predictions)
+    preds = _same_dtype([_headc(p.detach(), dev) for p in predictions])
+    ancs = [_anchors_dev(a, dev) for a in anchors_list[:S]]
+    for s, p in enumerate(preds):
+        if layout == LAYOUT_NCHW:
+            if p.dim() != 4 or p.shape[1] != ancs[s].shape[0] * (5 + int(num_classes)):
+                raise ValueError(f"predictions[{s}]: NCHW head must be (B, A*(5+nc), H, W), got {tuple(p.shape)}")
+        else:
+            _check_head(p, f"predictions[{s}]")
+    rows = sum(_grid(p, layout)[0] * _grid(p, layout)[1] * ancs[s].shape[0] for s, p in enumerate(preds))
+    return preds, ancs, rows
+
+
+def _letterbox_dev(letterbox, B, dev):
+    if letterbox is None:
+        return None
+    return torch.as_tensor(letterbox, dtype=torch.float32).reshape(B, 3).to(dev).contiguous()
+
+
 def filter_candidates(predictions, anchors_list, img_size, num_classes=1, conf_threshold=0.5, letterbox=None,
                       layout=LAYOUT_BHWAC):
     """Per-scale body of predict() (train.py:1152-1229) for a batch: decode, sigmoid, objectness
@@ -694,18 +716,9 @@ def filter_candidates(predictions, anchors_list, img_size, num_classes=1, conf_t
     cap = rows per image.
     """
     dev = _device()
-    S = len(predictions)
     with torch.cuda.device(dev):
-        preds = _same_dtype([_headc(p.detach(), dev) for p in predictions])
-        ancs = [_anchors_dev(a, dev) for a in anchors_list[:S]]
-        for s, p in enumerate(preds):
-            if layout == LAYOUT_NCHW:
-                if p.dim() != 4 or p.shape[1] != ancs[s].shape[0] * (5 + int(num_classes)):
-                    raise ValueError(f"predictions[{s}]: NCHW head must be (B, A*(5+nc), H, W), got {tuple(p.shape)}")
-            else:
-                _check_head(p, f"predictions[{s}]")
+        preds, ancs, cap = _stage_heads(predictions, anchors_list, num_classes, layout, dev)
         B = preds[0].shape[0]
-        cap = sum(_grid(p, layout)[0] * _grid(p, layout)[1] * ancs[s].shape[0] for s, p in enumerate(preds))
         d = _heads_desc(preds, ancs, img_size, int(num_classes), layout)
         L = _lib.lib()
         ws_bytes = L.yb_filter_workspace_bytes(ctypes.byref(d))
@@ -714,13 +727,49 @@ def filter_candidates(predictions, anchors_list, img_size, num_classes=1, conf_t
         scores = torch.empty(B, cap, dtype=torch.float32, device=dev)
         classes = torch.empty(B, cap, dtype=torch.int64, device=dev)
         counts = (torch.empty if B > 0 else torch.zeros)(B, dtype=torch.int32, device=dev)   # every image's count is written by the kernel
-        lb = None
-        if letterbox is not None:
-            lb = torch.as_tensor(letterbox, dtype=torch.float32).reshape(B, 3).to(dev).contiguous()
+        lb = _letterbox_dev(letterbox, B, dev)
         _lib.check(L.yb_filter_compact(ctypes.byref(d), float(conf_threshold), _ptr(lb), boxes.data_ptr(),
                                        scores.data_ptr(), classes.data_ptr(), counts.data_ptr(), cap,
                                        ws.data_ptr(), ws.numel(), _stream()), "yb_filter_compact")
     return boxes, scores, classes, counts
+
+
+MAX_CANDIDATES = 30000   # max_nms of YOLO validation tools: candidates per image kept before NMS
+
+
+def filter_candidates_multilabel(predictions, anchors_list, img_size, num_classes=1, conf_threshold=0.001,
+                                 letterbox=None, layout=LAYOUT_BHWAC, max_candidates=MAX_CANDIDATES):
+    """Multi-label candidates of a batch (include/yolo_b200.h, yb_filter_multilabel): every (row, class) pair with
+    sigmoid(obj) > conf and score = sigmoid(obj) * sigmoid(cls_c) > conf, in (row, class) order, each with the box
+    filter_candidates gives its row.  An image with more than max_candidates keeps the best max_candidates by (score
+    descending, candidate order), still in candidate order.  Inputs, layouts and dtypes as filter_candidates.
+
+    Returns (boxes (B,cap,4), scores (B,cap), classes (B,cap) int64, counts (B,) int32, totals (B,) int32) on the GPU:
+    cap = min(max_candidates, rows * nc), counts = kept candidates, totals = candidates before the cap.  Nothing is
+    synchronised; the call is capturable in a CUDA graph.
+    """
+    K = int(max_candidates)
+    if K < 1:
+        raise ValueError(f"max_candidates must be >= 1, got {max_candidates}")
+    dev = _device()
+    with torch.cuda.device(dev):
+        preds, ancs, rows = _stage_heads(predictions, anchors_list, num_classes, layout, dev)
+        B = preds[0].shape[0]
+        cap = min(K, rows * int(num_classes))
+        d = _heads_desc(preds, ancs, img_size, int(num_classes), layout)
+        L = _lib.lib()
+        ws = torch.empty(max(L.yb_filter_multilabel_workspace_bytes(ctypes.byref(d), K), 16), dtype=torch.uint8,
+                         device=dev)
+        boxes = torch.empty(B, cap, 4, dtype=torch.float32, device=dev)
+        scores = torch.empty(B, cap, dtype=torch.float32, device=dev)
+        classes = torch.empty(B, cap, dtype=torch.int64, device=dev)
+        counts = (torch.empty if B > 0 else torch.zeros)(B, dtype=torch.int32, device=dev)
+        totals = (torch.empty if B > 0 else torch.zeros)(B, dtype=torch.int32, device=dev)
+        lb = _letterbox_dev(letterbox, B, dev)
+        _lib.check(L.yb_filter_multilabel(ctypes.byref(d), float(conf_threshold), _ptr(lb), K, boxes.data_ptr(),
+                                          scores.data_ptr(), classes.data_ptr(), counts.data_ptr(), totals.data_ptr(),
+                                          cap, ws.data_ptr(), ws.numel(), _stream()), "yb_filter_multilabel")
+    return boxes, scores, classes, counts, totals
 
 
 NMS_GRAPH, NMS_BITMASK = _lib.NMS_GRAPH, _lib.NMS_BITMASK
@@ -822,33 +871,64 @@ def nms(boxes, scores, iou_threshold, algo=NMS_GRAPH):
 
 
 def detect_batch(predictions, anchors_list, img_size, num_classes=1, conf_threshold=0.5, iou_threshold=0.4,
-                 letterbox=None, trick_max_numel=TRICK_MAX_NUMEL_CUDA, algo=NMS_GRAPH, layout=LAYOUT_BHWAC):
+                 letterbox=None, trick_max_numel=TRICK_MAX_NUMEL_CUDA, algo=NMS_GRAPH, layout=LAYOUT_BHWAC, *,
+                 multi_label=False, max_candidates=None, agnostic=False, max_det=None):
     """predict() lines 1152-1238 for a whole batch on the GPU: decode + filter + global NMS.
 
     Returns a dict of device tensors: boxes (B,cap,4), scores, classes, counts (candidates per
     image), keep (B,cap) indices into the candidates in descending score order, n_keep (B,).
     Nothing is synchronised; use `detections_to_lists` for the reference's list-of-tuples form.
+
+    multi_label=True takes the candidates of filter_candidates_multilabel (one per (row, class) pair that passes
+    conf; at most max_candidates per image, None = MAX_CANDIDATES) and adds "totals", the candidates before the cap.
+    The default single-label filter is bounded by the rows and takes no max_candidates.  agnostic and max_det are
+    nms_candidates'.  The dict records the options.
     """
-    boxes, scores, classes, counts = filter_candidates(predictions, anchors_list, img_size, num_classes,
-                                                       conf_threshold, letterbox, layout)
-    return nms_candidates(boxes, scores, classes, counts, iou_threshold, trick_max_numel, algo)
+    if multi_label:
+        K = MAX_CANDIDATES if max_candidates is None else int(max_candidates)
+        boxes, scores, classes, counts, totals = filter_candidates_multilabel(
+            predictions, anchors_list, img_size, num_classes, conf_threshold, letterbox, layout, K)
+    else:
+        if max_candidates is not None:
+            raise ValueError("max_candidates applies to multi_label=True only: the single-label filter keeps at most "
+                             "one candidate per row")
+        boxes, scores, classes, counts = filter_candidates(predictions, anchors_list, img_size, num_classes,
+                                                           conf_threshold, letterbox, layout)
+    det = nms_candidates(boxes, scores, classes, counts, iou_threshold, trick_max_numel, algo, agnostic=agnostic,
+                         max_det=max_det)
+    det["multi_label"] = bool(multi_label)
+    if multi_label:
+        det["totals"] = totals
+        det["max_candidates"] = K
+    return det
 
 
-def nms_candidates(boxes, scores, classes, counts, iou_threshold=0.4, trick_max_numel=TRICK_MAX_NUMEL_CUDA, algo=NMS_GRAPH):
-    """Second half of detect_batch: global NMS (train.py:1232-1233) over the padded candidates of filter_candidates."""
+def nms_candidates(boxes, scores, classes, counts, iou_threshold=0.4, trick_max_numel=TRICK_MAX_NUMEL_CUDA, algo=NMS_GRAPH,
+                   *, agnostic=False, max_det=None):
+    """Second half of detect_batch: global NMS (train.py:1232-1233) over the padded candidates of filter_candidates.
+    agnostic=True suppresses across classes (torchvision.ops.nms on the candidates; the detections keep their
+    classes).  max_det keeps the first max_det detections of every image (n_keep = min(n_keep, max_det), torchvision's
+    keep[:max_det]; a failed image's -1 stays -1)."""
+    if max_det is not None and int(max_det) < 0:
+        raise ValueError(f"max_det must be >= 0, got {max_det}")
     with torch.cuda.device(boxes.device):
-        keep, n_keep, ws = batched_nms_padded(boxes, scores, classes, counts, iou_threshold, trick_max_numel, algo,
-                                              return_workspace=True)
+        keep, n_keep, ws = batched_nms_padded(boxes, scores, None if agnostic else classes, counts, iou_threshold,
+                                              trick_max_numel, algo, return_workspace=True)
+        if max_det is not None:
+            n_keep = n_keep.clamp(max=int(max_det))
     return {"boxes": boxes, "scores": scores, "classes": classes, "counts": counts, "keep": keep, "n_keep": n_keep,
-            "iou_threshold": float(iou_threshold), "trick_max_numel": int(trick_max_numel), "algo": algo, "nms_ws": ws}
+            "iou_threshold": float(iou_threshold), "trick_max_numel": int(trick_max_numel), "algo": algo, "nms_ws": ws,
+            "agnostic": bool(agnostic), "max_det": None if max_det is None else int(max_det)}
 
 
 def detect_batch_nchw(raw_heads, anchors_list, img_size, num_classes=1, conf_threshold=0.5, iou_threshold=0.4,
-                      letterbox=None, trick_max_numel=TRICK_MAX_NUMEL_CUDA, algo=NMS_GRAPH):
+                      letterbox=None, trick_max_numel=TRICK_MAX_NUMEL_CUDA, algo=NMS_GRAPH, *, multi_label=False,
+                      max_candidates=None, agnostic=False, max_det=None):
     """detect_batch on the head convs' own outputs (B, A*(5+nc), H, W) (SURVEY 8f-2); same candidates,
     same order, same keep sets as detect_batch on the permuted heads."""
     return detect_batch(raw_heads, anchors_list, img_size, num_classes, conf_threshold, iou_threshold, letterbox,
-                        trick_max_numel, algo, layout=LAYOUT_NCHW)
+                        trick_max_numel, algo, layout=LAYOUT_NCHW, multi_label=multi_label,
+                        max_candidates=max_candidates, agnostic=agnostic, max_det=max_det)
 
 
 def pack_detections(det):
