@@ -14,14 +14,12 @@ import torch
 
 from yolo_from_scratch_b200 import ops
 from oracle import ref_path as R
-import test_gpu_coco as GC
-import test_gpu_map as GM
-import test_gpu_report as GR
+import eval_data as E
 from test_dist_eval_cpu import run_ranks
 
 pytestmark = pytest.mark.gpu
 KINDS = ("map", "coco", "report")
-GENERATORS = {"map": GM.synthetic_batch, "coco": GC.synthetic_batch, "report": GR.synthetic_batch}
+GENERATORS = {"map": E.synthetic_batch, "coco": E.coco_synthetic_batch, "report": E.synthetic_batch}
 CUSTOM_THR = (0.3, 0.6, 0.75)
 CUSTOM_REC = tuple(np.linspace(0.0, 1.0, 11).tolist())
 COUNT_KEYS = {"map": ("n_gt", "n_det", "recall"), "coco": ("n_gt", "n_det", "recall"),
@@ -40,7 +38,7 @@ def make_metric(kind, nc, params="default", **over):
         kw = (dict(iou_thresholds=CUSTOM_THR, recall_thresholds=CUSTOM_REC, max_det=50, max_dets=(1, 5, 20))
               if custom else {})
         return ops.COCODetectionEval(nc, **{**kw, **over})
-    kw = dict(iou_thresholds=CUSTOM_THR, max_det=50, conf_grid=GR.CUSTOM["grid"], curve_iou=0.75, cm_conf=0.6,
+    kw = dict(iou_thresholds=CUSTOM_THR, max_det=50, conf_grid=E.CUSTOM_GRID, curve_iou=0.75, cm_conf=0.6,
               cm_iou=0.3) if custom else {}
     return ops.DetectionReport(nc, **{**kw, **over})
 
@@ -59,7 +57,7 @@ def batches(data, idx, batch):
         sel = idx[i0:i0 + batch]
         t = torch.tensor(sel, dtype=torch.int64, device=det["boxes"].device)
         out.append(({k: v.index_select(0, t) for k, v in det.items()},
-                    GM.packed([labels[i] for i in sel], [lb[i] for i in sel])))
+                    E.packed([labels[i] for i in sel], [lb[i] for i in sel])))
     return out
 
 
@@ -232,7 +230,7 @@ def test_bad_class_on_one_rank_raises_on_every_rank():
         assert errors == ["IndexError"] * len(KINDS)
 
 
-class _ImageHeads(GM._PresetHeads):
+class _ImageHeads(E._PresetHeads):
     """Preset heads selected by image: image i is filled with the pixel value i, so each image gets the same heads
     whichever rank and batch it is in."""
 
@@ -266,8 +264,8 @@ def write_dataset(path):
 
 def evaluate_all(dataset, batch_size, group=None):
     from yolo_from_scratch_b200.install import install, uninstall
-    model = _ImageHeads(GM.prior_heads(N_FILES, IMG, NC, 7), IMG, [a.cuda() for a in R.default_anchors()])
-    train = install(GM._train_stand_in(*LETTERBOX))
+    model = _ImageHeads(E.prior_heads(N_FILES, IMG, NC, 7), IMG, [a.cuda() for a in R.default_anchors()])
+    train = install(E._train_stand_in(*LETTERBOX))
     try:
         dev = torch.device("cuda")
         return [train.evaluate_map(model, dataset, dev, num_classes=NC, batch_size=batch_size, group=group),

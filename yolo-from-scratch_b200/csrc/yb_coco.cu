@@ -1,10 +1,10 @@
 // yb_coco.cu — COCO's bbox summary (COCOeval.evaluateImg + accumulate with area ranges and per-(image, category)
 // maxDets, no crowd) on the device; the header states the semantics.
 //
-// Stage 1, coco_match_kernel: one CTA per (image, area range).  The image's ground truths are staged in shared
-// memory as fp64 corners with their "ignored in this range" flag; warp t runs COCO's greedy matching for IoU
-// threshold t over the kept detections in keep order, a warp arg-max on (not ignored, IoU, index) resolving each
-// step, exactly as map_match_kernel does with the flag as the leading key.  The CTA of range 0 also writes each
+// Stage 1, coco_match_kernel: one CTA per (image, area range) on yb_match.cuh's front end.  The image's ground truths
+// are staged in shared memory as fp64 corners with their "ignored in this range" flag; warp t runs COCO's greedy
+// matching for IoU threshold t over the kept detections in keep order, a warp arg-max on (not ignored, IoU, index)
+// resolving each step: greedy_match<true>, map_match_kernel's step with the flag as the leading key.  The CTA of range 0 also writes each
 // detection's rank within its (image, class): warp 0 groups 32 detections at a time by class with
 // __match_any_sync and carries per-class counts in shared memory.  Output: one 32-byte record per detection slot
 // (score, class, rank, TP and ignored bits per threshold for every range), plus the non-ignored ground-truth
@@ -15,41 +15,34 @@
 // a shared-memory (M,T,R) table keeps the largest pr per bucket (a non-negative double's bits order like an
 // integer, so an integer atomicMax is exact), and its suffix maximum over r is COCO's precision table.
 // Every fp64 expression is the oracle's (oracle/coco_ref.py) operation for operation (-fmad=false).
-#include "yb_common.cuh"
-#include "yb_iou.cuh"
+#include "yb_match.cuh"
 
 namespace yb {
 
 constexpr int kCocoPrecThreads = 256;
 
 struct CocoMatchArgs {
-    const float4* boxes;
-    const float* scores;
-    const int64_t* classes;
-    const int64_t* keep;
-    const int* n_keep;
-    const double* labels;
-    const int* n_gt;
-    const double* letterbox;
+    MatchInputs in;
     const double* thr;
     yb_coco_record* records;
     unsigned long long* gt_count;   // (A, nc)
     int* status;
     double rng[2 * YB_COCO_MAX_A];
-    int cap, slots, max_gt, nc, T, A;
+    int T, A;
 };
 
 __device__ __forceinline__ bool outside(double area, double lo, double hi) { return area < lo || area > hi; }
 
 __global__ void __launch_bounds__(512) coco_match_kernel(const CocoMatchArgs a) {
     extern __shared__ __align__(16) unsigned char smem[];
+    const MatchInputs& in = a.in;
     const int chunk = blockDim.x;
-    const int words = (a.max_gt + 31) / 32;
+    const int words = (in.max_gt + 31) / 32;
     GtBox* s_gt = reinterpret_cast<GtBox*>(smem);
-    float4* s_box = reinterpret_cast<float4*>(s_gt + a.max_gt);
+    float4* s_box = reinterpret_cast<float4*>(s_gt + in.max_gt);
     int* s_gcls = reinterpret_cast<int*>(s_box + chunk);
-    int* s_gnig = s_gcls + a.max_gt;              // 1: the ground truth is inside this range (not ignored)
-    int* s_dcls = s_gnig + a.max_gt;
+    int* s_gnig = s_gcls + in.max_gt;             // 1: the ground truth is inside this range (not ignored)
+    int* s_dcls = s_gnig + in.max_gt;
     int* s_dout = s_dcls + chunk;                 // 1: the detection is outside this range
     int* s_rank = s_dout + chunk;
     float* s_score = reinterpret_cast<float*>(s_rank + chunk);
@@ -58,48 +51,37 @@ __global__ void __launch_bounds__(512) coco_match_kernel(const CocoMatchArgs a) 
     unsigned int* s_matched = s_ig + chunk;       // [T][words]: ground truth g already taken at threshold t
     int* s_cnt = reinterpret_cast<int*>(s_matched + a.T * words);   // [nc] detections per class so far (range 0)
 
-    const int b = blockIdx.x, ar = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int ar = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const bool first = ar == 0;   // the CTA of range 0 writes the shared fields and reports the status
     const double lo = a.rng[2 * ar], hi = a.rng[2 * ar + 1];
-    const int nk = a.n_keep[b];
-    int bad = 0;
-    if (nk < 0) bad |= 2;
-    const int nd = nk < 0 ? 0 : min(nk, a.slots);
-    const int ng = min(max(a.n_gt[b], 0), a.max_gt);
-    const double ow = a.letterbox[(size_t)b * 5 + 0], oh = a.letterbox[(size_t)b * 5 + 1];
-    for (int g = tid; g < ng; g += blockDim.x) {
-        const double* L = a.labels + ((size_t)b * a.max_gt + g) * 5;
-        const double xc = L[1], yc = L[2], w = L[3], h = L[4];
-        const GtBox box{(xc - w / 2.0) * ow, (yc - h / 2.0) * oh, (xc + w / 2.0) * ow, (yc + h / 2.0) * oh};
-        s_gt[g] = box;
-        int c = 0;
-        if (a.nc > 1) {   // nc == 1: every ground truth is class 0 (train.py:201-202)
-            c = (int)L[0];
-            if (c < 0 || c >= a.nc) { bad |= 1; c = -1; }
-        }
+    int bad;
+    const MatchImage im = match_image(in, blockIdx.x, bad);
+    const int nd = im.nd;
+    for (int g = tid; g < im.ng; g += blockDim.x) {
+        GtBox box;
+        const int c = stage_gt(in, im, g, box, bad);
         const int nig = outside((box.x2 - box.x1) * (box.y2 - box.y1), lo, hi) ? 0 : 1;
+        s_gt[g] = box;
         s_gcls[g] = c;
         s_gnig[g] = nig;
-        if (c >= 0 && nig) atomicAdd(a.gt_count + (size_t)ar * a.nc + c, 1ull);
+        if (c >= 0 && nig) atomicAdd(a.gt_count + (size_t)ar * in.nc + c, 1ull);
     }
     for (int i = tid; i < a.T * words; i += blockDim.x) s_matched[i] = 0u;
     if (first)
-        for (int i = tid; i < a.nc; i += blockDim.x) s_cnt[i] = 0;
+        for (int i = tid; i < in.nc; i += blockDim.x) s_cnt[i] = 0;
 
-    yb_coco_record* rec = a.records + (size_t)b * a.slots;
+    yb_coco_record* rec = a.records + (size_t)im.b * in.slots;
     const unsigned int tmask = (1u << a.T) - 1u;
     const double thr_lim = 1.0 - 1e-10;
     for (int j0 = 0; j0 < nd; j0 += chunk) {
         const int j = j0 + tid;
         __syncthreads();   // previous chunk consumed; on the first pass: ground truths and counters staged
         if (j < nd) {
-            const size_t src = (size_t)b * a.cap + (size_t)a.keep[(size_t)b * a.cap + j];
-            const int64_t c = a.classes[src];
-            const float4 q = a.boxes[src];
+            const Kept d = load_kept(in, im, j, bad);
+            const float4 q = in.boxes[d.src];
             s_box[tid] = q;
-            s_score[tid] = a.scores[src];
-            s_dcls[tid] = (c >= 0 && c < a.nc) ? (int)c : -1;
-            if (!(c >= 0 && c < a.nc)) bad |= 1;
+            s_score[tid] = in.scores[d.src];
+            s_dcls[tid] = d.cls;
             s_dout[tid] = outside(((double)q.z - (double)q.x) * ((double)q.w - (double)q.y), lo, hi) ? 1 : 0;
             s_tp[tid] = 0u;
             s_ig[tid] = 0u;
@@ -127,37 +109,8 @@ __global__ void __launch_bounds__(512) coco_match_kernel(const CocoMatchArgs a) 
         }
         if (warp < a.T) {
             const double t0 = a.thr[warp];
-            const double thr = thr_lim < t0 ? thr_lim : t0;   // min([t, 1-1e-10])
-            unsigned int* matched = s_matched + warp * words;
-            for (int k = 0; k < n; ++k) {
-                const int c = s_dcls[k];
-                if (c < 0) continue;
-                const float4 q = s_box[k];
-                const GtBox d{(double)q.x, (double)q.y, (double)q.z, (double)q.w};
-                double best = -INFINITY;
-                int bn = 0, bi = -1;
-                for (int g = lane; g < ng; g += 32) {
-                    if (s_gcls[g] != c || ((matched[g >> 5] >> lane) & 1u)) continue;
-                    const double iou = corner_iou(d, s_gt[g]);
-                    if (!(iou >= thr)) continue;   // a NaN IoU never matches
-                    const int nig = s_gnig[g];
-                    if (nig > bn || (nig == bn && iou >= best)) { best = iou; bn = nig; bi = g; }   // later one wins ties
-                }
-#pragma unroll
-                for (int o = 16; o > 0; o >>= 1) {
-                    const double ob = __shfl_xor_sync(0xffffffffu, best, o);
-                    const int on = __shfl_xor_sync(0xffffffffu, bn, o);
-                    const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-                    if (oi >= 0 && (bi < 0 || on > bn || (on == bn && (ob > best || (ob == best && oi > bi))))) {
-                        best = ob; bn = on; bi = oi;
-                    }
-                }
-                if (bi >= 0 && lane == 0) {
-                    matched[bi >> 5] |= 1u << (bi & 31);
-                    atomicOr((bn ? s_tp : s_ig) + k, 1u << warp);
-                }
-                __syncwarp();
-            }
+            greedy_match<true>(n, s_box, s_dcls, im.ng, s_gt, s_gcls, s_gnig, thr_lim < t0 ? thr_lim : t0,   // min([t, 1-1e-10])
+                               warp, s_matched + warp * words, s_tp, s_ig);
         }
         __syncthreads();
         if (j < nd) {
@@ -178,7 +131,7 @@ __global__ void __launch_bounds__(512) coco_match_kernel(const CocoMatchArgs a) 
         }
     }
     if (first) {
-        for (int j = nd + tid; j < a.slots; j += blockDim.x) {
+        for (int j = nd + tid; j < in.slots; j += blockDim.x) {
             yb_coco_record& r = rec[j];
             r.score = 0.0f;
             r.cls = -1;
@@ -326,26 +279,21 @@ extern "C" int yb_coco_match(const float* boxes, const float* scores, const int6
                              const double* area_rng, int A, yb_coco_record* records, long long* gt_count, int* status,
                              void* stream) {
     using namespace yb;
-    YB_CHECK_ARG(B >= 0 && cap >= 0 && max_det >= 0 && nc >= 1, "coco_match: bad B/cap/max_det/nc");
     YB_CHECK_ARG(T >= 1 && T <= YB_MAP_MAX_T, "coco_match: 1 <= T <= %d thresholds", YB_MAP_MAX_T);
     YB_CHECK_ARG(A >= 1 && A <= YB_COCO_MAX_A && area_rng, "coco_match: 1 <= A <= %d area ranges", YB_COCO_MAX_A);
-    YB_CHECK_ARG(max_gt >= 0 && max_gt <= YB_MAP_MAX_GT, "coco_match: max_gt must be in [0, %d]", YB_MAP_MAX_GT);
-    if (B == 0) return 0;
     const int slots = max_det < cap ? max_det : cap;
-    YB_CHECK_ARG(n_keep && n_gt && letterbox && iou_thr && gt_count && status && (slots == 0 || records),
-                 "coco_match: null pointer");
-    YB_CHECK_ARG(cap == 0 || (boxes && scores && classes && keep && aligned16(boxes)), "coco_match: null or unaligned candidates");
-    YB_CHECK_ARG(max_gt == 0 || labels, "coco_match: null labels");
-    CocoMatchArgs a{reinterpret_cast<const float4*>(boxes), scores, classes, keep, n_keep, labels, n_gt, letterbox, iou_thr,
-                    records, reinterpret_cast<unsigned long long*>(gt_count), status, {}, cap, slots, max_gt, nc, T, A};
+    CocoMatchArgs a{{reinterpret_cast<const float4*>(boxes), scores, classes, keep, n_keep, labels, n_gt, letterbox, cap,
+                     slots, max_gt, nc},
+                    iou_thr, records, reinterpret_cast<unsigned long long*>(gt_count), status, {}, T, A};
     for (int i = 0; i < 2 * A; ++i) a.rng[i] = area_rng[i];
     const int threads = T * 32 < 128 ? 128 : T * 32;
     const size_t smem = (size_t)max_gt * (sizeof(GtBox) + 2 * sizeof(int)) +
                         (size_t)threads * (sizeof(float4) + 6 * sizeof(int)) +
                         (size_t)T * ((max_gt + 31) / 32) * sizeof(unsigned int) + (size_t)nc * sizeof(int);
-    YB_CHECK_ARG(smem <= (size_t)max_smem_optin(), "coco_match: %zu bytes of shared memory (nc = %d, max_gt = %d) exceed one CTA",
-                 smem, nc, max_gt);
-    if (smem > 48 * 1024) YB_CUDA(cudaFuncSetAttribute(coco_match_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (int e = check_match("coco_match", coco_match_kernel, a.in, B, max_det,
+                            iou_thr && gt_count && status && (slots == 0 || records), smem))
+        return e;
+    if (B == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
     YB_LAUNCH("coco_match_kernel", st, coco_match_kernel<<<dim3(B, A), threads, smem, st>>>(a));
     return 0;

@@ -22,6 +22,7 @@ computed there, and staged back.  That is staging, not a fallback: without CUDA 
 raises.
 """
 import ctypes
+import math
 import zlib
 from typing import List, Optional, Sequence
 
@@ -1016,24 +1017,43 @@ def _raise_status(status, who):
         raise RuntimeError(f"{who}: a class has more true positives than ground truths")
 
 
-class DetectionMAP:
-    """mAP@[.5:.95] and mAP@0.5 of the kept detections of `detect_batch`, accumulated over batches on the device.
-    COCO's bbox protocol (evaluateImg + accumulate, area range "all", no crowd) with one overall cap of `max_det`
-    detections per image instead of COCO's per-category maxDets; include/yolo_b200.h states the semantics.
+def _unpack(host, shapes):
+    """The consecutive pieces of the flat array `host` with the given shapes, as views."""
+    out, o = [], 0
+    for shape in shapes:
+        n = math.prod(shape)
+        out.append(host[o:o + n].reshape(shape))
+        o += n
+    return out
 
-    update(det, labels) enqueues one matching kernel per batch and keeps its records; it never synchronises.
-    compute() sorts the records once, runs the precision kernel and synchronises once.
 
-    compute(group) evaluates an image-sharded run: a collective over the torch.distributed process group `group`
-    (every rank calls it) that returns on every rank the dict one process would return after update() with every
-    rank's batches in rank order (DESIGN §3.11).  It synchronises twice and leaves the local state unchanged.  The
-    result is bit-identical to that process when rank r updated the r-th contiguous block of images
-    (dist.shard_range) in image order.  With any other assignment, such as DistributedSampler's interleaving,
-    n_gt, n_det and recall are still identical, and the precision table (with the AP values taken from it) can
-    differ only through the order of equal-score detections of different images."""
+def _mean_valid(s):
+    """The mean of the entries > -1, -1 when there are none (COCOeval.summarize)."""
+    s = s[s > -1]
+    return float(np.mean(s)) if s.size else -1.0
 
-    def __init__(self, num_classes, iou_thresholds=COCO_IOU_THRESHOLDS, recall_thresholds=COCO_RECALL_THRESHOLDS,
-                 max_det=300):
+
+def _compute_metric(metric, group):
+    """compute(group) of the three metrics: _local_state(), merged over `group` by dist.gather_eval_state, goes
+    through _compute_device into flat float64 device tensors, which _copy_back copies to the host with the status
+    word appended (the one synchronisation, the second with a group); _compute_host reads their _host_shapes()."""
+    with torch.cuda.device(metric.device):
+        state = metric._local_state()
+        if group is not None:
+            from .dist import gather_eval_state
+            state = gather_eval_state(metric._fingerprint(), *state, group)
+        host = metric._copy_back(metric._compute_device(state) + [state[-1].double()])
+    _raise_status(int(host[-1]), type(metric).__name__)
+    return metric._compute_host(_unpack(host, metric._host_shapes()), state)
+
+
+class _MatchMetric:
+    """What DetectionMAP and COCODetectionEval share: the common arguments, update() and the state compute(group)
+    starts from.  A subclass sets _RECORD_WORDS, creates _gt_count and provides _match and the hooks of
+    _compute_metric.  DetectionReport drives its DetectionMAP through update(), _match_prefix, the hooks and _status,
+    the device word every kernel of the metric ORs its YB_MAP_* bits into."""
+
+    def __init__(self, num_classes, iou_thresholds, recall_thresholds, max_det):
         self.nc = int(num_classes)
         self.iou_thresholds = np.asarray(iou_thresholds, dtype=np.float64).reshape(-1)
         self.recall_thresholds = np.asarray(recall_thresholds, dtype=np.float64).reshape(-1)
@@ -1050,66 +1070,101 @@ class DetectionMAP:
         with torch.cuda.device(self.device):
             self._iou_thr = torch.tensor(self.iou_thresholds, dtype=torch.float64, device=self.device)
             self._rec_thr = torch.tensor(self.recall_thresholds, dtype=torch.float64, device=self.device)
-            self._gt_count = torch.zeros(self.nc, dtype=torch.int64, device=self.device)
             self._status = torch.zeros(1, dtype=torch.int32, device=self.device)
-        self.reset()
 
     def reset(self):
         """Forget every batch seen so far."""
         self._records = []
-        self._gt_total = 0   # upper bound on the ground truths seen: sum of B * max_gt (sizes the workspace)
+        self._gt_total = 0   # upper bound on the ground truths seen: sum of B * max_gt (sizes DetectionMAP's workspace)
         with torch.cuda.device(self.device):
             self._gt_count.zero_()
             self._status.zero_()
 
     def update(self, det, labels: PackedLabels):
         """Match one batch: `det` is a detect_batch result (letterbox reversed, original-image pixels) and `labels`
-        the batch's PackedLabels (labels normalised to the original image, letterbox rows [orig_w, orig_h, ...])."""
-        boxes, keep = det["boxes"], det["keep"]
+        the batch's PackedLabels (labels normalised to the original image, letterbox rows [orig_w, orig_h, ...]).
+        Returns the batch's records on the device."""
+        B, cap = self._check_batch(det, labels)
+        with torch.cuda.device(self.device):
+            rec = torch.empty(B * min(self.max_det, cap), self._RECORD_WORDS, dtype=torch.int32, device=self.device)
+            self._match(self._match_prefix(det, labels), rec)
+        self._records.append(rec)
+        self._gt_total += B * labels.max_gt
+        return rec
+
+    def _check_batch(self, det, labels):
+        """update()'s checks of one batch; returns (B, cap)."""
+        boxes = det["boxes"]
         if boxes.device != self.device:
-            raise ValueError(f"detections on {boxes.device}, DetectionMAP on {self.device}")
+            raise ValueError(f"detections on {boxes.device}, {type(self).__name__} on {self.device}")
         B, cap = boxes.shape[0], boxes.shape[1]
         if labels.labels.shape[0] != B or labels.labels.device != self.device:
             raise ValueError("labels and detections disagree on the batch size or the device")
         if labels.max_gt > _lib.MAP_MAX_GT:
             raise ValueError(f"at most {_lib.MAP_MAX_GT} ground truths per image, got max_gt={labels.max_gt}")
-        slots = min(self.max_det, cap)
-        with torch.cuda.device(self.device):
-            rec = torch.empty(B * slots, 3, dtype=torch.int32, device=self.device)   # yb_map_record: score, class, tp
-            _lib.check(_lib.lib().yb_map_match(
-                boxes.data_ptr(), det["scores"].data_ptr(), det["classes"].data_ptr(), keep.data_ptr(),
+        return B, cap
+
+    def _match_prefix(self, det, labels):
+        """The arguments every yb_*_match entry point starts with: the batch's candidates and kept lists, max_det, its
+        labels and num_classes."""
+        B, cap = det["boxes"].shape[0], det["boxes"].shape[1]
+        return (det["boxes"].data_ptr(), det["scores"].data_ptr(), det["classes"].data_ptr(), det["keep"].data_ptr(),
                 det["n_keep"].data_ptr(), B, cap, self.max_det, labels.labels.data_ptr(), labels.n_gt.data_ptr(),
-                labels.letterbox.data_ptr(), labels.max_gt, self.nc, self._iou_thr.data_ptr(), len(self.iou_thresholds),
-                rec.data_ptr(), self._gt_count.data_ptr(), self._status.data_ptr(), _stream()), "yb_map_match")
-        self._records.append(rec)
-        self._gt_total += B * labels.max_gt
+                labels.letterbox.data_ptr(), labels.max_gt, self.nc)
+
+    def _local_state(self):
+        """(records in image order, gt_count, gt_total, images_total, status) of this process."""
+        rec = (torch.cat(self._records) if self._records
+               else torch.empty(0, self._RECORD_WORDS, dtype=torch.int32, device=self.device))
+        return rec, self._gt_count, self._gt_total, 0, self._status
+
+    def _copy_back(self, tensors):
+        return torch.cat(tensors).cpu().numpy()
+
+
+class DetectionMAP(_MatchMetric):
+    """mAP@[.5:.95] and mAP@0.5 of the kept detections of `detect_batch`, accumulated over batches on the device.
+    COCO's bbox protocol (evaluateImg + accumulate, area range "all", no crowd) with one overall cap of `max_det`
+    detections per image instead of COCO's per-category maxDets; include/yolo_b200.h states the semantics.
+
+    update(det, labels) enqueues one matching kernel per batch and keeps its records; it never synchronises.
+    compute() sorts the records once, runs the precision kernel and synchronises once.
+
+    compute(group) evaluates an image-sharded run: a collective over the torch.distributed process group `group`
+    (every rank calls it) that returns on every rank the dict one process would return after update() with every
+    rank's batches in rank order (DESIGN §3.11).  It synchronises twice and leaves the local state unchanged.  The
+    result is bit-identical to that process when rank r updated the r-th contiguous block of images
+    (dist.shard_range) in image order.  With any other assignment, such as DistributedSampler's interleaving,
+    n_gt, n_det and recall are still identical, and the precision table (with the AP values taken from it) can
+    differ only through the order of equal-score detections of different images."""
+    _RECORD_WORDS = 3   # yb_map_record: score, class, tp
+
+    def __init__(self, num_classes, iou_thresholds=COCO_IOU_THRESHOLDS, recall_thresholds=COCO_RECALL_THRESHOLDS,
+                 max_det=300):
+        super().__init__(num_classes, iou_thresholds, recall_thresholds, max_det)
+        with torch.cuda.device(self.device):
+            self._gt_count = torch.zeros(self.nc, dtype=torch.int64, device=self.device)
+        self.reset()
+
+    def _match(self, prefix, rec):
+        _lib.check(_lib.lib().yb_map_match(*prefix, self._iou_thr.data_ptr(), len(self.iou_thresholds), rec.data_ptr(),
+                                           self._gt_count.data_ptr(), self._status.data_ptr(), _stream()),
+                   "yb_map_match")
 
     def compute(self, group=None):
         """{map, map50, ap (nc,T), precision (T,R,nc), recall (T,nc), n_gt (nc), n_det (nc)} on the host (float64 /
         int64; map50 is None when 0.5 is not a threshold).  Entries of a class without ground truth are -1, and
         map / map50 are the means of the entries > -1 (-1 when there are none), as COCOeval.summarize.
         group: a torch.distributed process group to merge over (see the class docstring)."""
-        with torch.cuda.device(self.device):
-            state = self._local_state()
-            if group is not None:
-                from .dist import gather_eval_state
-                fp = _eval_fingerprint(1, self.nc, len(self.iou_thresholds), len(self.recall_thresholds), 0, 0, 0,
-                                       self.max_det, (self.iou_thresholds, self.recall_thresholds))
-                rec, gt_count, gt_total, _, status = gather_eval_state(fp, *state[:3], 0, state[3], group)
-                state = (rec, gt_count, gt_total, status)
-            host = torch.cat(self._compute_device(*state)).cpu().numpy()   # the one synchronisation (2nd with a group)
-        return self._compute_host(host, "DetectionMAP")
+        return _compute_metric(self, group)
 
-    def _local_state(self):
-        """(records in image order, gt_count, gt_total, status): what _compute_device reads of one process."""
-        rec = (torch.cat(self._records) if self._records
-               else torch.empty(0, 3, dtype=torch.int32, device=self.device))
-        return rec, self._gt_count, self._gt_total, self._status
+    def _fingerprint(self):
+        return _eval_fingerprint(1, self.nc, len(self.iou_thresholds), len(self.recall_thresholds), 0, 0, 0,
+                                 self.max_det, (self.iou_thresholds, self.recall_thresholds))
 
-    def _compute_device(self, rec, gt_count, gt_total, status):
-        """Device half of compute() on the state _local_state returns or a merge of it: sort the records and run the
-        precision kernel.  Returns the flat float64 device tensors compute() copies back, in the order _compute_host
-        reads them (the status word last)."""
+    def _compute_device(self, state):
+        """Sort the records and run the precision kernel: precision, recall, gt_count and seg as flat float64."""
+        rec, gt_count, gt_total, _, status = state
         T, R, nc = len(self.iou_thresholds), len(self.recall_thresholds), self.nc
         dev = self.device
         rec, seg = _sort_records(rec, nc)
@@ -1122,35 +1177,23 @@ class DetectionMAP:
                                                self._rec_thr.data_ptr(), R, precision.data_ptr(), recall.data_ptr(),
                                                ws.data_ptr(), ws_bytes, status.data_ptr(), _stream()),
                    "yb_map_precision")
-        return [precision.reshape(-1), recall.reshape(-1), gt_count.double(), seg.double(), status.double()]
+        return [precision.reshape(-1), recall.reshape(-1), gt_count.double(), seg.double()]
 
-    def _host_size(self):
-        """Number of doubles _compute_device's tensors hold."""
+    def _host_shapes(self):
         T, R, nc = len(self.iou_thresholds), len(self.recall_thresholds), self.nc
-        return T * R * nc + T * nc + nc + nc + 1 + 1
+        return [(T, R, nc), (T, nc), (nc,), (nc + 1,)]
 
-    def _compute_host(self, host, who):
-        """Host half of compute(): raise on the status bits, unpack the first _host_size() doubles of `host` and
-        summarise them."""
-        T, R, nc = len(self.iou_thresholds), len(self.recall_thresholds), self.nc
-        _raise_status(int(host[self._host_size() - 1]), who)
-        o = 0
-        precision = host[o:o + T * R * nc].reshape(T, R, nc); o += T * R * nc
-        recall = host[o:o + T * nc].reshape(T, nc); o += T * nc
-        n_gt = host[o:o + nc].astype(np.int64); o += nc
-        n_det = np.diff(host[o:o + nc + 1]).astype(np.int64)
+    def _compute_host(self, parts, state):
+        precision, recall, n_gt, seg = parts[:4]
         return dict(summarize_precision(precision, self.iou_thresholds), precision=precision, recall=recall,
-                    n_gt=n_gt, n_det=n_det)
+                    n_gt=n_gt.astype(np.int64), n_det=np.diff(seg).astype(np.int64))
 
 
 def summarize_precision(precision, iou_thresholds):
     """map, map50 and ap (nc,T) from a (T,R,nc) precision table, as COCOeval.summarize averages it."""
-    def mean(s):
-        s = s[s > -1]
-        return float(np.mean(s)) if s.size else -1.0
     hit = np.flatnonzero(np.asarray(iou_thresholds) == 0.5)
     ap = np.where(precision.min(axis=1) > -1, precision.mean(axis=1), -1.0).T   # (nc,T)
-    return {"map": mean(precision), "map50": mean(precision[hit]) if hit.size else None, "ap": ap}
+    return {"map": _mean_valid(precision), "map50": _mean_valid(precision[hit]) if hit.size else None, "ap": ap}
 
 
 COCO_AREA_RANGES = ((0.0, 1e5 ** 2), (0.0, 32.0 ** 2), (32.0 ** 2, 96.0 ** 2), (96.0 ** 2, 1e5 ** 2))   # Params.areaRng
@@ -1158,7 +1201,7 @@ COCO_AREA_LABELS = ("all", "small", "medium", "large")                          
 COCO_MAX_DETS = (1, 10, 100)                                                                          # Params.maxDets
 
 
-class COCODetectionEval:
+class COCODetectionEval(_MatchMetric):
     """COCO's bbox summary of the kept detections of `detect_batch`, accumulated over batches on the device: the
     twelve numbers pycocotools prints (AP, AP50, AP75, AP_S/M/L, AR@maxDets, AR_S/M/L) and COCOeval.eval's
     precision (T,R,nc,A,M) and recall (T,nc,A,M) tables.  COCO's protocol (evaluateImg + accumulate + summarize,
@@ -1178,63 +1221,28 @@ class COCODetectionEval:
     rank r updated the r-th contiguous block of images in image order.  With any other assignment n_gt, n_det and
     recall are still identical, and precision (with the stats and AP values taken from it) can differ only through
     the order of equal-score detections of different images."""
+    _RECORD_WORDS = 8   # yb_coco_record, 32 bytes
 
     def __init__(self, num_classes, iou_thresholds=COCO_IOU_THRESHOLDS, recall_thresholds=COCO_RECALL_THRESHOLDS,
                  max_det=300, max_dets=COCO_MAX_DETS):
-        self.nc = int(num_classes)
-        self.iou_thresholds = np.asarray(iou_thresholds, dtype=np.float64).reshape(-1)
-        self.recall_thresholds = np.asarray(recall_thresholds, dtype=np.float64).reshape(-1)
-        self.max_det = int(max_det)
+        super().__init__(num_classes, iou_thresholds, recall_thresholds, max_det)
         self.max_dets = tuple(int(m) for m in max_dets)
         self.area_ranges = np.asarray(COCO_AREA_RANGES, dtype=np.float64)
-        if self.nc < 1:
-            raise ValueError("num_classes must be >= 1")
-        if not 1 <= len(self.iou_thresholds) <= _lib.MAP_MAX_T:
-            raise ValueError(f"1..{_lib.MAP_MAX_T} IoU thresholds supported, got {len(self.iou_thresholds)}")
-        if len(self.recall_thresholds) < 1 or not np.all(np.diff(self.recall_thresholds) >= 0):
+        if not np.all(np.diff(self.recall_thresholds) >= 0):
             raise ValueError("recall_thresholds must be a non-empty ascending sequence")
-        if self.max_det < 0:
-            raise ValueError("max_det must be >= 0")
         if len(self.max_dets) != 3 or not all(1 <= m <= 65535 for m in self.max_dets):
             raise ValueError(f"max_dets must be three values in [1, 65535], got {max_dets}")
-        self.device = _device()
         with torch.cuda.device(self.device):
-            self._iou_thr = torch.tensor(self.iou_thresholds, dtype=torch.float64, device=self.device)
-            self._rec_thr = torch.tensor(self.recall_thresholds, dtype=torch.float64, device=self.device)
             self._gt_count = torch.zeros(len(self.area_ranges), self.nc, dtype=torch.int64, device=self.device)
-            self._status = torch.zeros(1, dtype=torch.int32, device=self.device)
         self._rng_host = (ctypes.c_double * self.area_ranges.size)(*self.area_ranges.reshape(-1).tolist())
         self._md_host = (ctypes.c_int * len(self.max_dets))(*self.max_dets)
         self.reset()
 
-    def reset(self):
-        """Forget every batch seen so far."""
-        self._records = []
-        with torch.cuda.device(self.device):
-            self._gt_count.zero_()
-            self._status.zero_()
-
-    def update(self, det, labels: PackedLabels):
-        """Match one batch: `det` is a detect_batch result (letterbox reversed, original-image pixels) and `labels`
-        the batch's PackedLabels (labels normalised to the original image, letterbox rows [orig_w, orig_h, ...])."""
-        boxes, keep = det["boxes"], det["keep"]
-        if boxes.device != self.device:
-            raise ValueError(f"detections on {boxes.device}, COCODetectionEval on {self.device}")
-        B, cap = boxes.shape[0], boxes.shape[1]
-        if labels.labels.shape[0] != B or labels.labels.device != self.device:
-            raise ValueError("labels and detections disagree on the batch size or the device")
-        if labels.max_gt > _lib.MAP_MAX_GT:
-            raise ValueError(f"at most {_lib.MAP_MAX_GT} ground truths per image, got max_gt={labels.max_gt}")
-        slots = min(self.max_det, cap)
-        with torch.cuda.device(self.device):
-            rec = torch.empty(B * slots, 8, dtype=torch.int32, device=self.device)   # yb_coco_record, 32 bytes
-            _lib.check(_lib.lib().yb_coco_match(
-                boxes.data_ptr(), det["scores"].data_ptr(), det["classes"].data_ptr(), keep.data_ptr(),
-                det["n_keep"].data_ptr(), B, cap, self.max_det, labels.labels.data_ptr(), labels.n_gt.data_ptr(),
-                labels.letterbox.data_ptr(), labels.max_gt, self.nc, self._iou_thr.data_ptr(), len(self.iou_thresholds),
-                self._rng_host, len(self.area_ranges), rec.data_ptr(), self._gt_count.data_ptr(),
-                self._status.data_ptr(), _stream()), "yb_coco_match")
-        self._records.append(rec)
+    def _match(self, prefix, rec):
+        _lib.check(_lib.lib().yb_coco_match(*prefix, self._iou_thr.data_ptr(), len(self.iou_thresholds),
+                                            self._rng_host, len(self.area_ranges), rec.data_ptr(),
+                                            self._gt_count.data_ptr(), self._status.data_ptr(), _stream()),
+                   "yb_coco_match")
 
     def compute(self, group=None):
         """{stats (12,), precision (T,R,nc,A,M), recall (T,nc,A,M), n_gt (nc,A), n_det (nc), and ap (nc,T), map,
@@ -1242,40 +1250,38 @@ class COCODetectionEval:
         ground truth are -1; stats are pycocotools' _summarizeDets, map / map50 DetectionMAP's means.  n_gt counts
         the ground truths inside each area range, n_det the records of each class (at most max_det per image).
         group: a torch.distributed process group to merge over (see the class docstring)."""
+        return _compute_metric(self, group)
+
+    def _fingerprint(self):
+        return _eval_fingerprint(2, self.nc, len(self.iou_thresholds), len(self.recall_thresholds),
+                                 len(self.area_ranges), len(self.max_dets), 0, self.max_det,
+                                 (self.iou_thresholds, self.recall_thresholds, self.area_ranges, self.max_dets))
+
+    def _compute_device(self, state):
+        """Sort the records and run the precision kernel: precision, recall, gt_count and seg as flat float64."""
+        rec, gt_count, _, _, status = state
+        T, R, nc, dev = len(self.iou_thresholds), len(self.recall_thresholds), self.nc, self.device
+        A, M = len(self.area_ranges), len(self.max_dets)
+        rec, seg = _sort_records(rec, nc)
+        precision = torch.empty(T, R, nc, A, M, dtype=torch.float64, device=dev)
+        recall = torch.empty(T, nc, A, M, dtype=torch.float64, device=dev)
+        _lib.check(_lib.lib().yb_coco_precision(rec.data_ptr(), seg.data_ptr(), gt_count.data_ptr(), nc, A, T,
+                                                self._rec_thr.data_ptr(), R, self._md_host, M, precision.data_ptr(),
+                                                recall.data_ptr(), status.data_ptr(), _stream()),
+                   "yb_coco_precision")
+        return [precision.reshape(-1), recall.reshape(-1), gt_count.reshape(-1).double(), seg.double()]
+
+    def _host_shapes(self):
         T, R, nc = len(self.iou_thresholds), len(self.recall_thresholds), self.nc
         A, M = len(self.area_ranges), len(self.max_dets)
-        dev = self.device
-        with torch.cuda.device(dev):
-            rec = torch.cat(self._records) if self._records else torch.empty(0, 8, dtype=torch.int32, device=dev)
-            gt_count, status = self._gt_count, self._status
-            if group is not None:
-                from .dist import gather_eval_state
-                fp = _eval_fingerprint(2, nc, T, R, A, M, 0, self.max_det,
-                                       (self.iou_thresholds, self.recall_thresholds, self.area_ranges, self.max_dets))
-                rec, gt_count, _, _, status = gather_eval_state(fp, rec, gt_count, 0, 0, status, group)
-            rec, seg = _sort_records(rec, nc)
-            precision = torch.empty(T, R, nc, A, M, dtype=torch.float64, device=dev)
-            recall = torch.empty(T, nc, A, M, dtype=torch.float64, device=dev)
-            _lib.check(_lib.lib().yb_coco_precision(rec.data_ptr(), seg.data_ptr(), gt_count.data_ptr(), nc, A, T,
-                                                    self._rec_thr.data_ptr(), R, self._md_host, M, precision.data_ptr(),
-                                                    recall.data_ptr(), status.data_ptr(), _stream()),
-                       "yb_coco_precision")
-            host = torch.cat([precision.reshape(-1), recall.reshape(-1), gt_count.reshape(-1).double(),
-                              seg.double(), status.double()]).cpu().numpy()   # the one sync (2nd with a group)
-        _raise_status(int(host[-1]), "COCODetectionEval")
-        o = 0
-        precision = host[o:o + T * R * nc * A * M].reshape(T, R, nc, A, M); o += T * R * nc * A * M
-        recall = host[o:o + T * nc * A * M].reshape(T, nc, A, M); o += T * nc * A * M
-        n_gt = host[o:o + A * nc].reshape(A, nc).T.astype(np.int64); o += A * nc
-        n_det = np.diff(host[o:o + nc + 1]).astype(np.int64)
+        return [(T, R, nc, A, M), (T, nc, A, M), (A, nc), (nc + 1,)]
+
+    def _compute_host(self, parts, state):
+        precision, recall, n_gt, seg = parts
         stats = summarize_coco(precision, recall, self.iou_thresholds, self.max_dets)
-        return dict(summarize_precision(precision[..., 0, M - 1], self.iou_thresholds), stats=stats,
-                    precision=precision, recall=recall, n_gt=n_gt, n_det=n_det)
-
-
-def _coco_mean(s):
-    s = s[s > -1]
-    return float(np.mean(s)) if s.size else -1.0
+        return dict(summarize_precision(precision[..., 0, -1], self.iou_thresholds), stats=stats,
+                    precision=precision, recall=recall, n_gt=n_gt.T.astype(np.int64),
+                    n_det=np.diff(seg).astype(np.int64))
 
 
 def summarize_coco(precision, recall, iou_thresholds, max_dets, area_labels=COCO_AREA_LABELS):
@@ -1290,7 +1296,7 @@ def summarize_coco(precision, recall, iou_thresholds, max_dets, area_labels=COCO
         if iou_thr is not None:
             s = s[np.where(iou_thr == iou_thresholds)[0]]
         s = s[:, :, :, aind, mind] if ap else s[:, :, aind, mind]
-        return _coco_mean(s)
+        return _mean_valid(s)
 
     md = max_dets
     return np.array([summ(1), summ(1, .5, md=md[2]), summ(1, .75, md=md[2]), summ(1, area="small", md=md[2]),
@@ -1354,41 +1360,35 @@ class DetectionReport:
         if not (np.isfinite(self.cm_conf) and np.isfinite(self.cm_iou)):
             raise ValueError("cm_conf and cm_iou must be finite")
         nc, K, dev = self.nc, self.conf_grid.size, self.map.device
+        self.device = dev
         with torch.cuda.device(dev):
             self._grid = torch.tensor(self.conf_grid, dtype=torch.float64, device=dev)
             # one buffer, zeroed at once: confusion (nc+1)^2, images (nc), det_hist (nc,K), tp_hist (nc,K)
             self._counts = torch.zeros((nc + 1) ** 2 + nc + 2 * nc * K, dtype=torch.int64, device=dev)
         # compute()'s one copy back goes to page-locked memory: about 16 bytes per class and grid point
-        self._host = torch.empty(self.map._host_size() + (nc + 1) ** 2 + nc + 2 * nc * K, dtype=torch.float64,
+        self._host = torch.empty(sum(map(math.prod, self._host_shapes())) + 1, dtype=torch.float64,
                                  pin_memory=True)
-        o = 0
-        self._confusion = self._counts[o:o + (nc + 1) ** 2].view(nc + 1, nc + 1); o += (nc + 1) ** 2
-        self._images = self._counts[o:o + nc]; o += nc
-        self._det_hist = self._counts[o:o + nc * K].view(nc, K); o += nc * K
-        self._tp_hist = self._counts[o:o + nc * K].view(nc, K)
+        self._confusion, self._images, self._det_hist, self._tp_hist = _unpack(
+            self._counts, [(nc + 1, nc + 1), (nc,), (nc, K), (nc, K)])
         self.reset()
 
     def reset(self):
         """Forget every batch seen so far."""
         self.map.reset()
         self.images_total = 0
-        with torch.cuda.device(self.map.device):
+        with torch.cuda.device(self.device):
             self._counts.zero_()
 
     def update(self, det, labels: PackedLabels):
         """Match one batch: the arguments of DetectionMAP.update.  After an error, reset() before the next update."""
-        self.map.update(det, labels)
-        boxes, keep = det["boxes"], det["keep"]
-        B, cap = boxes.shape[0], boxes.shape[1]
-        with torch.cuda.device(self.map.device):
+        rec = self.map.update(det, labels)
+        with torch.cuda.device(self.device):
             _lib.check(_lib.lib().yb_report_match(
-                boxes.data_ptr(), det["scores"].data_ptr(), det["classes"].data_ptr(), keep.data_ptr(),
-                det["n_keep"].data_ptr(), B, cap, self.map.max_det, labels.labels.data_ptr(), labels.n_gt.data_ptr(),
-                labels.letterbox.data_ptr(), labels.max_gt, self.nc, self.map._records[-1].data_ptr(), self._t_curve,
-                self._grid.data_ptr(), self.conf_grid.size, self.cm_conf, self.cm_iou, self._confusion.data_ptr(),
-                self._images.data_ptr(), self._det_hist.data_ptr(), self._tp_hist.data_ptr(),
-                self.map._status.data_ptr(), _stream()), "yb_report_match")
-        self.images_total += B
+                *self.map._match_prefix(det, labels), rec.data_ptr(), self._t_curve, self._grid.data_ptr(),
+                self.conf_grid.size, self.cm_conf, self.cm_iou, self._confusion.data_ptr(), self._images.data_ptr(),
+                self._det_hist.data_ptr(), self._tp_hist.data_ptr(), self.map._status.data_ptr(), _stream()),
+                "yb_report_match")
+        self.images_total += det["boxes"].shape[0]
 
     def compute(self, group=None):
         """DetectionMAP.compute()'s dict plus, on the host:
@@ -1397,35 +1397,45 @@ class DetectionReport:
         first arg-max of the mean F1 over the classes with ground truth (None when there are none); p, r, f1 (nc,)
         at k*; confusion (nc+1,nc+1) and images (nc) int64; images_total; iou_thresholds (the columns of ap).
         group: a torch.distributed process group to merge over (see the class docstring)."""
+        return _compute_metric(self, group)
+
+    def _local_state(self):
+        """The map's state with this report's counts appended to gt_count, and images_total."""
+        rec, gt_count, gt_total, _, status = self.map._local_state()
+        return rec, torch.cat([gt_count, self._counts]), gt_total, self.images_total, status
+
+    def _fingerprint(self):
+        mp = self.map
+        return _eval_fingerprint(3, self.nc, len(mp.iou_thresholds), len(mp.recall_thresholds), 0, 0, self.conf_grid.size,
+                                 mp.max_det, (mp.iou_thresholds, mp.recall_thresholds, self.conf_grid,
+                                              (self.curve_iou, self.cm_conf, self.cm_iou)))
+
+    def _compute_device(self, state):
+        """The map's tensors, then the confusion matrix and images, then the histograms' suffix sums."""
+        rec, counts, gt_total, images_total, status = state
         nc, K = self.nc, self.conf_grid.size
-        m = self.map._host_size()
-        with torch.cuda.device(self.map.device):
-            rec, gt_count, gt_total, status = self.map._local_state()
-            counts, images_total = self._counts, self.images_total
-            if group is not None:
-                from .dist import gather_eval_state
-                mp = self.map
-                fp = _eval_fingerprint(3, nc, len(mp.iou_thresholds), len(mp.recall_thresholds), 0, 0, K, mp.max_det,
-                                       (mp.iou_thresholds, mp.recall_thresholds, self.conf_grid,
-                                        (self.curve_iou, self.cm_conf, self.cm_iou)))
-                rec, both, gt_total, images_total, status = gather_eval_state(
-                    fp, rec, torch.cat([gt_count, counts]), gt_total, images_total, status, group)
-                gt_count, counts = both[:nc], both[nc:]
-            hist = counts[(nc + 1) ** 2 + nc:].view(2, nc, K)   # det_hist, tp_hist
-            rev = hist.flip(2).cumsum(2)   # [.., K-1-k] = detections / TPs with score > grid[k]
-            dev = torch.cat(self.map._compute_device(rec, gt_count, gt_total, status)
-                            + [counts[:(nc + 1) ** 2 + nc].double(), rev.reshape(-1).double()])
-            self._host.copy_(dev, non_blocking=True)
-            torch.cuda.current_stream().synchronize()   # the one synchronisation (the second with a group)
-        host = self._host.numpy()
-        out = self.map._compute_host(host[:m].copy(), "DetectionReport")   # its tables are returned as views
-        o = m
-        confusion = host[o:o + (nc + 1) ** 2].astype(np.int64).reshape(nc + 1, nc + 1); o += (nc + 1) ** 2
-        images = host[o:o + nc].astype(np.int64); o += nc
-        n_det = host[o:o + nc * K].astype(np.int64).reshape(nc, K)[:, ::-1]; o += nc * K
-        n_tp = host[o:o + nc * K].astype(np.int64).reshape(nc, K)[:, ::-1]
-        out.update(report_curves(n_det, n_tp, out["n_gt"], self.conf_grid), confusion=confusion, images=images,
-                   images_total=images_total, iou_thresholds=self.map.iou_thresholds.copy())
+        gt_count, counts = counts[:nc], counts[nc:]
+        hist = counts[(nc + 1) ** 2 + nc:].view(2, nc, K)   # det_hist, tp_hist
+        rev = hist.flip(2).cumsum(2)   # [.., K-1-k] = detections / TPs with score > grid[k]
+        return (self.map._compute_device((rec, gt_count, gt_total, images_total, status))
+                + [counts[:(nc + 1) ** 2 + nc].double(), rev.reshape(-1).double()])
+
+    def _copy_back(self, tensors):
+        self._host.copy_(torch.cat(tensors), non_blocking=True)
+        torch.cuda.current_stream().synchronize()
+        return self._host.numpy()
+
+    def _host_shapes(self):
+        nc, K = self.nc, self.conf_grid.size
+        return self.map._host_shapes() + [(nc + 1, nc + 1), (nc,), (2, nc, K)]
+
+    def _compute_host(self, parts, state):
+        m = len(self.map._host_shapes())
+        out = self.map._compute_host([p.copy() for p in parts[:m]], state)   # it returns views; the buffer is reused
+        confusion, images, hist = parts[m:]
+        n_det, n_tp = hist.astype(np.int64)[:, :, ::-1]
+        out.update(report_curves(n_det, n_tp, out["n_gt"], self.conf_grid), confusion=confusion.astype(np.int64),
+                   images=images.astype(np.int64), images_total=state[3], iou_thresholds=self.map.iou_thresholds.copy())
         return out
 
 
