@@ -24,7 +24,7 @@ raises.
 import ctypes
 import math
 import zlib
-from typing import List, Optional, Sequence
+from typing import List, NamedTuple, Optional, Sequence
 
 import numpy as np
 import torch
@@ -70,39 +70,20 @@ def _ptr(t: Optional[torch.Tensor]) -> int:
     return 0 if t is None else t.data_ptr()
 
 
-def _f32c(t: torch.Tensor, dev: torch.device) -> torch.Tensor:
-    """fp32, contiguous, on `dev`, 16-byte aligned (differentiable)."""
-    if t.device != dev:
-        t = t.to(dev)
-    if t.dtype != torch.float32:
-        t = t.float()
-    t = t.contiguous()
-    if t.data_ptr() % 16:
-        t = t.clone()
-    return t
-
-
 _HEAD_DTYPES = {torch.float32: _lib.DTYPE_F32, torch.bfloat16: _lib.DTYPE_BF16, torch.float16: _lib.DTYPE_F16}
 
 
-def _headc(t: torch.Tensor, dev: torch.device) -> torch.Tensor:
-    """A head tensor as the kernels read it: fp32, bf16 and fp16 keep their dtype (a CPU half tensor is staged as
-    half), any other dtype becomes fp32; contiguous, on `dev`, 16-byte aligned (differentiable)."""
+def _contig(t: torch.Tensor, dev: torch.device, half: bool = False) -> torch.Tensor:
+    """`t` as the kernels read it: on `dev`, contiguous, 16-byte aligned (differentiable); fp32, or with half=True
+    bf16 and fp16 kept as they are (a CPU half tensor is staged as half) and any other dtype made fp32."""
     if t.device != dev:
         t = t.to(dev)
-    if t.dtype not in _HEAD_DTYPES:
+    if t.dtype != torch.float32 and not (half and t.dtype in _HEAD_DTYPES):
         t = t.float()
     t = t.contiguous()
     if t.data_ptr() % 16:
         t = t.clone()
     return t
-
-
-def _same_dtype(ts: List[torch.Tensor]) -> List[torch.Tensor]:
-    """Heads of mixed dtypes are all read as fp32."""
-    if len({t.dtype for t in ts}) > 1:
-        ts = [t.float() for t in ts]
-    return ts
 
 
 _anchor_cache = {}
@@ -132,13 +113,98 @@ def default_anchors(device=None) -> List[torch.Tensor]:
     return [torch.tensor(a, dtype=torch.float32, device=device) for a in DEFAULT_ANCHORS]
 
 
-def _check_head(t: torch.Tensor, what: str):
-    if t.dim() != 5:
-        raise ValueError(f"{what} must be (B, H, W, A, 5+nc), got {tuple(t.shape)}")
-    if t.shape[3] > MAX_ANCHORS:
-        raise ValueError(f"{what}: at most {MAX_ANCHORS} anchors per scale")
-    if t.shape[4] < 5:
-        raise ValueError(f"{what}: last dimension must be 5+nc")
+LAYOUT_BHWAC, LAYOUT_NCHW = _lib.LAYOUT_BHWAC, _lib.LAYOUT_NCHW
+
+
+def _grid(p: torch.Tensor, layout: int):
+    """(H, W) of a head tensor: (B,H,W,A,5+nc) or, NCHW, (B, A*(5+nc), H, W)."""
+    return (p.shape[2], p.shape[3]) if layout == LAYOUT_NCHW else (p.shape[1], p.shape[2])
+
+
+def _stage_heads(predictions, anchors_list, num_classes, layout, targets=None, *, half=True, detach=True, dev=None):
+    """Heads, anchors and dense targets as the kernels read them: every op that reads head tensors stages them here.
+
+    The kernels receive pointers and the sizes of one descriptor: B of scale 0, A of the first anchor set and rows
+    of 5+nc.  So every scale's shapes are checked first, on the host, before anything touches the device; a
+    mismatch raises ValueError naming the scale.
+
+    predictions: S heads (B,H,W,A,5+nc), or (B,A*(5+nc),H,W) with layout=LAYOUT_NCHW.  num_classes: None takes nc
+    from scale 0's rows (reference layout).  targets: None, S dense targets (B,H,W,A,5+nc) in either layout, or a
+    PackedLabels.  half: bf16 / fp16 heads are kept (heads of mixed dtypes are all read as fp32); False reads every
+    head as fp32.  detach: drop the heads' autograd history (the filters do; the loss and decode keep it).
+    dev: where to stage, None = the current CUDA device.
+    Returns (preds, tgts, ancs), S device tensors each; tgts is None unless dense targets were given."""
+    S = len(predictions)
+    if not 1 <= S <= MAX_SCALES:
+        raise ValueError(f"1..{MAX_SCALES} scales supported, got {S}")
+    dense = targets is not None and not isinstance(targets, PackedLabels)
+    if len(anchors_list) < S:
+        raise ValueError(f"scale {len(anchors_list)}: no anchor set ({S} heads, {len(anchors_list)} anchor sets)")
+    if dense and len(targets) < S:
+        raise ValueError(f"scale {len(targets)}: no targets ({S} heads, {len(targets)} targets)")
+    nc = None if num_classes is None else int(num_classes)
+    if nc is not None and nc < 0:
+        raise ValueError(f"num_classes must be >= 0, got {nc}")
+    for s, p in enumerate(predictions):
+        a = anchors_list[s]
+        a_shape = a.shape if isinstance(a, torch.Tensor) else np.shape(a)
+        if len(a_shape) != 2 or a_shape[1] != 2:
+            raise ValueError(f"scale {s}: anchors must be (A, 2), got shape {tuple(a_shape)}")
+        A = a_shape[0]
+        if A > MAX_ANCHORS:
+            raise ValueError(f"scale {s}: at most {MAX_ANCHORS} anchors per scale, got {A}")
+        shape = p.shape
+        if layout == LAYOUT_NCHW:
+            if len(shape) != 4 or shape[1] != A * (5 + nc):
+                raise ValueError(f"scale {s}: NCHW head must be (B, {A}*(5+num_classes), H, W), got {tuple(shape)}")
+            B, _, H, W = shape
+        else:
+            if len(shape) != 5:
+                raise ValueError(f"scale {s}: head must be (B, H, W, A, 5+nc), got {tuple(shape)}")
+            B, H, W, A_head, row = shape
+            if row < 5:
+                raise ValueError(f"scale {s}: last dimension must be 5+nc, got {row}")
+            if nc is None:
+                nc = row - 5
+            if A_head != A:
+                raise ValueError(f"scale {s}: head has {A_head} anchors, its anchor set {A}")
+            if row != 5 + nc:
+                raise ValueError(f"scale {s}: last dimension {row} != 5+num_classes = {5 + nc}")
+        if s == 0:
+            B0, A0 = B, A
+        elif B != B0:
+            raise ValueError(f"scale {s}: batch {B}, scale 0 has {B0}")
+        elif A != A0:
+            raise ValueError(f"scale {s}: {A} anchors, scale 0 has {A0}")
+        if dense:
+            t = targets[s]
+            if not isinstance(t, torch.Tensor) or t.shape != (B, H, W, A, 5 + nc):
+                got = tuple(t.shape) if isinstance(t, torch.Tensor) else t
+                raise ValueError(f"scale {s}: targets {got} do not match the head, expected {(B, H, W, A, 5 + nc)}")
+    if isinstance(targets, PackedLabels) and targets.labels.shape[0] != B0:
+        raise ValueError(f"labels of {targets.labels.shape[0]} images, the heads' batch is {B0} (scale 0)")
+    if dev is None:
+        dev = _device()
+    preds = [_contig(p.detach() if detach else p, dev, half) for p in predictions]
+    if len({p.dtype for p in preds}) > 1:
+        preds = [p.float() for p in preds]
+    tgts = [_contig(t.detach(), dev) for t in targets[:S]] if dense else None
+    ancs = [_anchors_dev(a, dev) for a in anchors_list[:S]]
+    return preds, tgts, ancs
+
+
+def _heads_desc(d, preds, ancs, nc, img_size, layout):
+    """Fill the fields yb_heads_desc and yb_loss_desc share (S, B, A, nc, img_size, layout, dtype, H, W, pred,
+    anchors) of `d` from staged heads; returns d."""
+    d.S, d.B, d.A, d.nc = len(preds), preds[0].shape[0], ancs[0].shape[0], nc
+    d.img_size = float(img_size)
+    d.layout = layout
+    d.dtype = _HEAD_DTYPES[preds[0].dtype]
+    for s, p in enumerate(preds):
+        d.H[s], d.W[s] = _grid(p, layout)
+        d.pred[s] = p.data_ptr()
+        d.anchors[s] = ancs[s].data_ptr()
+    return d
 
 
 # --------------------------------------------------------------------------------------------
@@ -159,7 +225,7 @@ class _DecodeFn(torch.autograd.Function):
     def backward(ctx, grad_out):
         pred, anchors = ctx.saved_tensors
         B, H, W, A, row = pred.shape
-        grad_out = _headc(grad_out.to(pred.dtype), pred.device)
+        grad_out = _contig(grad_out.to(pred.dtype), pred.device, half=True)
         grad_in = torch.empty_like(pred)
         _lib.check(_lib.lib().yb_decode_bwd_t(pred.data_ptr(), anchors.data_ptr(), grad_out.data_ptr(),
                                               grad_in.data_ptr(), B, H, W, A, row - 5, ctx.img_size,
@@ -171,14 +237,10 @@ def decode_predictions(raw_preds: torch.Tensor, anchors, img_size=640) -> torch.
     """train.py:712-779.  (B,H,W,A,5+nc) raw logits -> same shape with xywh decoded to
     normalised coordinates; objectness/class logits unchanged.  Differentiable.  bf16 / fp16 heads are
     decoded natively: the result is the fp32 decode of the upcast heads rounded to the head dtype."""
-    _check_head(raw_preds, "raw_preds")
-    dev = _device()
+    (pred,), _, (anc,) = _stage_heads([raw_preds], [anchors], None, LAYOUT_BHWAC, detach=False)
+    dev = pred.device
     orig_dev, orig_dtype = raw_preds.device, raw_preds.dtype
     with torch.cuda.device(dev):
-        pred = _headc(raw_preds, dev)
-        anc = _anchors_dev(anchors, dev)
-        if anc.shape[0] != pred.shape[3]:
-            raise ValueError("anchors must be (num_anchors, 2)")
         out = _DecodeFn.apply(pred, anc, img_size)
     if out.dtype != orig_dtype:
         out = out.to(orig_dtype)
@@ -217,8 +279,8 @@ def ciou_loss(pred_boxes: torch.Tensor, target_boxes: torch.Tensor, eps=CIOU_EPS
     dev = _device()
     orig_dev = pred_boxes.device
     with torch.cuda.device(dev):
-        p = _f32c(pred_boxes, dev)
-        t = _f32c(target_boxes, dev)
+        p = _contig(pred_boxes, dev)
+        t = _contig(target_boxes, dev)
         out = _CiouFn.apply(p, t, eps)
     return out if orig_dev == dev else out.to(orig_dev)
 
@@ -226,14 +288,6 @@ def ciou_loss(pred_boxes: torch.Tensor, target_boxes: torch.Tensor, eps=CIOU_EPS
 # --------------------------------------------------------------------------------------------
 # a-3 / a-4 fused loss
 # --------------------------------------------------------------------------------------------
-LAYOUT_BHWAC, LAYOUT_NCHW = _lib.LAYOUT_BHWAC, _lib.LAYOUT_NCHW
-
-
-def _grid(p: torch.Tensor, layout: int):
-    """(H, W) of a head tensor: (B,H,W,A,5+nc) or, NCHW, (B, A*(5+nc), H, W)."""
-    return (p.shape[2], p.shape[3]) if layout == LAYOUT_NCHW else (p.shape[1], p.shape[2])
-
-
 def heads_from_nchw(raw: torch.Tensor, num_anchors: int = 3) -> torch.Tensor:
     """The reference's own head reshape (train.py:608-609): (B, A*(5+nc), H, W) -> contiguous
     (B, H, W, A, 5+nc).  The *_nchw entry points make this pass unnecessary; tests use it."""
@@ -241,27 +295,25 @@ def heads_from_nchw(raw: torch.Tensor, num_anchors: int = 3) -> torch.Tensor:
     return raw.view(B, num_anchors, C // num_anchors, H, W).permute(0, 3, 4, 1, 2).contiguous()
 
 
-def _fill_loss_desc(preds, tgts, ancs, grads, nc, obj_weights, coef, B_global=None, img_size=LOSS_DECODE_IMG_SIZE,
-                    layout=LAYOUT_BHWAC):
-    S = len(preds)
-    d = LossDesc()
-    d.S = S
-    d.layout = layout
-    d.B = preds[0].shape[0]
-    d.B_global = d.B if B_global is None else int(B_global)
-    d.A = ancs[0].shape[0]
-    d.nc = nc
-    d.img_size = img_size
+class _LossCfg(NamedTuple):
+    """The fused loss's configuration besides its tensors."""
+    nc: int
+    obj_weights: tuple   # objectness weight of each scale
+    group: object        # torch.distributed process group of an image-sharded batch, or None
+    sparse: object       # PackedLabels: targets assigned on the device from label lists; None: dense targets
+    layout: int
+    S: int
+
+
+def _fill_loss_desc(preds, tgts, ancs, grads, cfg, coef, B_global):
+    d = _heads_desc(LossDesc(), preds, ancs, cfg.nc, LOSS_DECODE_IMG_SIZE, cfg.layout)
+    d.B_global = B_global
     d.eps = CIOU_EPS
-    d.dtype = _HEAD_DTYPES[preds[0].dtype]
     d.w_box, d.w_cls = BOX_WEIGHT, CLS_WEIGHT
-    for s in range(S):
-        d.H[s], d.W[s] = _grid(preds[s], layout)
-        d.w_obj[s] = obj_weights[s]
+    for s in range(cfg.S):
+        d.w_obj[s] = cfg.obj_weights[s]
         d.coef_box[s], d.coef_obj[s], d.coef_cls[s] = coef[s]
-        d.pred[s] = preds[s].data_ptr()
-        d.tgt[s] = _ptr(tgts[s])
-        d.anchors[s] = ancs[s].data_ptr()
+        d.tgt[s] = 0 if tgts is None else _ptr(tgts[s])
         d.grad[s] = _ptr(grads[s])
     return d
 
@@ -277,39 +329,33 @@ def loss_forward_backward(preds, tgts, ancs, nc, obj_weights, want_grad, coef=No
     `grad_scale`: bf16 / fp16 heads only, an optional (1,) fp32 device tensor s; the gradients are then those
     of s * total (what `GradScaler.scale(total).backward()` gives), rounded to the head dtype after the scaling.
     """
-    out4, per_scale, grads, emit = _loss_run(preds, tgts, ancs, nc, obj_weights, want_grad, coef, group, equal_shards,
-                                             b_global, reduce_fn, sparse, layout)
+    preds, tgts, ancs = _stage_heads(preds, ancs, nc, layout, tgts if sparse is None else sparse, detach=False,
+                                     dev=preds[0].device if len(preds) else None)
+    cfg = _LossCfg(int(nc), tuple(float(w) for w in obj_weights), group, sparse, layout, len(preds))
+    out4, per_scale, grads, emit = _loss_run(cfg, preds, tgts, ancs, want_grad, coef, equal_shards, b_global, reduce_fn)
     if emit is not None:
-        if grad_scale is None:
-            grad_scale = torch.ones(1, dtype=torch.float32, device=preds[0].device)
-        grads = _loss_emit(emit, grad_scale)
+        grads = emit(torch.ones(1, dtype=torch.float32, device=preds[0].device) if grad_scale is None else grad_scale)
     return out4, per_scale, grads
 
 
-def _loss_run(preds, tgts, ancs, nc, obj_weights, want_grad, coef=None, group=None, equal_shards=True, b_global=None,
-              reduce_fn=None, sparse=None, layout=LAYOUT_BHWAC):
-    """Both stages.  fp32 heads: (out4, per_scale, grads, None), the gradient written by stage 1.  Half heads:
-    (out4, per_scale, [None]*S, emit) where `emit` holds what `_loss_emit` needs to write the gradients later, once
-    the upstream gradient is known (None when no gradient is wanted)."""
+def _loss_run(cfg, preds, tgts, ancs, want, coef=None, equal_shards=True, b_global=None, reduce_fn=None):
+    """Both stages on staged tensors: (out4, per_scale, grads, emit).  fp32 heads: stage 1 writes the gradients into
+    grads and emit is None.  Half heads: grads is [None]*S and, when a gradient is wanted, emit(grad_scale) writes and
+    returns the gradients of grad_scale * total ((1,) fp32, read on the device) from this call's partials; the
+    descriptor it launches with points at preds, tgts and ancs, so they must still be alive then."""
     L = _lib.lib()
-    S = len(preds)
+    S, sparse = cfg.S, cfg.sparse
     dev = preds[0].device
     half = preds[0].dtype != torch.float32
     if coef is None:
-        coef = [(BOX_WEIGHT, obj_weights[s], CLS_WEIGHT) for s in range(S)]
-    grads = [torch.empty_like(p) if w and not half else None for p, w in zip(preds, want_grad)]
-    world = 1
-    explicit = b_global
-    b_global = preds[0].shape[0]
-    if explicit is not None:
-        b_global = int(explicit)
-    elif group is not None:
+        coef = [(BOX_WEIGHT, cfg.obj_weights[s], CLS_WEIGHT) for s in range(S)]
+    grads = [torch.empty_like(p) if w and not half else None for p, w in zip(preds, want)]
+    world, B = 1, preds[0].shape[0]
+    if b_global is None and cfg.group is not None:
         import torch.distributed as dist
-        world = dist.get_world_size(group)
-        b_global = b_global * world if equal_shards else dist_global_batch(preds[0].shape[0], group)
-    if sparse is not None:
-        tgts = [None] * S
-    d = _fill_loss_desc(preds, tgts, ancs, grads, nc, obj_weights, coef, B_global=b_global, layout=layout)
+        world = dist.get_world_size(cfg.group)
+        b_global = B * world if equal_shards else dist_global_batch(B, cfg.group)
+    d = _fill_loss_desc(preds, tgts, ancs, grads, cfg, coef, B if b_global is None else int(b_global))
     if sparse is None:
         ws_bytes = L.yb_loss_workspace_bytes(ctypes.byref(d))
     else:
@@ -323,8 +369,6 @@ def _loss_run(preds, tgts, ancs, nc, obj_weights, want_grad, coef=None, group=No
         _lib.check(L.yb_loss_partials(ctypes.byref(d), partials.data_ptr(), ws.data_ptr(), ws_bytes, st),
                    "yb_loss_partials")
     else:
-        if sparse.labels.shape[0] != preds[0].shape[0]:
-            raise ValueError("labels and predictions disagree on the batch size")
         anc_all = torch.stack(list(ancs)).contiguous()  # (S,A,2)
         _lib.check(L.yb_loss_partials_sparse(ctypes.byref(d), sparse.labels.data_ptr(), sparse.n_gt.data_ptr(),
                                              sparse.letterbox.data_ptr(), anc_all.data_ptr(), sparse.max_gt,
@@ -334,118 +378,80 @@ def _loss_run(preds, tgts, ancs, nc, obj_weights, want_grad, coef=None, group=No
         partials = reduce_fn(partials)          # test hook: emulate the collective on one GPU
     elif world > 1:
         from .dist import allreduce_partials
-        allreduce_partials(partials, group)
+        allreduce_partials(partials, cfg.group)
     _lib.check(L.yb_loss_finalize(ctypes.byref(d), partials.data_ptr(), out4.data_ptr(), per_scale.data_ptr(),
                                   ws.data_ptr(), ws_bytes, st), "yb_loss_finalize")
-    emit = None
-    if half and any(want_grad):
-        # the tensors the emit pass reads (heads, dense targets, anchors) are referenced by d's pointers: keep them
-        emit = (d, partials, ws, -1 if sparse is None else sparse.max_gt, list(want_grad), (preds, tgts, ancs))
+    if not (half and any(want)):
+        return out4, per_scale, grads, None
+
+    def emit(grad_scale):
+        grads = [torch.empty_like(p) if w else None for p, w in zip(preds, want)]
+        for s, g in enumerate(grads):
+            d.grad[s] = _ptr(g)
+        _lib.check(L.yb_loss_grad_emit(ctypes.byref(d), partials.data_ptr(), grad_scale.data_ptr(),
+                                       -1 if sparse is None else sparse.max_gt, ws.data_ptr(), ws.numel(), _stream()),
+                   "yb_loss_grad_emit")
+        return grads
     return out4, per_scale, grads, emit
 
 
-def _loss_emit(emit, grad_scale):
-    """Half heads: the gradients of grad_scale * total (grad_scale: (1,) fp32 on the device, read by the kernels)."""
-    d, partials, ws, max_gt, want, (preds, _, _) = emit
-    grads = [torch.empty_like(p) if w else None for p, w in zip(preds, want)]
-    for s, g in enumerate(grads):
-        d.grad[s] = _ptr(g)
-    _lib.check(_lib.lib().yb_loss_grad_emit(ctypes.byref(d), partials.data_ptr(), grad_scale.data_ptr(), max_gt,
-                                            ws.data_ptr(), ws.numel(), _stream()), "yb_loss_grad_emit")
-    return grads
-
-
 class _YoloLossFn(torch.autograd.Function):
-    """(total, bbox, obj, cls) = f(preds...) with the gradient of `total` produced in the same
-    pass.  Gradients that arrive on bbox/obj/cls as well are honoured by re-running the kernels
-    with the combined coefficients (rare: the reference only calls total.backward())."""
+    """(total, bbox, obj, cls) = f(cfg, preds..., targets..., anchors...), S of each (targets None with label
+    lists), with the gradient of `total` produced in the same pass.  Gradients that arrive on bbox/obj/cls as well are
+    honoured by re-running the kernels with the combined coefficients (rare: the reference only calls
+    total.backward())."""
 
     @staticmethod
-    def forward(ctx, nc, obj_weights, group, S, *tensors):
-        sparse, layout = None, LAYOUT_BHWAC
-        if isinstance(group, tuple):  # (process group, PackedLabels or None, layout)
-            group, sparse, layout = group
-        preds, tgts, ancs = tensors[:S], tensors[S:2 * S], tensors[2 * S:3 * S]
-        want = [ctx.needs_input_grad[4 + s] for s in range(S)]
-        out4, per_scale, grads, emit = _loss_run(preds, tgts, ancs, nc, obj_weights, want, group=group, sparse=sparse,
-                                                 layout=layout)
+    def forward(ctx, cfg, *tensors):
+        S = cfg.S
+        want = list(ctx.needs_input_grad[1:1 + S])
+        out4, _, grads, emit = _loss_run(cfg, tensors[:S], tensors[S:2 * S], tensors[2 * S:], want)
         ctx.set_materialize_grads(False)
-        ctx.sparse, ctx.layout = sparse, layout
-        ctx.cfg = (nc, obj_weights, group, S, want)
-        ctx.fused_grads = grads if emit is None else None
-        ctx.emit = emit   # half heads: the gradient is written in backward, after the upstream gradient is applied
+        ctx.cfg, ctx.want = cfg, want
+        ctx.fused = (grads, emit)   # fp32: stage 1's gradients; half: emit, run once the upstream gradient is known
         ctx.save_for_backward(*tensors)
         return out4[0], out4[1], out4[2], out4[3]
 
     @staticmethod
     def backward(ctx, g_total, g_bbox, g_obj, g_cls):
-        nc, obj_weights, group, S, want = ctx.cfg
-        none = (None,) * 4
+        cfg, want, S = ctx.cfg, ctx.want, ctx.cfg.S
+        fused, ctx.fused = ctx.fused, None
         if not any(want):
-            return none + (None,) * (3 * S)
-        if g_bbox is None and g_obj is None and g_cls is None and ctx.emit is not None:
-            tensors = ctx.saved_tensors
+            grads = [None] * S
+        elif fused is not None and g_bbox is None and g_obj is None and g_cls is None:
+            # the first backward, with a gradient on `total` only (or none)
+            grads, emit = fused
             if g_total is None:
-                grads = [torch.zeros_like(p) if w else None for p, w in zip(tensors[:S], want)]
-            else:   # read on the device: no synchronisation
-                grads = _loss_emit(ctx.emit, g_total.detach().to(torch.float32).reshape(1).contiguous())
-        elif g_bbox is None and g_obj is None and g_cls is None and ctx.fused_grads is not None:
-            grads = ctx.fused_grads
-            if g_total is None:
-                grads = [None if g is None else torch.zeros_like(g) for g in grads]
+                grads = [torch.zeros_like(p) if w else None for p, w in zip(ctx.saved_tensors[:S], want)]
             else:
-                L = _lib.lib()
-                f = g_total.detach().to(torch.float32).reshape(1).contiguous()
-                for g in grads:
-                    if g is not None:
-                        _lib.check(L.yb_scale_inplace(g.data_ptr(), g.numel(), f.data_ptr(), _stream()),
-                                   "yb_scale_inplace")
+                f = g_total.detach().to(torch.float32).reshape(1).contiguous()   # read on the device: no sync
+                if emit is not None:   # half heads: written now, rounded to the head dtype after the scaling
+                    grads = emit(f)
+                else:                  # fp32: stage 1's gradients, scaled in place
+                    for g in grads:
+                        if g is not None:
+                            _lib.check(_lib.lib().yb_scale_inplace(g.data_ptr(), g.numel(), f.data_ptr(), _stream()),
+                                       "yb_scale_inplace")
         else:
             # gradients on bbox/obj/cls as well, or a second backward through the same graph (retain_graph=True:
             # the fused buffers were handed out, and possibly scaled in place, by the first one): recompute
             tensors = ctx.saved_tensors
-            preds, tgts, ancs = tensors[:S], tensors[S:2 * S], tensors[2 * S:3 * S]
             z = lambda g: 0.0 if g is None else float(g)
             gt_, gb_, go_, gc_ = z(g_total), z(g_bbox), z(g_obj), z(g_cls)
-            coef = [(BOX_WEIGHT * gt_ + gb_, obj_weights[s] * gt_ + go_, CLS_WEIGHT * gt_ + gc_) for s in range(S)]
-            _, _, grads = loss_forward_backward(preds, tgts, ancs, nc, obj_weights, want, coef=coef, group=group,
-                                                sparse=ctx.sparse, layout=ctx.layout)
-        ctx.fused_grads = ctx.emit = None
-        return none + tuple(grads) + (None,) * (2 * S)
+            coef = [(BOX_WEIGHT * gt_ + gb_, cfg.obj_weights[s] * gt_ + go_, CLS_WEIGHT * gt_ + gc_) for s in range(S)]
+            _, _, grads = loss_forward_backward(tensors[:S], tensors[S:2 * S], tensors[2 * S:], cfg.nc, cfg.obj_weights,
+                                                want, coef=coef, group=cfg.group, sparse=cfg.sparse, layout=cfg.layout)
+        return (None,) + tuple(grads) + (None,) * (2 * S)
 
 
 def _loss_common(predictions, targets, anchors_list, num_classes, obj_weights, group=None, sparse=None,
                  layout=LAYOUT_BHWAC):
-    S = len(predictions)
-    if not 1 <= S <= MAX_SCALES:
-        raise ValueError(f"1..{MAX_SCALES} scales supported, got {S}")
-    dev = _device()
-    orig_dev = predictions[0].device
+    preds, tgts, ancs = _stage_heads(predictions, anchors_list, num_classes, layout,
+                                     targets if sparse is None else sparse, detach=False)
+    S, dev, orig_dev = len(preds), preds[0].device, predictions[0].device
+    cfg = _LossCfg(int(num_classes), tuple(float(w) for w in obj_weights), group, sparse, layout, S)
     with torch.cuda.device(dev):
-        preds, tgts, ancs = [], [], []
-        for s in range(S):
-            if layout == LAYOUT_NCHW:
-                p, A = predictions[s], len(anchors_list[s])
-                if p.dim() != 4 or p.shape[1] != A * (5 + num_classes):
-                    raise ValueError(f"scale {s}: NCHW head must be (B, {A}*(5+num_classes), H, W), got {tuple(p.shape)}")
-                if sparse is None and tuple(targets[s].shape) != (p.shape[0], p.shape[2], p.shape[3], A, 5 + num_classes):
-                    raise ValueError(f"scale {s}: targets {tuple(targets[s].shape)} do not match the head")
-            else:
-                _check_head(predictions[s], f"predictions[{s}]")
-                if sparse is None and predictions[s].shape != targets[s].shape:
-                    raise ValueError(f"scale {s}: predictions {tuple(predictions[s].shape)} vs targets {tuple(targets[s].shape)}")
-                if predictions[s].shape[4] != 5 + num_classes:
-                    raise ValueError(f"scale {s}: last dim {predictions[s].shape[4]} != 5+num_classes")
-            preds.append(_headc(predictions[s], dev))
-            # sparse targets: a placeholder keeps the autograd signature (preds, targets, anchors) x S
-            tgts.append(_f32c(targets[s].detach(), dev) if sparse is None else preds[-1].detach())
-            ancs.append(_anchors_dev(anchors_list[s], dev))
-        preds = _same_dtype(preds)
-        if sparse is not None:
-            tgts = [p.detach() for p in preds]
-        packed_cfg = group if (sparse is None and layout == LAYOUT_BHWAC) else (group, sparse, layout)
-        outs = _YoloLossFn.apply(int(num_classes), tuple(float(w) for w in obj_weights), packed_cfg, S,
-                                 *preds, *tgts, *ancs)
+        outs = _YoloLossFn.apply(cfg, *preds, *(tgts or [None] * S), *ancs)
     if orig_dev != dev:
         outs = tuple(o.to(orig_dev) for o in outs)
     return outs
@@ -562,17 +568,11 @@ EVAL_DECODE_IMG_SIZE = 640.0  # train.py:993 — eval_epoch decodes with the def
 def eval_counts(predictions, targets, anchors_list, conf_threshold=0.5, iou_threshold=0.5, out=None):
     """The TP/FP/FN loop of eval_epoch (train.py:993-1024) for one batch, all scales, in one kernel.
     Returns an int64 device tensor [TP, FP, FN]; pass `out` to accumulate over batches (no sync)."""
-    dev = _device()
     S = min(len(predictions), len(targets), len(anchors_list))
+    preds, tgts, ancs = _stage_heads(predictions[:S], anchors_list[:S], None, LAYOUT_BHWAC, targets[:S], half=False)
+    dev = preds[0].device
     with torch.cuda.device(dev):
-        preds = [_f32c(p.detach(), dev) for p in predictions[:S]]
-        tgts = [_f32c(t.detach(), dev) for t in targets[:S]]
-        for s in range(S):
-            _check_head(preds[s], f"predictions[{s}]")
-            if preds[s].shape != tgts[s].shape:
-                raise ValueError(f"scale {s}: predictions {tuple(preds[s].shape)} vs targets {tuple(tgts[s].shape)}")
-        ancs = [_anchors_dev(a, dev) for a in anchors_list[:S]]
-        d = _heads_desc(preds, ancs, EVAL_DECODE_IMG_SIZE, preds[0].shape[4] - 5)
+        d = _heads_desc(HeadsDesc(), preds, ancs, preds[0].shape[4] - 5, EVAL_DECODE_IMG_SIZE, LAYOUT_BHWAC)
         if out is None:
             out = torch.zeros(3, dtype=torch.int64, device=dev)
         tptr = (ctypes.c_void_p * MAX_SCALES)(*[t.data_ptr() for t in tgts])
@@ -619,7 +619,7 @@ def compute_anchor_iou(box_wh, anchors) -> torch.Tensor:
     orig_dev = box_wh.device
     single = box_wh.dim() == 1
     with torch.cuda.device(dev):
-        b = _f32c(box_wh.reshape(-1, 2), dev)
+        b = _contig(box_wh.reshape(-1, 2), dev)
         a = _anchors_dev(anchors, dev)
         out = torch.empty(b.shape[0], a.shape[0], dtype=torch.float32, device=dev)
         _lib.check(_lib.lib().yb_anchor_iou(b.data_ptr(), a.data_ptr(), out.data_ptr(), b.shape[0], a.shape[0], _stream()),
@@ -643,27 +643,18 @@ def build_targets(labels: Sequence, anchors_list, grid_sizes: Sequence[int], num
     with torch.cuda.device(dev):
         anc = torch.stack([_anchors_dev(a, dev) for a in anchors_list]).contiguous()  # (S,A,2)
         A = anc.shape[1]
-        rows = [torch.as_tensor(l, dtype=torch.float64).reshape(-1, 5) for l in labels]
-        max_gt = max([r.shape[0] for r in rows], default=0)
-        lab = torch.zeros(B, max(max_gt, 1), 5, dtype=torch.float64)
-        n_gt = torch.zeros(B, dtype=torch.int32)
-        for i, r in enumerate(rows):
-            lab[i, :r.shape[0]] = r
-            n_gt[i] = r.shape[0]
-        if letterbox is None:
-            lb = torch.tensor([[img_size, img_size, 1.0, 0.0, 0.0]] * B, dtype=torch.float64).reshape(B, 5)
-        else:
-            lb = torch.as_tensor(np.asarray(letterbox, dtype=np.float64)).reshape(B, 5)
-        lab_d, n_d, lb_d = lab.to(dev), n_gt.to(dev), lb.to(dev)
+        lab, n_gt, lb = pack_labels_host(labels, img_size, letterbox)
+        max_gt = int(n_gt.max()) if B > 0 else 0   # the kernel's bound: the largest label count, read on the host
+        packed = PackedLabels(lab.to(dev), n_gt.to(dev), lb.to(dev), img_size)
         row = 5 + num_classes
         targets = [torch.empty(B, g, g, A, row, dtype=torch.float32, device=dev) for g in grid_sizes]
-        status = torch.zeros(1, dtype=torch.int32, device=dev)
         tptr = (ctypes.c_void_p * MAX_SCALES)(*[t.data_ptr() for t in targets])
         G = (ctypes.c_int * S)(*[int(g) for g in grid_sizes])
-        _lib.check(_lib.lib().yb_build_targets(lab_d.data_ptr(), n_d.data_ptr(), lb_d.data_ptr(), anc.data_ptr(), tptr,
-                                               B, max_gt, S, G, A, int(num_classes), int(img_size),
-                                               status.data_ptr(), _stream()), "yb_build_targets")
-        if check and int(status.item()) != 0:
+        _lib.check(_lib.lib().yb_build_targets(packed.labels.data_ptr(), packed.n_gt.data_ptr(),
+                                               packed.letterbox.data_ptr(), anc.data_ptr(), tptr, B, max_gt, S, G, A,
+                                               int(num_classes), int(img_size), packed.status.data_ptr(), _stream()),
+                   "yb_build_targets")
+        if check and int(packed.status.item()) != 0:
             raise IndexError("build_targets: a label maps outside the grid or the class range "
                              "(the reference raises IndexError on the same input, train.py:193-205)")
     return targets
@@ -672,34 +663,6 @@ def build_targets(labels: Sequence, anchors_list, grid_sizes: Sequence[int], num
 # --------------------------------------------------------------------------------------------
 # a-6 candidate filter, a-7 NMS
 # --------------------------------------------------------------------------------------------
-def _heads_desc(preds, ancs, img_size, nc, layout=LAYOUT_BHWAC):
-    d = HeadsDesc()
-    d.S, d.B, d.A, d.nc = len(preds), preds[0].shape[0], ancs[0].shape[0], nc
-    d.img_size = float(img_size)
-    d.layout = layout
-    d.dtype = _HEAD_DTYPES[preds[0].dtype]
-    for s, p in enumerate(preds):
-        d.H[s], d.W[s] = _grid(p, layout)
-        d.pred[s] = p.data_ptr()
-        d.anchors[s] = ancs[s].data_ptr()
-    return d
-
-
-def _stage_heads(predictions, anchors_list, num_classes, layout, dev):
-    """The heads and anchors as the filter kernels read them, checked: (preds, ancs, rows per image)."""
-    S = len(predictions)
-    preds = _same_dtype([_headc(p.detach(), dev) for p in predictions])
-    ancs = [_anchors_dev(a, dev) for a in anchors_list[:S]]
-    for s, p in enumerate(preds):
-        if layout == LAYOUT_NCHW:
-            if p.dim() != 4 or p.shape[1] != ancs[s].shape[0] * (5 + int(num_classes)):
-                raise ValueError(f"predictions[{s}]: NCHW head must be (B, A*(5+nc), H, W), got {tuple(p.shape)}")
-        else:
-            _check_head(p, f"predictions[{s}]")
-    rows = sum(_grid(p, layout)[0] * _grid(p, layout)[1] * ancs[s].shape[0] for s, p in enumerate(preds))
-    return preds, ancs, rows
-
-
 def _letterbox_dev(letterbox, B, dev):
     if letterbox is None:
         return None
@@ -716,11 +679,12 @@ def filter_candidates(predictions, anchors_list, img_size, num_classes=1, conf_t
     Returns (boxes (B,cap,4), scores (B,cap), classes (B,cap) int64, counts (B,) int32) on the GPU,
     cap = rows per image.
     """
-    dev = _device()
+    preds, _, ancs = _stage_heads(predictions, anchors_list, num_classes, layout)
+    dev = preds[0].device
     with torch.cuda.device(dev):
-        preds, ancs, cap = _stage_heads(predictions, anchors_list, num_classes, layout, dev)
         B = preds[0].shape[0]
-        d = _heads_desc(preds, ancs, img_size, int(num_classes), layout)
+        d = _heads_desc(HeadsDesc(), preds, ancs, int(num_classes), img_size, layout)
+        cap = d.A * sum(d.H[s] * d.W[s] for s in range(d.S))   # rows per image
         L = _lib.lib()
         ws_bytes = L.yb_filter_workspace_bytes(ctypes.byref(d))
         ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=dev)
@@ -752,12 +716,12 @@ def filter_candidates_multilabel(predictions, anchors_list, img_size, num_classe
     K = int(max_candidates)
     if K < 1:
         raise ValueError(f"max_candidates must be >= 1, got {max_candidates}")
-    dev = _device()
+    preds, _, ancs = _stage_heads(predictions, anchors_list, num_classes, layout)
+    dev = preds[0].device
     with torch.cuda.device(dev):
-        preds, ancs, rows = _stage_heads(predictions, anchors_list, num_classes, layout, dev)
         B = preds[0].shape[0]
-        cap = min(K, rows * int(num_classes))
-        d = _heads_desc(preds, ancs, img_size, int(num_classes), layout)
+        d = _heads_desc(HeadsDesc(), preds, ancs, int(num_classes), img_size, layout)
+        cap = min(K, d.A * sum(d.H[s] * d.W[s] for s in range(d.S)) * int(num_classes))
         L = _lib.lib()
         ws = torch.empty(max(L.yb_filter_multilabel_workspace_bytes(ctypes.byref(d), K), 16), dtype=torch.uint8,
                          device=dev)
@@ -844,8 +808,8 @@ def _nms_single(boxes, scores, idxs, iou_threshold, algo=NMS_GRAPH):
     if n == 0:
         return torch.empty(0, dtype=torch.int64, device=orig_dev)
     with torch.cuda.device(dev):
-        b = _f32c(boxes.detach(), dev).unsqueeze(0)
-        s = _f32c(scores.detach(), dev).unsqueeze(0)
+        b = _contig(boxes.detach(), dev).unsqueeze(0)
+        s = _contig(scores.detach(), dev).unsqueeze(0)
         c = None
         if idxs is not None:
             c = idxs.detach().to(dev, torch.int64).contiguous().unsqueeze(0)
@@ -1548,10 +1512,8 @@ class HotPathGraph:
                 else:
                     self.targets = list(adopt_targets)
             elif targets == "labels":
-                self.labels = PackedLabels(torch.zeros(batch, max(max_gt, 1), 5, dtype=torch.float64, device=dev),
-                                           torch.zeros(batch, dtype=torch.int32, device=dev),
-                                           torch.tensor([[img_size, img_size, 1.0, 0.0, 0.0]] * batch, dtype=torch.float64,
-                                                        device=dev), img_size)
+                lab, n_gt, lb = pack_labels_host([()] * batch, img_size, max_gt=max_gt)
+                self.labels = PackedLabels(lab.to(dev), n_gt.to(dev), lb.to(dev), img_size)
             elif targets == "dense":
                 self.targets = [torch.zeros(batch, g, g, A, row, device=dev) for g in grids]
             else:
