@@ -100,6 +100,94 @@ def test_new_entry_points_validate_arguments(yb):
     assert lib.yb_eval_counts(ctypes.byref(h), None, 0.5, 0.5, None, None) != 0
 
 
+HEAD_CHECK_SCRIPT = r'''
+import ctypes, json, sys
+sys.path.insert(0, sys.argv[1])
+import torch
+import yolo_from_scratch_b200 as yb
+assert torch.cuda.device_count() == 0, "the calls below pass stand-in device addresses"
+L = yb._lib
+lib = L.lib()
+P = 1 << 20                                   # a 16-byte aligned stand-in address; no device is visible
+CASES = {
+    "valid": {}, "S=0": {"S": 0}, "S=5": {"S": 5}, "A=0": {"A": 0}, "A=9": {"A": 9}, "H=0": {"H": 0},
+    "layout=7": {"layout": 7}, "dtype=7": {"dtype": 7}, "layout=7,B=0": {"layout": 7, "B": 0},
+    "dtype=7,B=0": {"dtype": 7, "B": 0}, "2^32 elements": {"H": 1 << 14, "W": 1 << 14},
+    "null pred": {"pred": 0}, "misaligned pred": {"pred": P + 4},
+}
+DECODE_ONLY_S1 = ("S=0", "S=5", "layout=7", "layout=7,B=0")   # decode takes one scale and no layout
+
+def desc(cls, case, dtype):
+    d = cls()
+    d.S, d.B, d.A, d.nc, d.img_size, d.layout, d.dtype = 3, 2, 3, 2, 64.0, 0, dtype
+    for s, g in enumerate((8, 4, 2)):
+        d.H[s] = d.W[s] = g
+        d.pred[s], d.anchors[s] = P * (s + 1), P * (s + 5)
+    if cls is L.LossDesc:
+        d.B_global = 2
+        for s in range(3):
+            d.tgt[s], d.grad[s] = P * (s + 9), P * (s + 13)
+    for k, v in CASES[case].items():
+        if k in ("H", "W"):
+            getattr(d, k)[0] = v
+        elif k == "pred":
+            d.pred[0] = v
+        else:
+            setattr(d, k, v)
+    return d
+
+def decode(bwd):
+    def call(case):
+        d = desc(L.HeadsDesc, case, 0)
+        args = (d.pred[0], d.anchors[0]) + ((P,) if bwd else ()) + (P, d.B, d.H[0], d.W[0], d.A, d.nc, 64.0, d.dtype, None)
+        return (lib.yb_decode_bwd_t if bwd else lib.yb_decode_fwd_t)(*args)
+    return call
+
+big = 1 << 40
+ENTRIES = {
+    "decode_fwd": ("decode", decode(False)),
+    "decode_bwd": ("decode", decode(True)),
+    "loss_partials": ("loss", lambda c: lib.yb_loss_partials(ctypes.byref(desc(L.LossDesc, c, 0)), P, P, big, None)),
+    "loss_partials_sparse": ("loss(sparse)", lambda c: lib.yb_loss_partials_sparse(
+        ctypes.byref(desc(L.LossDesc, c, 0)), P, P, P, P, 4, 64, P, P, P, big, None)),
+    "loss_grad_emit": ("loss_grad_emit", lambda c: lib.yb_loss_grad_emit(
+        ctypes.byref(desc(L.LossDesc, c, 1)), P, P, -1, P, big, None)),
+    "filter_compact": ("filter", lambda c: lib.yb_filter_compact(
+        ctypes.byref(desc(L.HeadsDesc, c, 0)), 0.5, None, P, P, P, P, 100, P, big, None)),
+    "filter_multilabel": ("filter_multilabel", lambda c: lib.yb_filter_multilabel(
+        ctypes.byref(desc(L.HeadsDesc, c, 0)), 0.5, None, 100, P, P, P, P, None, 1 << 20, P, big, None)),
+    "eval_counts": ("eval_counts", lambda c: lib.yb_eval_counts(
+        ctypes.byref(desc(L.HeadsDesc, c, 0)), (ctypes.c_void_p * 4)(P, P, P, P), 0.5, 0.5, P, None)),
+}
+out = []
+for name, (who, call) in ENTRIES.items():
+    for case in CASES:
+        if name.startswith("decode") and case in DECODE_ONLY_S1:
+            continue
+        rc = call(case)
+        out.append([name, who, case, rc, lib.yb_last_error().decode() if rc else ""])
+print(json.dumps(out))
+'''
+
+
+def test_every_head_entry_point_rejects_the_same_malformed_descriptors(yb):
+    """Every entry point that reads head tensors checks its descriptor the same way: a table of malformed
+    descriptors comes back as YB_EINVAL with a message that names the entry point, at B = 0 too.  The calls run
+    in a process that sees no GPU, so that a missing check fails at the first CUDA call instead of launching; the
+    well-formed descriptor gets past the checks and fails there with a CUDA error."""
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    res = subprocess.run([sys.executable, "-c", HEAD_CHECK_SCRIPT, ROOT], env=env, capture_output=True, text=True,
+                         timeout=300)
+    assert res.returncode == 0, res.stderr
+    rows = __import__("json").loads(res.stdout.strip().splitlines()[-1])
+    assert len({r[0] for r in rows}) == 8 and len(rows) == 8 * 13 - 2 * 4
+    for name, who, case, rc, msg in rows:
+        if case == "valid":
+            assert rc > 0, (name, rc, msg)   # past the argument checks: a CUDA error, not YB_EINVAL
+        else:
+            assert rc == -1 and msg.startswith(who + ":"), (name, case, rc, msg)
+
+
 def fake_train_module():
     """A stand-in with the reference's hot-path names; internal callers resolve them through the
     module globals exactly like train.py does."""

@@ -9,46 +9,49 @@
 
 namespace yb {
 
-struct DecodeArgs {
-    const void* pred;       // element type T of the kernel (float, bf16, fp16)
-    const float* anchors;   // (A,2) device
+struct DecodeArgs : HeadScale {   // one scale: pred, anchors, geometry
     const void* grad_out;   // bwd only
     void* out;              // fwd: decoded; bwd: grad_in
     uint32_t n_vec;         // number of whole 16-byte vectors
     uint32_t n_elem;        // total elements
     uint32_t row;           // 5+nc
-    int A, W, H;
-    FastDiv d_row, d_A, d_W, d_H;
-    DecodeConsts k;
+    float inv_img;
+    FastDiv d_row;
 };
 
+// The four box channels of row r from their sigmoids s[0..3]: forward values, or the vector-Jacobian product with
+// the upstream gradients gr[0..3].
+template <bool BWD>
+__device__ __forceinline__ void decode_row4(const DecodeArgs& a, uint32_t r, const float* s, const float* gr, float* orow) {
+    uint32_t b, gy, gx, an;
+    head_row_coords(a, r, b, gy, gx, an);
+    const float aw = __ldg(a.anchors + an * 2), ah = __ldg(a.anchors + an * 2 + 1);
+    if (!BWD) {
+        orow[0] = box_xy(s[0], (float)gx, a.inv_w);
+        orow[1] = box_xy(s[1], (float)gy, a.inv_h);
+        orow[2] = box_wh(s[2], aw, a.inv_img);
+        orow[3] = box_wh(s[3], ah, a.inv_img);
+    } else {
+        orow[0] = box_xy_vjp(s[0], gr[0], a.inv_w);
+        orow[1] = box_xy_vjp(s[1], gr[1], a.inv_h);
+        orow[2] = box_wh_vjp(s[2], gr[2], aw, a.inv_img);
+        orow[3] = box_wh_vjp(s[3], gr[3], ah, a.inv_img);
+    }
+}
+
+// channel c of row r from its logit x (and upstream gradient g)
 template <bool BWD>
 __device__ __forceinline__ float decode_elem(const DecodeArgs& a, uint32_t r, uint32_t c, float x, float g) {
-    // r = flat row index ((b*H + gy)*W + gx)*A + an ; c = channel in row
     if (c >= 4) return BWD ? g : x;
-    uint32_t cell, an, gy_b, gx, gy, bi;
-    a.d_A.divmod(r, cell, an);
-    a.d_W.divmod(cell, gy_b, gx);
-    a.d_H.divmod(gy_b, bi, gy);
-    if (!BWD) {
-        if (c == 0) return decode_xy(x, (float)gx, a.k.inv_w);
-        if (c == 1) return decode_xy(x, (float)gy, a.k.inv_h);
-        float anc = __ldg(a.anchors + an * 2 + (c - 2));
-        return decode_wh(x, anc, a.k.inv_img);
-    } else {
-        // autograd order of train.py:758-759,773-774 (see DESIGN.md "decode backward")
-        float s = sigmoidf_ref(x);
-        float ds = (1.0f - s) * s;  // sigmoid_backward: grad * ((1 - y) * y)
-        if (c < 2) {
-            float inv = (c == 0) ? a.k.inv_w : a.k.inv_h;
-            return ((g * inv) * 2.0f) * ds;
-        }
-        float anc = __ldg(a.anchors + an * 2 + (c - 2));
-        float u = 2.0f * s;
-        float gp = g * (anc * a.k.inv_img);  // mul backward
-        float gu = gp * (2.0f * u);          // pow(u,2) backward
-        return (gu * 2.0f) * ds;             // (2*s) backward, then sigmoid backward
+    uint32_t b, gy, gx, an;
+    head_row_coords(a, r, b, gy, gx, an);
+    const float s = sigmoidf_ref(x);
+    if (c < 2) {
+        const float inv = c == 0 ? a.inv_w : a.inv_h;
+        return BWD ? box_xy_vjp(s, g, inv) : box_xy(s, (float)(c == 0 ? gx : gy), inv);
     }
+    const float anc = __ldg(a.anchors + an * 2 + (c - 2));
+    return BWD ? box_wh_vjp(s, g, anc, a.inv_img) : box_wh(s, anc, a.inv_img);
 }
 
 // element e of the flat head tensor, widened, decoded and rounded back (tails of the vector walks)
@@ -115,38 +118,14 @@ __global__ void __launch_bounds__(256) decode_rows_kernel(const DecodeArgs a) {
         }
 #pragma unroll
         for (int k = 0; k < R; ++k) {
-            const uint32_t r = gidx * R + k;
-            uint32_t cell, an, gy_b, gx, gy, bi;
-            a.d_A.divmod(r, cell, an);
-            a.d_W.divmod(cell, gy_b, gx);
-            a.d_H.divmod(gy_b, bi, gy);
-            const float aw = __ldg(a.anchors + an * 2), ah = __ldg(a.anchors + an * 2 + 1);
             const float* xr = x + k * ROW;
-            float* orow = o + k * ROW;
-            if (!BWD) {
-                orow[0] = decode_xy(xr[0], (float)gx, a.k.inv_w);
-                orow[1] = decode_xy(xr[1], (float)gy, a.k.inv_h);
-                orow[2] = decode_wh(xr[2], aw, a.k.inv_img);
-                orow[3] = decode_wh(xr[3], ah, a.k.inv_img);
+            const float* gr = g + k * ROW;
+            float sg[4];
 #pragma unroll
-                for (int c = 4; c < ROW; ++c) orow[c] = xr[c];
-            } else {
-                const float* gr = g + k * ROW;
+            for (int c = 0; c < 4; ++c) sg[c] = sigmoidf_ref(xr[c]);
+            decode_row4<BWD>(a, gidx * R + k, sg, gr, o + k * ROW);
 #pragma unroll
-                for (int c = 0; c < 4; ++c) {   // autograd order of train.py:758-759,773-774, as in decode_elem
-                    const float s = sigmoidf_ref(xr[c]);
-                    const float ds = (1.0f - s) * s;
-                    if (c < 2) {
-                        orow[c] = ((gr[c] * (c == 0 ? a.k.inv_w : a.k.inv_h)) * 2.0f) * ds;
-                    } else {
-                        const float u = 2.0f * s;
-                        const float gp = gr[c] * ((c == 2 ? aw : ah) * a.k.inv_img);
-                        orow[c] = ((gp * (2.0f * u)) * 2.0f) * ds;
-                    }
-                }
-#pragma unroll
-                for (int c = 4; c < ROW; ++c) orow[c] = gr[c];
-            }
+            for (int c = 4; c < ROW; ++c) o[k * ROW + c] = BWD ? gr[c] : xr[c];
         }
 #pragma unroll
         for (int v = 0; v < NV; ++v) __stcs(out4 + (size_t)gidx * NV + v, pack16<T>(o + V * v));
@@ -154,35 +133,6 @@ __global__ void __launch_bounds__(256) decode_rows_kernel(const DecodeArgs a) {
     // the last (< R) rows
     const uint32_t e0 = n_groups * (uint32_t)(ROW * R);
     if (blockIdx.x == 0 && e0 + threadIdx.x < a.n_elem) decode_one<T, BWD>(a, e0 + threadIdx.x);
-}
-
-// The four box channels of row r from their sigmoids s[0..3] (sigmoid_ref_batch): forward values, or the
-// vector-Jacobian product with the upstream gradients gr[0..3] — the same expressions as decode_elem.
-template <bool BWD>
-__device__ __forceinline__ void decode_row4(const DecodeArgs& a, uint32_t r, const float* s, const float* gr, float* orow) {
-    uint32_t cell, an, gy_b, gx, gy, bi;
-    a.d_A.divmod(r, cell, an);
-    a.d_W.divmod(cell, gy_b, gx);
-    a.d_H.divmod(gy_b, bi, gy);
-    const float aw = __ldg(a.anchors + an * 2), ah = __ldg(a.anchors + an * 2 + 1);
-    if (!BWD) {
-        orow[0] = decode_xy_s(s[0], (float)gx, a.k.inv_w);
-        orow[1] = decode_xy_s(s[1], (float)gy, a.k.inv_h);
-        orow[2] = decode_wh_s(s[2], aw, a.k.inv_img);
-        orow[3] = decode_wh_s(s[3], ah, a.k.inv_img);
-    } else {
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {   // autograd order of train.py:758-759,773-774, as in decode_elem
-            const float ds = (1.0f - s[c]) * s[c];
-            if (c < 2) {
-                orow[c] = ((gr[c] * (c == 0 ? a.k.inv_w : a.k.inv_h)) * 2.0f) * ds;
-            } else {
-                const float u = 2.0f * s[c];
-                const float gp = gr[c] * ((c == 2 ? aw : ah) * a.k.inv_img);
-                orow[c] = ((gp * (2.0f * u)) * 2.0f) * ds;
-            }
-        }
-    }
 }
 
 // Long rows (nc >= 4, e.g. 85 floats): in the flat walk a quarter of the lanes of every warp holds one of a row's
@@ -280,21 +230,22 @@ static int decode_launch_t(bool bwd, const DecodeArgs& a, unsigned long long n, 
 static int decode_launch(bool bwd, const void* pred, const float* anchors, const void* grad_out,
                          void* out, int B, int H, int W, int A, int nc, float img_size, int dtype,
                          void* stream) {
-    YB_CHECK_ARG(pred && anchors && out && (!bwd || grad_out), "decode: null pointer");
-    YB_CHECK_ARG(B >= 0 && H > 0 && W > 0 && A > 0 && A <= YB_MAX_ANCHORS && nc >= 0,
-                 "decode: bad shape B=%d H=%d W=%d A=%d nc=%d", B, H, W, A, nc);
-    YB_CHECK_ARG(aligned16(pred) && aligned16(out) && (!bwd || aligned16(grad_out)),
-                 "decode: tensors must be 16-byte aligned");
-    unsigned long long n = (unsigned long long)B * H * W * A * (5 + nc);
-    YB_CHECK_ARG(n < (1ull << 32), "decode: tensor too large (%llu elements)", n);
-    YB_CHECK_ARG(dtype == YB_DTYPE_F32 || dtype == YB_DTYPE_BF16 || dtype == YB_DTYPE_F16, "decode: unknown dtype %d", dtype);
-    if (n == 0) return 0;
+    yb_heads_desc d = {};
+    d.S = 1; d.B = B; d.A = A; d.nc = nc; d.H[0] = H; d.W[0] = W; d.img_size = img_size;
+    d.pred[0] = reinterpret_cast<const float*>(pred); d.anchors[0] = anchors;
+    d.layout = YB_LAYOUT_BHWAC; d.dtype = dtype;
+    int rc = heads_check(d, "decode", 0, false, true, true);
+    if (rc) return rc;
+    if (B == 0) return 0;
+    YB_CHECK_ARG(out && (!bwd || grad_out), "decode: null %s", out ? "grad_out" : "out");
+    YB_CHECK_ARG(aligned16(out) && (!bwd || aligned16(grad_out)), "decode: out and grad_out must be 16-byte aligned");
     DecodeArgs a;
-    a.pred = pred; a.anchors = anchors; a.grad_out = grad_out; a.out = out;
+    head_scale_fill(a, d, 0);
+    const unsigned long long n = (unsigned long long)a.img_rows * B * (5 + nc);
+    a.grad_out = grad_out; a.out = out;
     a.n_elem = (uint32_t)n; a.n_vec = (uint32_t)(n * dtype_size(dtype) / 16); a.row = 5 + nc;
-    a.A = A; a.W = W; a.H = H;
-    a.d_row = FastDiv(5 + nc); a.d_A = FastDiv(A); a.d_W = FastDiv(W); a.d_H = FastDiv(H);
-    a.k.inv_w = 1.0f / (float)W; a.k.inv_h = 1.0f / (float)H; a.k.inv_img = 1.0f / img_size;
+    a.d_row = FastDiv(5 + nc);
+    a.inv_img = 1.0f / img_size;
     cudaStream_t st = (cudaStream_t)stream;
     YB_DISPATCH_DTYPE(dtype, T, return decode_launch_t<T>(bwd, a, n, st));
     return 0;

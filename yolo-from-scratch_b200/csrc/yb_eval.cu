@@ -10,14 +10,9 @@
 
 namespace yb {
 
-struct EvalScale {
-    const float* pred;
+struct EvalScale : HeadScale {   // pred: fp32
     const float* tgt;
-    const float* anchors;
-    uint32_t rows;  // B*H*W*A
     uint32_t row_begin;
-    float inv_w, inv_h;
-    FastDiv d_A, d_W, d_H;
 };
 
 struct EvalArgs {
@@ -66,7 +61,7 @@ __global__ void __launch_bounds__(kEvalThreads) eval_count_kernel(const EvalArgs
                 for (int k = 1; k < YB_MAX_SCALES; ++k)
                     if (k < a.S && g >= a.sc[k].row_begin) s = k;
                 const uint32_t r = g - a.sc[s].row_begin;
-                px[u] = a.sc[s].pred + (size_t)r * a.row;
+                px[u] = reinterpret_cast<const float*>(a.sc[s].pred) + (size_t)r * a.row;
                 pt[u] = a.sc[s].tgt + (size_t)r * a.row;
                 xo[u] = __ldg(px[u] + 4);
                 to[u] = __ldg(pt[u] + 4);
@@ -81,13 +76,13 @@ __global__ void __launch_bounds__(kEvalThreads) eval_count_kernel(const EvalArgs
             const bool t_on = (double)to[u] > a.conf;
             if (p_on && t_on) {
                 const EvalScale& L = a.sc[sidx[u]];
-                uint32_t cell, an, gy_b, gx, gy, bi;
-                L.d_A.divmod(rr[u], cell, an);
-                L.d_W.divmod(cell, gy_b, gx);
-                L.d_H.divmod(gy_b, bi, gy);
+                uint32_t b, gy, gx, an;
+                head_row_coords(L, rr[u], b, gy, gx, an);
                 const float aw = __ldg(L.anchors + an * 2), ah = __ldg(L.anchors + an * 2 + 1);
-                const float pb[4] = {decode_xy(__ldg(px[u]), (float)gx, L.inv_w), decode_xy(__ldg(px[u] + 1), (float)gy, L.inv_h),
-                                     decode_wh(__ldg(px[u] + 2), aw, a.inv_img), decode_wh(__ldg(px[u] + 3), ah, a.inv_img)};
+                const float pb[4] = {box_xy(sigmoidf_ref(__ldg(px[u])), (float)gx, L.inv_w),
+                                     box_xy(sigmoidf_ref(__ldg(px[u] + 1)), (float)gy, L.inv_h),
+                                     box_wh(sigmoidf_ref(__ldg(px[u] + 2)), aw, a.inv_img),
+                                     box_wh(sigmoidf_ref(__ldg(px[u] + 3)), ah, a.inv_img)};
                 const float tb[4] = {__ldg(pt[u]), __ldg(pt[u] + 1), __ldg(pt[u] + 2), __ldg(pt[u] + 3)};
                 if (box_iou_xywh(pb, tb) > a.iou_thr) ++tp;  // :1012 fp32 tensor > python scalar
                 else ++fp;
@@ -116,9 +111,8 @@ extern "C" int yb_eval_counts(const yb_heads_desc* d, const float* const* target
                               double iou_threshold, long long* counts3, void* stream) {
     using namespace yb;
     YB_CHECK_ARG(d && targets_host && counts3, "eval_counts: null argument");
-    YB_CHECK_ARG(d->S >= 1 && d->S <= YB_MAX_SCALES && d->B >= 0 && d->A > 0 && d->A <= YB_MAX_ANCHORS && d->nc >= 0,
-                 "eval_counts: bad S/B/A/nc");
-    YB_CHECK_ARG(d->layout == YB_LAYOUT_BHWAC, "eval_counts: only the reference layout (B,H,W,A,5+nc) is supported");
+    int rc = heads_check(*d, "eval_counts", 0, false, false, true);
+    if (rc) return rc;
     if (d->B == 0) return 0;
     EvalArgs a;
     a.S = d->S; a.A = d->A; a.row = 5 + d->nc;
@@ -127,19 +121,15 @@ extern "C" int yb_eval_counts(const yb_heads_desc* d, const float* const* target
     a.conf = conf_threshold;
     a.counts = reinterpret_cast<unsigned long long*>(counts3);
     unsigned long long total = 0;
-    YB_CHECK_ARG(d->dtype == YB_DTYPE_F32, "eval_counts: heads must be fp32");
     for (int s = 0; s < d->S; ++s) {
-        YB_CHECK_ARG(d->H[s] > 0 && d->W[s] > 0 && d->pred[s] && targets_host[s] && d->anchors[s],
-                     "eval_counts: bad scale %d", s);
-        unsigned long long n = (unsigned long long)d->B * d->H[s] * d->W[s] * d->A;
-        YB_CHECK_ARG(n * (5 + d->nc) < (1ull << 32), "eval_counts: scale %d too large", s);
+        YB_CHECK_ARG(targets_host[s], "eval_counts: null targets at scale %d", s);
         EvalScale& L = a.sc[s];
-        L.pred = d->pred[s]; L.tgt = targets_host[s]; L.anchors = d->anchors[s];
-        L.rows = (uint32_t)n; L.row_begin = (uint32_t)total;
-        L.inv_w = 1.0f / (float)d->W[s]; L.inv_h = 1.0f / (float)d->H[s];
-        L.d_A = FastDiv(d->A); L.d_W = FastDiv(d->W[s]); L.d_H = FastDiv(d->H[s]);
-        total += n;
+        head_scale_fill(L, *d, s);
+        L.tgt = targets_host[s];
+        L.row_begin = (uint32_t)total;
+        total += (unsigned long long)L.img_rows * d->B;
     }
+    // the ILP-4 walk's row index g0 + 3 * stride must not wrap
     YB_CHECK_ARG(total < (1ull << 32) - (1ull << 24), "eval_counts: too many rows");
     a.total_rows = (uint32_t)total;
     const unsigned long long per_cta = (unsigned long long)kEvalThreads * kEvalIlp;

@@ -179,6 +179,8 @@ __device__ __forceinline__ int lb_exclusive(const unsigned long long* st, int g,
 template <typename Load>
 __device__ __forceinline__ void filter_emit_row(const FilterArgs& a, const FilterScale& L, uint32_t r, size_t o, Load X,
                                                 float inv_s, float pt, float pl) {
+    // r counts the rows of one image, so the split needs no division by H; head_row_coords' third division costs
+    // filter_onepass_kernel<true, *> 8 registers (64 -> 72, ptxas -v)
     uint32_t cell, an, gy, gx;
     L.d_A.divmod(r, cell, an);
     L.d_W.divmod(cell, gy, gx);
@@ -246,11 +248,11 @@ __global__ void __launch_bounds__(kFTile) filter_onepass_kernel(const FilterArgs
     const int s = group_scale(a, group);
     const FilterScale& L = a.sc[s];
     const uint32_t tile0 = (group - L.group_begin) * a.G;  // within the scale
-    const uint32_t ntiles = (L.rows + kFTile - 1) / kFTile;
+    const uint32_t ntiles = (L.img_rows + kFTile - 1) / kFTile;
     const int G = (int)min((uint32_t)a.G, ntiles - tile0);  // tiles of this group
     const uint32_t row0 = tile0 * kFTile;
-    const uint32_t nrows = min((uint32_t)(G * kFTile), L.rows - row0);
-    const size_t base = ((size_t)b * L.rows + row0) * a.row;  // element offset of the group
+    const uint32_t nrows = min((uint32_t)(G * kFTile), L.img_rows - row0);
+    const size_t base = ((size_t)b * L.img_rows + row0) * a.row;  // element offset of the group
     const T* g = reinterpret_cast<const T*>(L.pred) + base;
     unsigned long long* st = a.lb_state + (size_t)b * a.groups_per_img;
     const uint32_t tile_fl = (uint32_t)kFTile * a.row;        // elements of a full tile
@@ -429,11 +431,11 @@ __global__ void __launch_bounds__(kFTile) filter_count_nchw_kernel(const FilterA
     const FilterScale& L = a.sc[s];
     const uint32_t cell = (tile - n.tile_begin[s]) * kFTile + threadIdx.x;
     int cnt = 0;
-    if (cell < L.hw) {
+    if (cell < L.HW) {
         float x[YB_MAX_ANCHORS];
 #pragma unroll
         for (int an = 0; an < YB_MAX_ANCHORS; ++an)
-            if (an < a.A) x[an] = ldg_f(reinterpret_cast<const T*>(L.pred) + ((size_t)(b * (uint32_t)a.A + an) * a.row + 4) * L.hw + cell);
+            if (an < a.A) x[an] = ldg_f(reinterpret_cast<const T*>(L.pred) + ((size_t)(b * (uint32_t)a.A + an) * a.row + 4) * L.HW + cell);
 #pragma unroll
         for (int an = 0; an < YB_MAX_ANCHORS; ++an)
             if (an < a.A) cnt += sigmoidf_ref(x[an]) > a.conf ? 1 : 0;  // :1157,:1166-1167 objectness only
@@ -474,9 +476,9 @@ __global__ void __launch_bounds__(kFTile) filter_emit_nchw_kernel(const FilterAr
     const int s = nchw_tile_scale(a, n, tile);
     const FilterScale& L = a.sc[s];
     const uint32_t cell = (tile - n.tile_begin[s]) * kFTile + threadIdx.x;
-    const bool valid = cell < L.hw;
-    const T* plane0 = reinterpret_cast<const T*>(L.pred) + (size_t)b * a.A * a.row * L.hw + (valid ? cell : 0u);  // channel 0, anchor 0
-    const size_t hw = L.hw;
+    const bool valid = cell < L.HW;
+    const T* plane0 = reinterpret_cast<const T*>(L.pred) + (size_t)b * a.A * a.row * L.HW + (valid ? cell : 0u);  // channel 0, anchor 0
+    const size_t hw = L.HW;
 
     // phase A: objectness of this cell for every anchor
     float so[YB_MAX_ANCHORS];
@@ -525,10 +527,14 @@ __global__ void __launch_bounds__(kFTile) filter_emit_nchw_kernel(const FilterAr
         float cprob;
         int cid;
         class_max(a.nc, [&](int c) { return ldg_f(x + (size_t)(5 + c) * hw); }, cprob, cid);
-        const float bx = decode_xy(x0, (float)gx, L.inv_w);
-        const float by = decode_xy(x1r, (float)gy, L.inv_h);
-        const float bw = decode_wh(x2r, aw, a.inv_img);
-        const float bh = decode_wh(x3r, ah, a.inv_img);
+        // each channel's sigmoid inside a call of its own: with the sigmoids passed in (filter_box) ptxas allocates 72
+        // registers instead of 64, 7 CTAs per SM instead of 8 (nc=80, B=64, 640^2 on a B200 at a 1000 W power limit: 154 -> 172 us)
+        auto xy = [](float t, float g, float inv) { return box_xy(sigmoidf_ref(t), g, inv); };
+        auto wh = [](float t, float anc, float inv_img) { return box_wh(sigmoidf_ref(t), anc, inv_img); };
+        const float bx = xy(x0, (float)gx, L.inv_w);
+        const float by = xy(x1r, (float)gy, L.inv_h);
+        const float bw = wh(x2r, aw, a.inv_img);
+        const float bh = wh(x3r, ah, a.inv_img);
         const float xc = bx * a.img, yc = by * a.img, wp = bw * a.img, hp = bh * a.img;
         float x1 = xc - wp * 0.5f, y1 = yc - hp * 0.5f, x2 = xc + wp * 0.5f, y2 = yc + hp * 0.5f;
         if (a.letterbox) {
@@ -543,10 +549,10 @@ __global__ void __launch_bounds__(kFTile) filter_emit_nchw_kernel(const FilterAr
     }
 }
 
-static int filter_fill(const yb_heads_desc* d, FilterArgs& a) {
+static int filter_fill(const yb_heads_desc* d, bool need_ptrs, FilterArgs& a) {
     // tiles per CTA: kFMaxGroup in the reference layout (short rows stage the whole group, long rows stream tile by
     // tile); NCHW keeps its own cell tiling
-    return yb::filter_fill(d, a, kFMaxGroup, kFTile);   // (4 or 2 tiles per group measured no faster: 28 / 28 / 38 us on configs[1])
+    return yb::filter_fill(d, "filter", need_ptrs, a, kFMaxGroup, kFTile);   // (4 or 2 tiles per group measured no faster: 28 / 28 / 38 us on configs[1])
 }
 
 }  // namespace yb
@@ -593,7 +599,7 @@ static int filter_launch(const yb_heads_desc* d, FilterArgs& a, void* ws, cudaSt
 
 extern "C" size_t yb_filter_workspace_bytes(const yb_heads_desc* d) {
     yb::FilterArgs a;
-    if (yb::filter_fill(d, a)) return 0;
+    if (yb::filter_fill(d, false, a)) return 0;
     // NCHW: per-tile counts (4 B); reference layout: look-back state (8 B per group) + one ticket per image
     const size_t nchw = (size_t)d->B * a.tiles_per_img * sizeof(int);
     const size_t lb = (size_t)d->B * a.groups_per_img * sizeof(unsigned long long) + ((size_t)d->B + 2) * sizeof(unsigned int);
@@ -605,13 +611,11 @@ extern "C" int yb_filter_compact(const yb_heads_desc* d, float conf_thres, const
                                  void* ws, size_t ws_bytes, void* stream) {
     using namespace yb;
     FilterArgs a;
-    int rc = filter_fill(d, a);
+    int rc = filter_fill(d, true, a);
     if (rc) return rc;
     if (d->B == 0) return 0;
     YB_CHECK_ARG(boxes && scores && classes && counts && ws && cap > 0, "filter: null output");
     YB_CHECK_ARG(aligned16(boxes) && (reinterpret_cast<uintptr_t>(ws) & 7u) == 0, "filter: boxes must be 16-byte, the workspace 8-byte aligned");
-    for (int s = 0; s < d->S; ++s)
-        YB_CHECK_ARG(d->pred[s] && d->anchors[s] && aligned16(d->pred[s]), "filter: bad tensor at scale %d", s);
     if (ws_bytes < yb_filter_workspace_bytes(d)) {
         set_error("filter: workspace too small");
         return YB_EWORKSPACE;

@@ -39,6 +39,20 @@ struct MlArgs {
     int* totals;         // (B) or null
 };
 
+// Offset of channel 0 of row r of image b and the distance between its channels.  head_row_offset addresses the same
+// element, but its NCHW split also lets r run past image b; in these kernels that costs the multi-label filter 1-2%
+// (tools/bench_multilabel.py, nc = 80, B = 64, 640^2 on a B200 at a 1000 W power limit: 1.278 -> 1.302 ms).
+__device__ __forceinline__ size_t ml_row(const FilterArgs& a, const FilterScale& L, uint32_t b, uint32_t r, uint32_t& cstride) {
+    if (!a.nchw) {
+        cstride = 1u;
+        return ((size_t)b * L.img_rows + r) * a.row;
+    }
+    uint32_t cell, an;
+    L.d_A.divmod(r, cell, an);
+    cstride = L.HW;
+    return ((size_t)(b * (uint32_t)a.A + an) * a.row) * L.HW + cell;
+}
+
 // Calls f(an, c, key) for every candidate of cell `cell` (scale L, image b) in candidate order, anchors then classes
 // ascending; key = the bits of score = fp32(sigmoid(obj) * sigmoid(cls_c)) > conf.  The objectness test is the
 // single-label filter's sigmoid(obj) > conf; a NaN logit fails every test.
@@ -46,7 +60,7 @@ template <typename T, typename F>
 __device__ __forceinline__ void ml_cell(const FilterArgs& a, const FilterScale& L, uint32_t b, uint32_t cell, F f) {
     for (int an = 0; an < a.A; ++an) {
         uint32_t cs;
-        const T* x = reinterpret_cast<const T*>(L.pred) + frow_base(a, L, b, cell * (uint32_t)a.A + an, cs);
+        const T* x = reinterpret_cast<const T*>(L.pred) + ml_row(a, L, b, cell * (uint32_t)a.A + an, cs);
         const float so = sigmoidf_ref(ldg_f(x + (size_t)4 * cs));
         if (!(so > a.conf)) continue;
         const T* xc = x + (size_t)5 * cs;
@@ -123,7 +137,7 @@ __global__ void __launch_bounds__(kMlTile) filter_ml_count_kernel(const FilterAr
     uint32_t cell;
     const FilterScale L = ml_tile(a, m.n, tile, cell);
     int cnt = 0;
-    if (cell < L.hw)
+    if (cell < L.HW)
         ml_cell<T>(a, L, b, cell, [&](int, int, uint32_t key) {
             ++cnt;
             atomicAdd(&s_hist[key >> 20], 1u);
@@ -192,7 +206,7 @@ __global__ void __launch_bounds__(kMlTile) filter_ml_refine_kernel(const FilterA
         __syncthreads();
         const uint32_t prefix = (uint32_t)st[ML_PREFIX];
         const int shift = level == 2 ? 20 : 10;   // keys of the bin: key >> shift == prefix; digit: the next 10 bits
-        if (cell < L.hw)
+        if (cell < L.HW)
             ml_cell<T>(a, L, b, cell, [&](int, int, uint32_t key) {
                 if ((key >> shift) == prefix) atomicAdd(&s_hist[(key >> (shift - 10)) & (kMlBins - 1)], 1u);
             });
@@ -202,7 +216,7 @@ __global__ void __launch_bounds__(kMlTile) filter_ml_refine_kernel(const FilterA
     }
     const uint32_t t = (uint32_t)st[ML_T];
     int above = 0, ties = 0;
-    if (cell < L.hw)
+    if (cell < L.HW)
         ml_cell<T>(a, L, b, cell, [&](int, int, uint32_t key) {
             above += key > t ? 1 : 0;
             ties += key == t ? 1 : 0;
@@ -266,7 +280,7 @@ __global__ void __launch_bounds__(kMlTile) filter_ml_emit_kernel(const FilterArg
         if (!keep) return;
         if (an != box_an) {   // the row's box, exactly as yb_filter_compact builds it
             uint32_t cs;
-            const T* x = reinterpret_cast<const T*>(L.pred) + frow_base(a, L, b, cell * (uint32_t)a.A + an, cs);
+            const T* x = reinterpret_cast<const T*>(L.pred) + ml_row(a, L, b, cell * (uint32_t)a.A + an, cs);
             float v[4], sg[4];
 #pragma unroll
             for (int k = 0; k < 4; ++k) v[k] = ldg_f(x + (size_t)k * cs);
@@ -322,7 +336,7 @@ static int ml_launch(const yb_heads_desc* d, const FilterArgs& a, const MlArgs& 
 extern "C" size_t yb_filter_multilabel_workspace_bytes(const yb_heads_desc* d, int max_candidates) {
     (void)max_candidates;   // the workspace does not depend on the cap
     yb::FilterArgs a;
-    if (yb::filter_fill(d, a, 1, yb::kMlTile)) return 0;
+    if (yb::filter_fill(d, "filter_multilabel", false, a, 1, yb::kMlTile)) return 0;
     const yb::FilterNchw n = yb::filter_cell_tiles(a, d->S, yb::kMlTile);
     return yb::ml_workspace(d->B, n.tiles_per_img, nullptr, nullptr);
 }
@@ -332,11 +346,11 @@ extern "C" int yb_filter_multilabel(const yb_heads_desc* d, float conf_thres, co
                                     void* ws, size_t ws_bytes, void* stream) {
     using namespace yb;
     FilterArgs a;
-    int rc = filter_fill(d, a, 1, kMlTile);
+    int rc = filter_fill(d, "filter_multilabel", true, a, 1, kMlTile);
     if (rc) return rc;
     YB_CHECK_ARG(max_candidates >= 1, "filter_multilabel: max_candidates must be >= 1, got %d", max_candidates);
     unsigned long long rows = 0;
-    for (int s = 0; s < d->S; ++s) rows += a.sc[s].rows;
+    for (int s = 0; s < d->S; ++s) rows += a.sc[s].img_rows;
     const unsigned long long pairs = rows * (unsigned long long)d->nc;
     YB_CHECK_ARG(pairs < (1ull << 31), "filter_multilabel: rows * nc too large");
     const unsigned long long need_cap = pairs < (unsigned long long)max_candidates ? pairs : (unsigned long long)max_candidates;
@@ -346,8 +360,6 @@ extern "C" int yb_filter_multilabel(const yb_heads_desc* d, float conf_thres, co
     YB_CHECK_ARG(boxes && scores && classes && counts && ws && cap > 0, "filter_multilabel: null output");
     YB_CHECK_ARG(aligned16(boxes) && (reinterpret_cast<uintptr_t>(ws) & 3u) == 0,
                  "filter_multilabel: boxes must be 16-byte, the workspace 4-byte aligned");
-    for (int s = 0; s < d->S; ++s)
-        YB_CHECK_ARG(d->pred[s] && d->anchors[s] && aligned16(d->pred[s]), "filter_multilabel: bad tensor at scale %d", s);
     if (ws_bytes < yb_filter_multilabel_workspace_bytes(d, max_candidates)) {
         set_error("filter_multilabel: workspace too small");
         return YB_EWORKSPACE;

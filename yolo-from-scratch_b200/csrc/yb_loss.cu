@@ -149,24 +149,16 @@ __global__ void ciou_mean_kernel(const double* __restrict__ acc, long long N, fl
 // ------------------------------------------------------------------------------------------
 constexpr int kTileRows = 256;  // rows per tile == threads per CTA of loss_main_kernel
 
-struct LossScale {
-    const void* pred;     // element type T of the kernels
+struct LossScale : HeadScale {   // pred and grad: in the layout of head_row_offset
     const float* tgt;
-    const float* anchors;
     void* grad;           // fp32: written by stage 1; half: written by yb_loss_grad_emit only
     float* dobj;          // half heads: fp32 objectness gradient of every row (canonical order), else null
     const uint32_t* bits; // sparse targets: 1 bit per row (positive), else null
-    uint32_t rows;        // B*H*W*A (local)
+    uint32_t n_rows;      // rows of all (local) images = B*img_rows
+    uint32_t n_float;     // n_rows * row
     uint32_t tile_begin;  // first global tile index of this scale
     uint32_t list_begin;  // offset of this scale's positive list in ws
-    int H, W;
-    float inv_w, inv_h;
     float obj_scale;      // coef_obj / (B_global*H*W*A)
-    FastDiv d_A, d_W, d_H;
-    // NCHW layout (f-2): pred/grad are (B, A*row, H, W); element (r, c) of canonical row r=(b,gy,gx,a)
-    // lives at ((b*A + a)*row + c)*HW + gy*W + gx
-    uint32_t HW, n_float;
-    FastDiv d_HW;
 };
 
 struct LossArgs {
@@ -186,19 +178,6 @@ struct LossArgs {
     const double* red;   // half emit pass: the reduced partials (P_s of the normalisation), else null
     const float* gscale; // half emit pass: upstream gradient s of `total` (device), else null
 };
-
-// offset of channel 0 of canonical row r, and the distance between its channels
-__device__ __forceinline__ size_t row_base(const LossArgs& a, const LossScale& L, uint32_t r, uint32_t& cstride) {
-    if (!a.nchw) {
-        cstride = 1u;
-        return (size_t)r * a.row;
-    }
-    uint32_t cellb, an, b, cell;
-    L.d_A.divmod(r, cellb, an);
-    L.d_HW.divmod(cellb, b, cell);
-    cstride = L.HW;
-    return ((size_t)(b * a.A + an) * a.row) * L.HW + cell;
-}
 
 struct LossWs {
     int pos_count[YB_MAX_SCALES];
@@ -221,7 +200,7 @@ __global__ void __launch_bounds__(kTileRows) loss_main_kernel(const LossArgs a) 
             if (k < a.S && tile >= a.sc[k].tile_begin) s = k;
         const LossScale& L = a.sc[s];
         const uint32_t row0 = (tile - L.tile_begin) * kTileRows;
-        const uint32_t nrows = min((uint32_t)kTileRows, L.rows - row0);
+        const uint32_t nrows = min((uint32_t)kTileRows, L.n_rows - row0);
 
         // phase 1: objectness of one row per thread (4-byte loads at a stride of one row:
         // one 32-byte sector per row of pred and of target)
@@ -435,19 +414,17 @@ __global__ void __launch_bounds__(256) loss_positive_kernel(const LossArgs a) {
         for (uint32_t k = gwarp; k < P; k += nwarps) {
             const uint32_t r = a.pos_list[L.list_begin + k];
             uint32_t cs;
-            const size_t xb = row_base(a, L, r, cs);
+            const size_t xb = head_row_offset(L, a.nchw, a.row, 0, r, cs);
             const T* x = reinterpret_cast<const T*>(L.pred) + xb;
             const float* t = SPARSE ? nullptr : L.tgt + (size_t)r * a.row;  // dense targets keep the reference layout
             SparseEntry ent = {0.f, 0.f, 0.f, 0.f, 0, 0, 0, 0};
             if (SPARSE) ent = a.entries[a.pos_ent[L.list_begin + k]];
-            uint32_t cell, an, gy_b, gx, gy, bi;
-            L.d_A.divmod(r, cell, an);
-            L.d_W.divmod(cell, gy_b, gx);
-            L.d_H.divmod(gy_b, bi, gy);
+            uint32_t b, gy, gx, an;
+            head_row_coords(L, r, b, gy, gx, an);
             const float aw = __ldg(L.anchors + an * 2), ah = __ldg(L.anchors + an * 2 + 1);
             const float xr[4] = {to_f32(x[0]), to_f32(x[(size_t)cs]), to_f32(x[2 * (size_t)cs]), to_f32(x[3 * (size_t)cs])};
-            const float p[4] = {decode_xy(xr[0], (float)gx, L.inv_w), decode_xy(xr[1], (float)gy, L.inv_h),
-                                decode_wh(xr[2], aw, a.inv_img), decode_wh(xr[3], ah, a.inv_img)};
+            const float p[4] = {box_xy(sigmoidf_ref(xr[0]), (float)gx, L.inv_w), box_xy(sigmoidf_ref(xr[1]), (float)gy, L.inv_h),
+                                box_wh(sigmoidf_ref(xr[2]), aw, a.inv_img), box_wh(sigmoidf_ref(xr[3]), ah, a.inv_img)};
             const float tb[4] = {SPARSE ? ent.x : t[0], SPARSE ? ent.y : t[1], SPARSE ? ent.w : t[2],
                                  SPARSE ? ent.h : t[3]};
             float gp[4];
@@ -465,17 +442,10 @@ __global__ void __launch_bounds__(256) loss_positive_kernel(const LossArgs a) {
             }
             cls = warp_sum(cls);
             if (L.grad && lane < 4) {
-                // chain through decode (same order as decode_kernel<true>)
+                // chain through decode
                 const float sgm = sigmoidf_ref(xr[lane]);
-                const float ds = (1.0f - sgm) * sgm;
-                float g;
-                if (lane < 2) {
-                    g = ((gp[lane] * (lane == 0 ? L.inv_w : L.inv_h)) * 2.0f) * ds;
-                } else {
-                    const float anc = lane == 2 ? aw : ah;
-                    const float u = 2.0f * sgm;
-                    g = (((gp[lane] * (anc * a.inv_img)) * (2.0f * u)) * 2.0f) * ds;
-                }
+                const float g = lane < 2 ? box_xy_vjp(sgm, gp[lane], lane == 0 ? L.inv_w : L.inv_h)
+                                         : box_wh_vjp(sgm, gp[lane], lane == 2 ? aw : ah, a.inv_img);
                 put(xb + (size_t)lane * cs, g, k_box);
             }
             acc_box += (double)l;
@@ -518,7 +488,7 @@ __global__ void __launch_bounds__(256) loss_finalize_kernel(const FinalizeArgs f
         const float k_cls = a.nc > 0 ? (float)((double)f.coef_cls[s] / (Pg * (double)a.nc)) : 0.0f;
         for (uint32_t k = gwarp; k < P; k += nwarps) {
             uint32_t cs;
-            float* g = reinterpret_cast<float*>(L.grad) + row_base(a, L, a.pos_list[L.list_begin + k], cs);
+            float* g = reinterpret_cast<float*>(L.grad) + head_row_offset(L, a.nchw, a.row, 0, a.pos_list[L.list_begin + k], cs);
             if (lane < 4) g[(size_t)lane * cs] *= k_box;
             for (int c = lane; c < a.nc; c += 32) g[(size_t)(5 + c) * cs] *= k_cls;
         }
@@ -612,27 +582,28 @@ __global__ void __launch_bounds__(256) loss_grad_emit_kernel(const LossArgs a) {
 }
 
 // ---- host side ----------------------------------------------------------------------------
-static int loss_validate(const yb_loss_desc* d, bool need_ptrs, bool sparse = false) {
-    YB_CHECK_ARG(d, "loss: null descriptor");
-    YB_CHECK_ARG(d->S >= 1 && d->S <= YB_MAX_SCALES, "loss: S=%d out of range", d->S);
-    YB_CHECK_ARG(d->B >= 0 && d->A > 0 && d->A <= YB_MAX_ANCHORS && d->nc >= 0, "loss: bad B/A/nc");
-    YB_CHECK_ARG(d->B_global >= d->B, "loss: B_global < B");
-    YB_CHECK_ARG(d->layout == YB_LAYOUT_BHWAC || d->layout == YB_LAYOUT_NCHW, "loss: unknown layout %d", d->layout);
-    YB_CHECK_ARG(d->dtype == YB_DTYPE_F32 || d->dtype == YB_DTYPE_BF16 || d->dtype == YB_DTYPE_F16,
-                 "loss: unknown dtype %d", d->dtype);
-    unsigned long long tot = 0;
-    for (int s = 0; s < d->S; ++s) {
-        YB_CHECK_ARG(d->H[s] > 0 && d->W[s] > 0, "loss: bad grid at scale %d", s);
-        unsigned long long n = (unsigned long long)d->B * d->H[s] * d->W[s] * d->A * (5 + d->nc);
-        YB_CHECK_ARG(n < (1ull << 32), "loss: scale %d too large", s);
-        tot += (unsigned long long)d->B * d->H[s] * d->W[s] * d->A;
-        if (need_ptrs && d->B > 0) {
-            YB_CHECK_ARG(d->pred[s] && (sparse || d->tgt[s]) && d->anchors[s], "loss: null tensor at scale %d", s);
-            YB_CHECK_ARG(aligned16(d->pred[s]) && (sparse || aligned16(d->tgt[s])) && aligned16(d->grad[s]),
-                         "loss: tensors must be 16-byte aligned");
-        }
+// the head fields of the loss descriptor
+static yb_heads_desc loss_heads(const yb_loss_desc* d) {
+    yb_heads_desc h = {};
+    h.S = d->S; h.B = d->B; h.A = d->A; h.nc = d->nc;
+    h.img_size = d->img_size; h.layout = d->layout; h.dtype = d->dtype;
+    for (int s = 0; s < YB_MAX_SCALES; ++s) {
+        h.H[s] = d->H[s]; h.W[s] = d->W[s];
+        h.pred[s] = d->pred[s]; h.anchors[s] = d->anchors[s];
     }
-    YB_CHECK_ARG(tot < (1ull << 32), "loss: too many rows");
+    return h;
+}
+
+static int loss_validate(const yb_loss_desc* d, const char* who, bool need_ptrs, bool sparse = false) {
+    YB_CHECK_ARG(d, "%s: null descriptor", who);
+    const int rc = heads_check(loss_heads(d), who, 0, true, true, need_ptrs);
+    if (rc) return rc;
+    YB_CHECK_ARG(d->B_global >= d->B, "%s: B_global < B", who);
+    for (int s = 0; s < d->S && need_ptrs && d->B > 0; ++s) {
+        YB_CHECK_ARG(sparse || d->tgt[s], "%s: null tgt at scale %d", who, s);
+        YB_CHECK_ARG((sparse || aligned16(d->tgt[s])) && aligned16(d->grad[s]),
+                     "%s: tgt and grad must be 16-byte aligned (scale %d)", who, s);
+    }
     return 0;
 }
 
@@ -647,6 +618,7 @@ static size_t dobj_bytes(const yb_loss_desc* d) { return d->dtype == YB_DTYPE_F3
 
 static void loss_fill_args(const yb_loss_desc* d, void* ws, LossArgs& a) {
     const bool half = d->dtype != YB_DTYPE_F32;
+    const yb_heads_desc h = loss_heads(d);
     a.S = d->S; a.A = d->A; a.nc = d->nc; a.row = 5 + d->nc;
     a.nchw = d->layout == YB_LAYOUT_NCHW ? 1 : 0;
     a.inv_img = 1.0f / d->img_size; a.eps = d->eps;
@@ -657,25 +629,21 @@ static void loss_fill_args(const yb_loss_desc* d, void* ws, LossArgs& a) {
     uint32_t tile = 0, list = 0;
     for (int s = 0; s < d->S; ++s) {
         LossScale& L = a.sc[s];
-        L.pred = d->pred[s]; L.tgt = d->tgt[s]; L.anchors = d->anchors[s];
+        head_scale_fill(L, h, s);
+        L.tgt = d->tgt[s];
         L.grad = half ? nullptr : d->grad[s];   // half: only yb_loss_grad_emit writes the gradient
         L.dobj = half ? reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + dobj_offset(d)) + list : nullptr;
         L.bits = nullptr;
-        L.rows = (uint32_t)((unsigned long long)d->B * d->H[s] * d->W[s] * d->A);
+        L.n_rows = L.img_rows * (uint32_t)d->B;
         L.tile_begin = tile; L.list_begin = list;
-        L.HW = (uint32_t)d->H[s] * (uint32_t)d->W[s];
-        L.n_float = L.rows * a.row;
-        L.d_HW = FastDiv(L.HW);
+        L.n_float = L.n_rows * a.row;
         // reference layout: one tile = kTileRows rows; NCHW: one tile = kTileRows*kNchwVecs steps of 4 elements of the
         // flat tensor
         tile += a.nchw ? (L.n_float + kTileRows * 4 * kNchwVecs - 1) / (kTileRows * 4 * kNchwVecs)
-                       : (L.rows + kTileRows - 1) / kTileRows;
-        list += L.rows;
-        L.H = d->H[s]; L.W = d->W[s];
-        L.inv_w = 1.0f / (float)d->W[s]; L.inv_h = 1.0f / (float)d->H[s];
+                       : (L.n_rows + kTileRows - 1) / kTileRows;
+        list += L.n_rows;
         double n_obj = (double)d->B_global * d->H[s] * d->W[s] * d->A;
         L.obj_scale = (float)((double)d->coef_obj[s] / n_obj);
-        L.d_A = FastDiv(d->A); L.d_W = FastDiv(d->W[s]); L.d_H = FastDiv(d->H[s]);
     }
     a.n_tiles = tile;
     a.pos_ent = nullptr;
@@ -757,7 +725,7 @@ static int loss_stage1_launch(const LossArgs& a, cudaStream_t st) {
 extern "C" int yb_loss_partials(const yb_loss_desc* d, double* partials, void* ws, size_t ws_bytes,
                                 void* stream) {
     using namespace yb;
-    int rc = loss_validate(d, true);
+    int rc = loss_validate(d, "loss", true);
     if (rc) return rc;
     YB_CHECK_ARG(partials && ws, "loss: null partials/workspace");
     if (ws_bytes < yb_loss_workspace_bytes(d)) {
@@ -785,7 +753,7 @@ extern "C" int yb_loss_partials_sparse(const yb_loss_desc* d, const double* labe
                                        int assign_img_size, int* status, double* partials, void* ws,
                                        size_t ws_bytes, void* stream) {
     using namespace yb;
-    int rc = loss_validate(d, true, true);
+    int rc = loss_validate(d, "loss(sparse)", true, true);
     if (rc) return rc;
     YB_CHECK_ARG(partials && ws && n_gt && letterbox && anchors_all && max_gt >= 0 && (max_gt == 0 || labels) &&
                      assign_img_size > 0,
@@ -830,7 +798,7 @@ extern "C" int yb_loss_partials_sparse(const yb_loss_desc* d, const double* labe
 extern "C" int yb_loss_finalize(const yb_loss_desc* d, const double* partials, float* out4,
                                 float* per_scale, void* ws, size_t ws_bytes, void* stream) {
     using namespace yb;
-    int rc = loss_validate(d, false);
+    int rc = loss_validate(d, "loss_finalize", false);
     if (rc) return rc;
     YB_CHECK_ARG(partials && out4 && ws, "loss_finalize: null pointer");
     if (ws_bytes < yb_loss_workspace_bytes(d)) {
@@ -871,7 +839,7 @@ extern "C" int yb_loss_grad_emit(const yb_loss_desc* d, const double* partials, 
                                  void* ws, size_t ws_bytes, void* stream) {
     using namespace yb;
     const bool sparse = max_gt >= 0;
-    int rc = loss_validate(d, true, sparse);
+    int rc = loss_validate(d, "loss_grad_emit", true, sparse);
     if (rc) return rc;
     YB_CHECK_ARG(d->dtype != YB_DTYPE_F32, "loss_grad_emit: fp32 heads get their gradient from yb_loss_partials");
     YB_CHECK_ARG(partials && grad_scale && ws, "loss_grad_emit: null pointer");
